@@ -2,7 +2,7 @@
 """bench.py -- the headline metric of BASELINE.json on synthetic data: log-mel audio-hours/sec (n_fft 800, hop 160,
 128 mels) over an IEMOCAP-sized corpus, plus cloak+GRL training utterances/sec as a secondary figure.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 One step = one pass of the extraction hot path over one corpus-sized ragged batch (5531 utterances, 2-10 s each,
 ~9.2 audio-hours, 2.1 GB of fp32 waveform -- larger than the 126 MB L2, so no flush is needed between steps).
@@ -36,6 +36,7 @@ CORPUS_UTTS = 5531                         # IEMOCAP 4-class size (SURVEY 8d, co
 FLOP_PER_FRAME = 22999                     # BASELINE.md section 3: log-mel n_fft=800 (rFFT 2.5 N log2 N + window + power + mel + log)
 BYTES_PER_FRAME = 4 * HOP + 4 * N_MELS     # waveform read once + features written once = 1152 B
 FP32_LANES_PER_SM = 128
+DUMP_ROWS = 65536                          # feature rows --dump-outputs writes, split over the ranks: 32 MiB in all
 
 
 def dist_env():
@@ -273,6 +274,8 @@ def run_b200(args):
     total_ms = evs[0].elapsed_time(evs[-1])
     kernel_ms = [evs[k].elapsed_time(evs[k + 1]) for k in range(args.steps)]     # one launch per step on this stream
     clocks = sampler.window(t0, t1) if sampler else None
+    if args.dump_outputs:
+        dump_outputs(Path(args.dump_outputs), out, lay, rank, world)
 
     # ---- end to end through the public API with HOST buffers ("e2e") ----------------------------------------
     if args.no_extras:
@@ -346,6 +349,21 @@ def run_b200(args):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def dump_outputs(dst: Path, feats: torch.Tensor, lay, rank: int, world: int):
+    """What the last timed extraction.logmel call returned, for comparing two builds output by output: DUMP_ROWS //
+    world feature rows of this rank drawn with a seed fixed per rank (logmel.npy, float32), their row indices
+    (logmel_rows.npy) and the per-utterance frame offsets of the layout (frame_offsets.npy), both float64.  With
+    N > 1 every rank adds a _rank<r> suffix.  The total is about 34 MB at any N: 32 MiB of features, 0.5 MiB of
+    row indices and 44 KB of frame offsets per rank."""
+    dst.mkdir(parents=True, exist_ok=True)
+    n = feats.shape[0]
+    rows = np.sort(np.random.default_rng(rank).choice(n, size=min(DUMP_ROWS // world, n), replace=False))
+    suffix = "" if world == 1 else f"_rank{rank}"
+    np.save(dst / f"logmel{suffix}.npy", feats[torch.from_numpy(rows).to(feats.device)].cpu().numpy())
+    np.save(dst / f"logmel_rows{suffix}.npy", rows.astype(np.float64))
+    np.save(dst / f"frame_offsets{suffix}.npy", lay.frame_off_host.astype(np.float64))
 
 
 def measure_e2e(args, extraction, wav, utt_off, frames, out, dev, barrier):
@@ -548,7 +566,13 @@ def main():
     ap.add_argument("--utts", type=int, default=CORPUS_UTTS, help="utterances per GPU (debug only; the metric is quoted on the default)")
     ap.add_argument("--no-bulk", action="store_true", help="skip the 1000-audio-hour bulk extraction (BASELINE.json configs[3]) in extras")
     ap.add_argument("--bulk-hours", type=float, default=1000.0, help="size of the bulk extraction job in extras")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a seeded sample of the last step's "
+                                                          "log-mel features and its frame offsets to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the b200 path computes; the reference arm keeps no outputs")
     if args.impl == "reference":
         run_reference(args)
     else:

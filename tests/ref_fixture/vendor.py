@@ -7,15 +7,20 @@ TEST INFRASTRUCTURE ONLY.  These files are the unmodified MIT-licensed sources o
 own train() / test() functions "run unchanged" against the drop-in modules, and the GPU box that runs the parity tests
 has no /root/reference.  Nothing in the product package imports, reads or executes anything under tests/ref_fixture/;
 tests/ref_harness.py drives them.  `--check` verifies the committed copies still equal the reference byte for byte.
+Copying also records the SHA-256 of every copied file in tests/golden/ref_fixture_sha256.json, so the test suite can
+check the copies against the reference without a checkout of it; `--check` verifies that file against the reference too.
 """
 from __future__ import annotations
 
+import hashlib
+import json
 import shutil
 import sys
 from pathlib import Path
 
 REF = Path("/root/reference")
 HERE = Path(__file__).resolve().parent
+DIGESTS = HERE.parent / "golden" / "ref_fixture_sha256.json"
 FILES = [
     "LICENSE",
     "training/training_cloak_with_grl.py",
@@ -41,6 +46,13 @@ def main(check: bool) -> int:
             dst.parent.mkdir(parents=True, exist_ok=True)
             shutil.copyfile(src, dst)
             print("copied", rel)
+    digests = {rel: hashlib.sha256((REF / rel).read_bytes()).hexdigest() for rel in FILES}
+    if check:
+        same = DIGESTS.exists() and json.loads(DIGESTS.read_text()) == digests
+        print(("ok      " if same else "DIFFERS ") + str(DIGESTS.relative_to(HERE.parent.parent)))
+        bad += not same
+    else:
+        DIGESTS.write_text(json.dumps(digests, indent=1) + "\n")
     return bad
 
 
