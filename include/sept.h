@@ -46,6 +46,7 @@ const char* sept_last_error(void);
 const char* sept_source_hash(void);
 
 /* Build the constant cache of the current device for n_fft in {400, 800, 1600} x n_mels, and the 128x40 DCT basis.
+ * The log-mel backward (sept_logmel_bwd_f32) runs on the same constants.
  * Optional (first use does it), but call it before CUDA-graph capture. */
 int sept_init(int n_mels);
 
@@ -69,6 +70,18 @@ int sept_extract_layout(const int64_t* utt_off_host, int n_utts, int n_fft, int 
 int sept_logmel_f32(const float* wav_dev, const int64_t* utt_off_dev, const int64_t* frame_off_dev,
                     const int32_t* item_off_dev, int n_utts, int n_fft, int hop, int n_mels, int deriv, int layout,
                     float* out_dev, sept_stream_t stream);
+
+/* Waveform gradient of the frame-major, deriv-0 log-mel of sept_logmel_f32 (the gradient torchaudio's MelSpectrogram +
+ * AmplitudeToDB give under autograd): dwav = d(sum_{f,b} grad[f,b] * logmel[f,b]) / d wav, where grad_dev holds
+ * total_frames * n_mels floats in the frame-major layout.  The clamp at 1e-10 passes no gradient (bands of zero power
+ * give exactly 0).  Writes dwav for every sample of every utterance (samples outside all utterances are untouched).
+ * n_items = item_off[n_utts]; workspace_dev holds sept_logmel_bwd_workspace_bytes(n_fft, hop, n_items) bytes (16-byte
+ * aligned; about 0.46 GB per audio-hour at n_fft 800, hop 160).  Accepts every (n_fft, hop, n_mels) sept_logmel_f32
+ * accepts.  Deterministic (no atomics), no allocation, capturable. */
+size_t sept_logmel_bwd_workspace_bytes(int n_fft, int hop, int64_t n_items);
+int sept_logmel_bwd_f32(const float* wav_dev, const int64_t* utt_off_dev, const int64_t* frame_off_dev,
+                        const int32_t* item_off_dev, int n_utts, int64_t n_items, int n_fft, int hop, int n_mels,
+                        const float* grad_dev, void* workspace_dev, float* dwav_dev, sept_stream_t stream);
 
 /* MFCC-40 of the waveform, of np.gradient(waveform) and of np.gradient(waveform, 2).  Replaces mfcc(audio)
  * (feature_extraction/audio_feature_extraction.py:15-26 -> torchaudio/transforms/_transforms.py:634-718): n_fft 400,

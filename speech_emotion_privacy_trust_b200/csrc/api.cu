@@ -15,6 +15,7 @@
 #include "augment.h"
 #include "cloak.h"
 #include "extract.h"
+#include "extract_bwd.h"
 #include "norm.h"
 #include "resample.h"
 #include "tables.h"
@@ -232,6 +233,34 @@ int sept_logmel_f32(const float* wav, const int64_t* utt_off, const int64_t* fra
     p.out = out;
     const int mode = layout == SEPT_LAYOUT_FRAME_MAJOR ? sept::kModeDbFrameMajor : sept::kModeDbBandMajor;
     SEPT_CUDA(sept::launch_extract(p, n_fft, mode, sms, static_cast<cudaStream_t>(stream)));
+    return SEPT_OK;
+}
+
+size_t sept_logmel_bwd_workspace_bytes(int n_fft, int hop, int64_t n_items) {
+    return sept::logmel_bwd_workspace_bytes(n_fft, hop, n_items);
+}
+
+int sept_logmel_bwd_f32(const float* wav, const int64_t* utt_off, const int64_t* frame_off, const int32_t* item_off,
+                        int n_utts, int64_t n_items, int n_fft, int hop, int n_mels, const float* grad, void* workspace,
+                        float* dwav, sept_stream_t stream) {
+    if (n_utts == 0 || n_items == 0) return SEPT_OK;
+    if (!wav || !utt_off || !frame_off || !item_off || !grad || !workspace || !dwav || n_utts < 0 || n_items < 0)
+        return fail(SEPT_E_BADARG, "sept_logmel_bwd_f32: null pointer or negative size");
+    if (!aligned16(workspace)) return fail(SEPT_E_BADARG, "sept_logmel_bwd_f32: workspace must be 16-byte aligned");
+    int rc = check_extract_shape(n_fft, hop, n_mels, -1);
+    if (rc) return rc;
+    ExtractConsts c;
+    int sms = 0;
+    rc = get_consts(n_fft, n_mels, &c, &sms);
+    if (rc) return rc;
+    rc = check_extract_shape(n_fft, hop, n_mels, c.n_mel_entries);   // what the forward accepts, the backward takes
+    if (rc) return rc;
+    sept::LogmelBwdParams p{};
+    p.wav = wav; p.utt_off = utt_off; p.frame_off = frame_off; p.item_off = item_off; p.n_utts = n_utts; p.n_items = n_items;
+    p.hop = hop; p.n_mels = n_mels; p.n_mel_entries = c.n_mel_entries; p.n_mel_head = c.n_mel_head; p.fast_dn = c.mel_fast;
+    p.window = c.window; p.tws = c.tws; p.mel_prog = c.mel_prog;
+    p.grad = grad; p.ws = static_cast<float*>(workspace); p.dwav = dwav;
+    SEPT_CUDA(sept::launch_logmel_bwd(p, n_fft, sms, static_cast<cudaStream_t>(stream)));
     return SEPT_OK;
 }
 

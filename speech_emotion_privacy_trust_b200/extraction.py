@@ -10,6 +10,7 @@ from typing import Sequence
 
 import numpy as np
 import torch
+from torch.autograd.function import once_differentiable
 
 from . import _lib
 
@@ -114,6 +115,53 @@ def logmel(batch: RaggedAudio, n_fft: int = 800, n_mels: int = 128, hop: int = H
                                               lay.item_off.data_ptr(), batch.n_utts, n_fft, hop, n_mels, int(deriv),
                                               1 if band_major else 0, out.data_ptr(), _stream(dev)))
     return out, lay
+
+
+class LogMelFunction(torch.autograd.Function):
+    """Frame-major log-mel dB with a waveform gradient: forward is one sept_logmel_f32 launch, backward one
+    sept_logmel_bwd_f32 launch (recomputes the spectrum from the saved waveform; no double backward)."""
+
+    @staticmethod
+    def forward(ctx, wav, batch, n_fft, n_mels, hop):
+        out, lay = logmel(batch, n_fft, n_mels, hop)
+        ctx.save_for_backward(wav)
+        fpw = _lib.lib().sept_frames_per_item(n_fft)
+        ctx.n_items = int((-(-np.diff(lay.frame_off_host) // fpw)).sum())   # item_off[n_utts], from host data
+        ctx.batch, ctx.lay, ctx.shape = batch, lay, (n_fft, n_mels, hop)
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad):
+        (wav,) = ctx.saved_tensors
+        batch, lay = ctx.batch, ctx.lay
+        n_fft, n_mels, hop = ctx.shape
+        n_items = ctx.n_items
+        lib = _lib.lib()
+        dwav = torch.zeros_like(wav)                              # samples outside every utterance get no gradient
+        ws = torch.empty(max(1, lib.sept_logmel_bwd_workspace_bytes(n_fft, hop, n_items)), dtype=torch.uint8,
+                         device=wav.device)
+        grad = grad.contiguous()
+        with torch.cuda.device(wav.device):
+            _lib.check(lib.sept_logmel_bwd_f32(wav.data_ptr(), batch.utt_off.data_ptr(), lay.frame_off.data_ptr(),
+                                               lay.item_off.data_ptr(), batch.n_utts, n_items, n_fft, hop, n_mels,
+                                               grad.data_ptr(), ws.data_ptr(), dwav.data_ptr(), _stream(wav.device)))
+        return dwav, None, None, None, None
+
+
+def logmel_grad(batch: RaggedAudio, n_fft: int = 800, n_mels: int = 128, hop: int = HOP_MEL, band_major: bool = False,
+                deriv: bool = False) -> tuple[torch.Tensor, Layout]:
+    """logmel() with a gradient: the (total_frames, n_mels) frame-major features carry a grad_fn back to batch.wav.
+
+    Values are bit-identical to logmel().  The backward writes d/d wav for every sample of every utterance (zero
+    elsewhere), deterministically.  Only the frame-major waveform stream is differentiable: band_major (one transpose in
+    torch away) and deriv raise ValueError."""
+    if band_major:
+        raise ValueError("logmel_grad: only the frame-major layout has a gradient; transpose the result instead")
+    if deriv:
+        raise ValueError("logmel_grad: the np.gradient stream (deriv) has no gradient")
+    lay = batch.layout(n_fft, hop)
+    return LogMelFunction.apply(batch.wav, batch, n_fft, n_mels, hop), lay
 
 
 def mfcc(batch: RaggedAudio, out: torch.Tensor | None = None) -> tuple[torch.Tensor, Layout]:
