@@ -94,6 +94,20 @@ int sept_mfcc_f32(const float* wav_dev, const int64_t* utt_off_dev, const int64_
                   const int32_t* item_off_dev, int n_utts, int64_t total_frames, float* scratch_dev,
                   int32_t* utt_max_dev, float* out_dev, sept_stream_t stream);
 
+/* Waveform gradient of sept_mfcc_f32 (what torch autograd gives through torchaudio's MFCC for the three streams of
+ * mfcc(audio): x, np.gradient(x), np.gradient(x, 2)): dwav = d(sum grad * mfcc) / d wav, where grad_dev holds
+ * total_frames * 120 floats in sept_mfcc_f32's (120, T_u) block layout.  The top_db floor sends the gradient of every
+ * floored value to the utterance's maximum (split evenly among tied maxima), the clamp at 1e-10 passes none.  Layouts
+ * from sept_extract_layout(n_fft = 400, hop = 200); n_items = item_off[n_utts].  Writes dwav for every sample of every
+ * utterance (samples outside all utterances are untouched).  workspace_dev holds
+ * sept_mfcc_bwd_workspace_bytes(n_utts, total_frames, n_items) bytes, 16-byte aligned: 2876 bytes per frame plus 8 per
+ * utterance, about 0.83 GB per audio-hour (288 000 frames), computed from the shapes.  Recomputes the mel power from
+ * the waveform; deterministic (no atomics), no allocation, capturable. */
+size_t sept_mfcc_bwd_workspace_bytes(int n_utts, int64_t total_frames, int64_t n_items);
+int sept_mfcc_bwd_f32(const float* wav_dev, const int64_t* utt_off_dev, const int64_t* frame_off_dev,
+                      const int32_t* item_off_dev, int n_utts, int64_t total_frames, int64_t n_items,
+                      const float* grad_dev, void* workspace_dev, float* dwav_dev, sept_stream_t stream);
+
 /* ---- resampling ahead of extraction --------------------------------------------------------------------------------
  * Band-limited sinc resampling of a ragged batch.  Replaces torchaudio.transforms.Resample(sample_rate, 16000) as the
  * reference applies it to the 44.1 kHz MSP-Improv corpus (feature_extraction/audio_feature_extraction.py:139-141 ->

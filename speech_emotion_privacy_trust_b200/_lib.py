@@ -24,6 +24,8 @@ _SIGNATURES = {
     "sept_logmel_bwd_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr,
                                       c_ptr]),
     "sept_mfcc_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int64, c_ptr, c_ptr, c_ptr, c_ptr]),
+    "sept_mfcc_bwd_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int64, C.c_int64]),
+    "sept_mfcc_bwd_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int64, C.c_int64, c_ptr, c_ptr, c_ptr, c_ptr]),
     "sept_resample_layout": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, c_ptr]),
     "sept_resample_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int64, C.c_int, C.c_int, c_ptr, c_ptr]),
     "sept_pcm16_to_f32": (C.c_int, [c_ptr, C.c_int64, c_ptr, c_ptr]),

@@ -17,7 +17,7 @@ from pathlib import Path
 PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB = PKG / "libsept_b200.so"
-SOURCES = ["api.cu", "extract.cu", "extract_bwd.cu", "mfcc_dct.cu", "mfcc_tc.cu", "cloak.cu", "norm.cu", "resample.cu", "augment.cu"]
+SOURCES = ["api.cu", "extract.cu", "extract_bwd.cu", "mfcc_bwd.cu", "mfcc_dct.cu", "mfcc_tc.cu", "cloak.cu", "norm.cu", "resample.cu", "augment.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--expt-relaxed-constexpr",
               "-Xcompiler", "-fPIC,-O2", "-diag-suppress", "20013"]
 

@@ -16,6 +16,7 @@
 #include "cloak.h"
 #include "extract.h"
 #include "extract_bwd.h"
+#include "mfcc_bwd.h"
 #include "norm.h"
 #include "resample.h"
 #include "tables.h"
@@ -294,6 +295,50 @@ int sept_mfcc_f32(const float* wav, const int64_t* utt_off, const int64_t* frame
     const char* which = getenv("SEPT_MFCC_DCT");
     if (which && which[0] == 't') SEPT_CUDA(sept::launch_mfcc_dct_tc(d, sms, st));
     else SEPT_CUDA(sept::launch_mfcc_dct(d, st));
+    return SEPT_OK;
+}
+
+size_t sept_mfcc_bwd_workspace_bytes(int n_utts, int64_t total_frames, int64_t n_items) {
+    return sept::mfcc_bwd_layout(n_utts, total_frames, n_items).bytes;
+}
+
+int sept_mfcc_bwd_f32(const float* wav, const int64_t* utt_off, const int64_t* frame_off, const int32_t* item_off,
+                      int n_utts, int64_t total_frames, int64_t n_items, const float* grad, void* workspace, float* dwav,
+                      sept_stream_t stream) {
+    if (n_utts == 0) return SEPT_OK;
+    if (!wav || !utt_off || !frame_off || !item_off || !grad || !workspace || !dwav || n_utts < 0 || total_frames <= 0 ||
+        n_items <= 0)
+        return fail(SEPT_E_BADARG, "sept_mfcc_bwd_f32: null pointer or bad size");
+    if (!aligned16(workspace)) return fail(SEPT_E_BADARG, "sept_mfcc_bwd_f32: workspace must be 16-byte aligned");
+    ExtractConsts c;
+    int sms = 0;
+    int rc = get_consts(400, 128, &c, &sms);
+    if (rc) return rc;
+    float* dct = nullptr;
+    rc = get_dct(&dct);
+    if (rc) return rc;
+    const sept::MfccBwdLayout l = sept::mfcc_bwd_layout(n_utts, total_frames, n_items);
+    unsigned char* ws = static_cast<unsigned char*>(workspace);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    // the forward's power launch (sept_mfcc_f32), deterministic: the same power, maxima and frame map bit for bit
+    int32_t* utt_max = reinterpret_cast<int32_t*>(ws + l.utt_max);
+    SEPT_CUDA(cudaMemsetAsync(utt_max, 0, sizeof(int32_t) * 2 * (size_t)n_utts, st));
+    sept::ExtractParams p{};
+    p.wav = wav; p.utt_off = utt_off; p.frame_off = frame_off; p.item_off = item_off;
+    p.n_utts = n_utts; p.hop = 200; p.n_mels = 128; p.n_mel_entries = c.n_mel_entries; p.n_mel_head = c.n_mel_head; p.mel_fast = c.mel_fast; p.total_frames = total_frames;
+    p.window = c.window; p.tws = c.tws; p.mel_prog = c.mel_prog;
+    p.out = reinterpret_cast<float*>(ws + l.power); p.utt_max = utt_max;
+    p.frame_utt = reinterpret_cast<int*>(ws + l.frame_utt);
+    SEPT_CUDA(sept::launch_extract(p, 400, sept::kModeMfccPower, sms, st));
+    sept::MfccBwdParams b{};
+    sept::LogmelBwdParams& f = b.frames;
+    f.wav = wav; f.utt_off = utt_off; f.frame_off = frame_off; f.item_off = item_off; f.n_utts = n_utts; f.n_items = n_items;
+    f.hop = 200; f.n_mels = 128; f.n_mel_entries = c.n_mel_entries; f.n_mel_head = c.n_mel_head; f.fast_dn = c.mel_fast;
+    f.window = c.window; f.tws = c.tws; f.mel_prog = c.mel_prog;
+    b.grad = grad; b.dct = dct; b.frame_utt = p.frame_utt; b.utt_max = utt_max; b.total_frames = total_frames;
+    b.power = p.out; b.part = reinterpret_cast<float*>(ws + l.part); b.amask = reinterpret_cast<uint32_t*>(ws + l.amask);
+    b.rows0 = reinterpret_cast<float*>(ws + l.rows0); b.rows1 = reinterpret_cast<float*>(ws + l.rows1); b.dwav = dwav;
+    SEPT_CUDA(sept::launch_mfcc_bwd(b, sms, st));
     return SEPT_OK;
 }
 

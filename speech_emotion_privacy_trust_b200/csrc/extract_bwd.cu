@@ -15,21 +15,6 @@
 
 namespace sept {
 
-constexpr int kBwdWarps = 8;     // warps per CTA at most (shared memory decides below)
-
-__device__ __forceinline__ int bwd_find_utt(const int32_t* __restrict__ item_off, int n_utts, long long item) {
-    int lo_ = 0, hi_ = n_utts - 1;
-    while (lo_ < hi_) {
-        const int mid = (lo_ + hi_) >> 1;
-        if (__ldg(item_off + mid + 1) > item) hi_ = mid; else lo_ = mid + 1;
-    }
-    return lo_;
-}
-
-__host__ __device__ inline int bwd_const_bytes(int R, int n_mel_entries) {
-    return (n_mel_entries * 16 + R * 25 * 8 + 13 * (R + 1) * 8 + 15) & ~15;
-}
-
 template <int R>
 __global__ void __launch_bounds__(kBwdWarps * 32, 1) logmel_bwd_frames_kernel(const LogmelBwdParams prm) {
     using G = Geo<R>;
@@ -128,15 +113,21 @@ static int bwd_warps(int hop, int n_mels, int n_mel_entries) {
 }
 
 template <int R>
-static cudaError_t launch_r(const LogmelBwdParams& prm, int sms, cudaStream_t stream) {
+static cudaError_t launch_frames(LogmelBwdFramesKernel kernel, const LogmelBwdParams& prm, int sms, cudaStream_t stream) {
     const int warps = bwd_warps<R>(prm.hop, prm.n_mels, prm.n_mel_entries);
     if (warps == 0) return cudaErrorInvalidConfiguration;
     const size_t smem = (size_t)bwd_const_bytes(R, prm.n_mel_entries) +
                         (size_t)warps * Bwd<Geo<R>>::warp_floats(prm.hop, prm.n_mels) * 4;
-    cudaError_t e = cudaFuncSetAttribute(logmel_bwd_frames_kernel<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
-    logmel_bwd_frames_kernel<R><<<sms, warps * 32, smem, stream>>>(prm);
-    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    kernel<<<sms, warps * 32, smem, stream>>>(prm);
+    return cudaGetLastError();
+}
+
+template <int R>
+static cudaError_t launch_r(const LogmelBwdParams& prm, int sms, cudaStream_t stream) {
+    cudaError_t e = launch_frames<R>(logmel_bwd_frames_kernel<R>, prm, sms, stream);
+    if (e != cudaSuccess) return e;
     logmel_bwd_gather_kernel<R><<<sms * 8, 256, 0, stream>>>(prm);
     return cudaGetLastError();
 }
@@ -148,6 +139,11 @@ cudaError_t launch_logmel_bwd(const LogmelBwdParams& prm, int n_fft, int sms, cu
         case 1600: return launch_r<32>(prm, sms, stream);
     }
     return cudaErrorInvalidValue;
+}
+
+cudaError_t launch_logmel_bwd_frames_400(const LogmelBwdParams& prm, LogmelBwdFramesKernel kernel, int sms,
+                                         cudaStream_t stream) {
+    return launch_frames<8>(kernel ? kernel : logmel_bwd_frames_kernel<8>, prm, sms, stream);
 }
 
 size_t logmel_bwd_workspace_bytes(int n_fft, int hop, long long n_items) {

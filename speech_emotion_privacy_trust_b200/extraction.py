@@ -182,6 +182,46 @@ def mfcc(batch: RaggedAudio, out: torch.Tensor | None = None) -> tuple[torch.Ten
     return out, lay
 
 
+class MfccFunction(torch.autograd.Function):
+    """MFCC blocks with a waveform gradient: forward is one sept_mfcc_f32 call, backward one sept_mfcc_bwd_f32 call
+    (recomputes the mel power from the saved waveform; no double backward)."""
+
+    @staticmethod
+    def forward(ctx, wav, batch):
+        out, lay = mfcc(batch)
+        ctx.save_for_backward(wav)
+        fpw = _lib.lib().sept_frames_per_item(N_FFT_MFCC)
+        ctx.n_items = int((-(-np.diff(lay.frame_off_host) // fpw)).sum())   # item_off[n_utts], from host data
+        ctx.batch, ctx.lay = batch, lay
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad):
+        (wav,) = ctx.saved_tensors
+        batch, lay, n_items = ctx.batch, ctx.lay, ctx.n_items
+        lib = _lib.lib()
+        dwav = torch.zeros_like(wav)                              # samples outside every utterance get no gradient
+        ws = torch.empty(max(1, lib.sept_mfcc_bwd_workspace_bytes(batch.n_utts, lay.total_frames, n_items)),
+                         dtype=torch.uint8, device=wav.device)
+        grad = grad.contiguous()
+        with torch.cuda.device(wav.device):
+            _lib.check(lib.sept_mfcc_bwd_f32(wav.data_ptr(), batch.utt_off.data_ptr(), lay.frame_off.data_ptr(),
+                                             lay.item_off.data_ptr(), batch.n_utts, lay.total_frames, n_items,
+                                             grad.data_ptr(), ws.data_ptr(), dwav.data_ptr(), _stream(wav.device)))
+        return dwav, None
+
+
+def mfcc_grad(batch: RaggedAudio) -> tuple[torch.Tensor, Layout]:
+    """mfcc() with a gradient: the flat (120, T_u) blocks carry a grad_fn back to batch.wav.
+
+    Values are bit-identical to mfcc().  The backward is what torch autograd gives through the reference's chain (the
+    top_db floor sends the gradient of floored values to the utterance's maximum) and writes d/d wav for every sample
+    of every utterance (zero elsewhere), deterministically."""
+    lay = batch.layout(N_FFT_MFCC, HOP_MFCC)
+    return MfccFunction.apply(batch.wav, batch), lay
+
+
 def split_band_major(flat: torch.Tensor, lay: Layout, rows: int) -> list[torch.Tensor]:
     """Views (rows, T_u) of a band-major flat buffer, one per utterance."""
     fo = lay.frame_off_host
