@@ -163,6 +163,40 @@ int check_extract_shape(int n_fft, int hop, int n_mels, int n_mel_entries) {
     return SEPT_OK;
 }
 
+// launch parameters shared by every extraction launch: the batch, its layout and the (n_fft, n_mels) constants
+sept::ExtractParams extract_params(const ExtractConsts& c, const float* wav, const int64_t* utt_off,
+                                   const int64_t* frame_off, const int32_t* item_off, int n_utts, int hop, int n_mels) {
+    sept::ExtractParams p{};
+    p.wav = wav; p.utt_off = utt_off; p.frame_off = frame_off; p.item_off = item_off;
+    p.n_utts = n_utts; p.hop = hop; p.n_mels = n_mels; p.n_mel_entries = c.n_mel_entries; p.n_mel_head = c.n_mel_head; p.mel_fast = c.mel_fast;
+    p.window = c.window; p.tws = c.tws; p.mel_prog = c.mel_prog;
+    return p;
+}
+
+// ... and of every frame pass of a backward
+sept::LogmelBwdParams logmel_bwd_params(const ExtractConsts& c, const float* wav, const int64_t* utt_off,
+                                        const int64_t* frame_off, const int32_t* item_off, int n_utts, long long n_items,
+                                        int hop, int n_mels) {
+    sept::LogmelBwdParams p{};
+    p.wav = wav; p.utt_off = utt_off; p.frame_off = frame_off; p.item_off = item_off; p.n_utts = n_utts; p.n_items = n_items;
+    p.hop = hop; p.n_mels = n_mels; p.n_mel_entries = c.n_mel_entries; p.n_mel_head = c.n_mel_head; p.fast_dn = c.mel_fast;
+    p.window = c.window; p.tws = c.tws; p.mel_prog = c.mel_prog;
+    return p;
+}
+
+// The MFCC forward's power launch: mel power of x and np.gradient(x) to power [2][total_frames][128], the bits of each
+// utterance's largest value to utt_max [2][n_utts], the utterance of every frame to frame_utt.  It is deterministic, so
+// the backward, which runs this same launch, recomputes the forward's values bit for bit.
+int launch_mfcc_power(const ExtractConsts& c, int sms, const float* wav, const int64_t* utt_off, const int64_t* frame_off,
+                      const int32_t* item_off, int n_utts, int64_t total_frames, float* power, int32_t* utt_max,
+                      int* frame_utt, cudaStream_t st) {
+    SEPT_CUDA(cudaMemsetAsync(utt_max, 0, sizeof(int32_t) * 2 * (size_t)n_utts, st));
+    sept::ExtractParams p = extract_params(c, wav, utt_off, frame_off, item_off, n_utts, 200, 128);
+    p.total_frames = total_frames; p.out = power; p.utt_max = utt_max; p.frame_utt = frame_utt;
+    SEPT_CUDA(sept::launch_extract(p, 400, sept::kModeMfccPower, sms, st));
+    return SEPT_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -227,10 +261,8 @@ int sept_logmel_f32(const float* wav, const int64_t* utt_off, const int64_t* fra
     if (rc) return rc;
     rc = check_extract_shape(n_fft, hop, n_mels, c.n_mel_entries);
     if (rc) return rc;
-    sept::ExtractParams p{};
-    p.wav = wav; p.utt_off = utt_off; p.frame_off = frame_off; p.item_off = item_off;
-    p.n_utts = n_utts; p.hop = hop; p.n_mels = n_mels; p.n_mel_entries = c.n_mel_entries; p.n_mel_head = c.n_mel_head; p.mel_fast = c.mel_fast; p.deriv = deriv ? 1 : 0;
-    p.window = c.window; p.tws = c.tws; p.mel_prog = c.mel_prog;
+    sept::ExtractParams p = extract_params(c, wav, utt_off, frame_off, item_off, n_utts, hop, n_mels);
+    p.deriv = deriv ? 1 : 0;
     p.out = out;
     const int mode = layout == SEPT_LAYOUT_FRAME_MAJOR ? sept::kModeDbFrameMajor : sept::kModeDbBandMajor;
     SEPT_CUDA(sept::launch_extract(p, n_fft, mode, sms, static_cast<cudaStream_t>(stream)));
@@ -256,10 +288,7 @@ int sept_logmel_bwd_f32(const float* wav, const int64_t* utt_off, const int64_t*
     if (rc) return rc;
     rc = check_extract_shape(n_fft, hop, n_mels, c.n_mel_entries);   // what the forward accepts, the backward takes
     if (rc) return rc;
-    sept::LogmelBwdParams p{};
-    p.wav = wav; p.utt_off = utt_off; p.frame_off = frame_off; p.item_off = item_off; p.n_utts = n_utts; p.n_items = n_items;
-    p.hop = hop; p.n_mels = n_mels; p.n_mel_entries = c.n_mel_entries; p.n_mel_head = c.n_mel_head; p.fast_dn = c.mel_fast;
-    p.window = c.window; p.tws = c.tws; p.mel_prog = c.mel_prog;
+    sept::LogmelBwdParams p = logmel_bwd_params(c, wav, utt_off, frame_off, item_off, n_utts, n_items, hop, n_mels);
     p.grad = grad; p.ws = static_cast<float*>(workspace); p.dwav = dwav;
     SEPT_CUDA(sept::launch_logmel_bwd(p, n_fft, sms, static_cast<cudaStream_t>(stream)));
     return SEPT_OK;
@@ -278,16 +307,11 @@ int sept_mfcc_f32(const float* wav, const int64_t* utt_off, const int64_t* frame
     rc = get_dct(&dct);
     if (rc) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    SEPT_CUDA(cudaMemsetAsync(utt_max, 0, sizeof(int32_t) * 2 * (size_t)n_utts, st));
-    sept::ExtractParams p{};
-    p.wav = wav; p.utt_off = utt_off; p.frame_off = frame_off; p.item_off = item_off;
-    p.n_utts = n_utts; p.hop = 200; p.n_mels = 128; p.n_mel_entries = c.n_mel_entries; p.n_mel_head = c.n_mel_head; p.mel_fast = c.mel_fast; p.total_frames = total_frames;
-    p.window = c.window; p.tws = c.tws; p.mel_prog = c.mel_prog;
-    p.out = scratch; p.utt_max = utt_max;
-    p.frame_utt = reinterpret_cast<int*>(scratch + 2 * (size_t)total_frames * 128);
-    SEPT_CUDA(sept::launch_extract(p, 400, sept::kModeMfccPower, sms, st));
+    int* frame_utt = reinterpret_cast<int*>(scratch + 2 * (size_t)total_frames * 128);
+    rc = launch_mfcc_power(c, sms, wav, utt_off, frame_off, item_off, n_utts, total_frames, scratch, utt_max, frame_utt, st);
+    if (rc) return rc;
     sept::MfccDctParams d{};
-    d.power = scratch; d.utt_max = utt_max; d.frame_utt = p.frame_utt; d.frame_off = frame_off; d.dct = dct; d.n_utts = n_utts;
+    d.power = scratch; d.utt_max = utt_max; d.frame_utt = frame_utt; d.frame_off = frame_off; d.dct = dct; d.n_utts = n_utts;
     d.total_frames = total_frames; d.top_db = 80.0f; d.out = out;
     // Two implementations of the dB + floor + DCT phase, both parity tested.  Default: the packed-FMA kernel (mfcc_dct.cu,
     // 125 us per audio-hour).  SEPT_MFCC_DCT=tc selects the tcgen05 / tensor-memory kernel (mfcc_tc.cu, 3 x TF32 split,
@@ -320,23 +344,15 @@ int sept_mfcc_bwd_f32(const float* wav, const int64_t* utt_off, const int64_t* f
     const sept::MfccBwdLayout l = sept::mfcc_bwd_layout(n_utts, total_frames, n_items);
     unsigned char* ws = static_cast<unsigned char*>(workspace);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    // the forward's power launch (sept_mfcc_f32), deterministic: the same power, maxima and frame map bit for bit
+    float* power = reinterpret_cast<float*>(ws + l.power);
     int32_t* utt_max = reinterpret_cast<int32_t*>(ws + l.utt_max);
-    SEPT_CUDA(cudaMemsetAsync(utt_max, 0, sizeof(int32_t) * 2 * (size_t)n_utts, st));
-    sept::ExtractParams p{};
-    p.wav = wav; p.utt_off = utt_off; p.frame_off = frame_off; p.item_off = item_off;
-    p.n_utts = n_utts; p.hop = 200; p.n_mels = 128; p.n_mel_entries = c.n_mel_entries; p.n_mel_head = c.n_mel_head; p.mel_fast = c.mel_fast; p.total_frames = total_frames;
-    p.window = c.window; p.tws = c.tws; p.mel_prog = c.mel_prog;
-    p.out = reinterpret_cast<float*>(ws + l.power); p.utt_max = utt_max;
-    p.frame_utt = reinterpret_cast<int*>(ws + l.frame_utt);
-    SEPT_CUDA(sept::launch_extract(p, 400, sept::kModeMfccPower, sms, st));
+    int* frame_utt = reinterpret_cast<int*>(ws + l.frame_utt);
+    rc = launch_mfcc_power(c, sms, wav, utt_off, frame_off, item_off, n_utts, total_frames, power, utt_max, frame_utt, st);
+    if (rc) return rc;
     sept::MfccBwdParams b{};
-    sept::LogmelBwdParams& f = b.frames;
-    f.wav = wav; f.utt_off = utt_off; f.frame_off = frame_off; f.item_off = item_off; f.n_utts = n_utts; f.n_items = n_items;
-    f.hop = 200; f.n_mels = 128; f.n_mel_entries = c.n_mel_entries; f.n_mel_head = c.n_mel_head; f.fast_dn = c.mel_fast;
-    f.window = c.window; f.tws = c.tws; f.mel_prog = c.mel_prog;
-    b.grad = grad; b.dct = dct; b.frame_utt = p.frame_utt; b.utt_max = utt_max; b.total_frames = total_frames;
-    b.power = p.out; b.part = reinterpret_cast<float*>(ws + l.part); b.amask = reinterpret_cast<uint32_t*>(ws + l.amask);
+    b.frames = logmel_bwd_params(c, wav, utt_off, frame_off, item_off, n_utts, n_items, 200, 128);
+    b.grad = grad; b.dct = dct; b.frame_utt = frame_utt; b.utt_max = utt_max; b.total_frames = total_frames;
+    b.power = power; b.part = reinterpret_cast<float*>(ws + l.part); b.amask = reinterpret_cast<uint32_t*>(ws + l.amask);
     b.rows0 = reinterpret_cast<float*>(ws + l.rows0); b.rows1 = reinterpret_cast<float*>(ws + l.rows1); b.dwav = dwav;
     SEPT_CUDA(sept::launch_mfcc_bwd(b, sms, st));
     return SEPT_OK;

@@ -1,9 +1,10 @@
 // Waveform gradient of the frame-major log-mel (sm_100a): d(sum G * logmel) / d wav.  Maths and per-lane phases in
 // extract_bwd.cuh.
 //
-//   logmel_bwd_frames_kernel<R>  persistent, one CTA per SM, one warp per item: recompute spectrum, power and mel power
-//                                with the forward's phase functions, form dM and dP, inverse split, inverse prime-factor
-//                                transform, window, overlap-add of the item's frames -> one workspace row per item
+//   logmel_bwd_frames_kernel<R, DERIV>  persistent, one CTA per SM, one warp per item: recompute spectrum, power and mel
+//                                power with the forward's phase functions, form dM and dP, inverse split, inverse
+//                                prime-factor transform, window, overlap-add of the item's frames -> one workspace row per
+//                                item.  DERIV = 1 stages np.gradient(x) instead of x (the MFCC backward, mfcc_bwd.cu).
 //   logmel_bwd_gather_kernel<R>  one thread per waveform sample: sums the rows covering it (and its reflect mirrors) in
 //                                item order and writes dwav once.  No atomics: the result is bit-deterministic and an
 //                                utterance's gradient does not depend on the rest of the batch.
@@ -15,7 +16,7 @@
 
 namespace sept {
 
-template <int R>
+template <int R, int DERIV = 0>
 __global__ void __launch_bounds__(kBwdWarps * 32, 1) logmel_bwd_frames_kernel(const LogmelBwdParams prm) {
     using G = Geo<R>;
     using B = Bwd<G>;
@@ -50,7 +51,7 @@ __global__ void __launch_bounds__(kBwdWarps * 32, 1) logmel_bwd_frames_kernel(co
         const int T = (int)(__ldg(prm.frame_off + u + 1) - f0);
         const int t0 = (int)(item - __ldg(prm.item_off + u)) * G::FPW;
         __syncwarp();                                            // previous item's frame tile reads are done
-        stage_item<G>(lane, prm.wav + s0, n, t0, hop, 0, stage);
+        stage_item<G>(lane, prm.wav + s0, n, t0, hop, DERIV, stage);
         __syncwarp();
         pass1<G, false>(lane, stage, hop, WinShared{win2}, Y);
         __syncwarp();
@@ -90,14 +91,10 @@ __global__ void __launch_bounds__(256) logmel_bwd_gather_kernel(const LogmelBwdP
     const int row = Bwd<G>::row_floats(prm.hop);
     const long long first = __ldg(prm.utt_off), last = __ldg(prm.utt_off + prm.n_utts);
     for (long long i = first + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < last; i += (long long)gridDim.x * blockDim.x) {
-        int lo_ = 0, hi_ = prm.n_utts - 1;                       // utterance of sample i
-        while (lo_ < hi_) {
-            const int mid = (lo_ + hi_) >> 1;
-            if (__ldg(prm.utt_off + mid + 1) > i) hi_ = mid; else lo_ = mid + 1;
-        }
-        const long long s0 = __ldg(prm.utt_off + lo_);
-        const int n = (int)(__ldg(prm.utt_off + lo_ + 1) - s0);
-        const int i0 = __ldg(prm.item_off + lo_), n_items = __ldg(prm.item_off + lo_ + 1) - i0;
+        const int u = bwd_find_utt(prm.utt_off, prm.n_utts, i);
+        const long long s0 = __ldg(prm.utt_off + u);
+        const int n = (int)(__ldg(prm.utt_off + u + 1) - s0);
+        const int i0 = __ldg(prm.item_off + u), n_items = __ldg(prm.item_off + u + 1) - i0;
         prm.dwav[i] = bwd_gather<G>(prm.ws + (long long)i0 * row, row, n_items, n, (int)(i - s0), prm.hop);
     }
 }
@@ -112,8 +109,9 @@ static int bwd_warps(int hop, int n_mels, int n_mel_entries) {
     return fit < kBwdWarps ? fit : kBwdWarps;
 }
 
-template <int R>
-static cudaError_t launch_frames(LogmelBwdFramesKernel kernel, const LogmelBwdParams& prm, int sms, cudaStream_t stream) {
+template <int R, int DERIV>
+static cudaError_t launch_frames(const LogmelBwdParams& prm, int sms, cudaStream_t stream) {
+    const auto kernel = logmel_bwd_frames_kernel<R, DERIV>;
     const int warps = bwd_warps<R>(prm.hop, prm.n_mels, prm.n_mel_entries);
     if (warps == 0) return cudaErrorInvalidConfiguration;
     const size_t smem = (size_t)bwd_const_bytes(R, prm.n_mel_entries) +
@@ -126,7 +124,7 @@ static cudaError_t launch_frames(LogmelBwdFramesKernel kernel, const LogmelBwdPa
 
 template <int R>
 static cudaError_t launch_r(const LogmelBwdParams& prm, int sms, cudaStream_t stream) {
-    cudaError_t e = launch_frames<R>(logmel_bwd_frames_kernel<R>, prm, sms, stream);
+    cudaError_t e = launch_frames<R, 0>(prm, sms, stream);
     if (e != cudaSuccess) return e;
     logmel_bwd_gather_kernel<R><<<sms * 8, 256, 0, stream>>>(prm);
     return cudaGetLastError();
@@ -141,9 +139,8 @@ cudaError_t launch_logmel_bwd(const LogmelBwdParams& prm, int n_fft, int sms, cu
     return cudaErrorInvalidValue;
 }
 
-cudaError_t launch_logmel_bwd_frames_400(const LogmelBwdParams& prm, LogmelBwdFramesKernel kernel, int sms,
-                                         cudaStream_t stream) {
-    return launch_frames<8>(kernel ? kernel : logmel_bwd_frames_kernel<8>, prm, sms, stream);
+cudaError_t launch_logmel_bwd_frames_400(const LogmelBwdParams& prm, int deriv, int sms, cudaStream_t stream) {
+    return deriv ? launch_frames<8, 1>(prm, sms, stream) : launch_frames<8, 0>(prm, sms, stream);
 }
 
 size_t logmel_bwd_workspace_bytes(int n_fft, int hop, long long n_items) {

@@ -35,11 +35,13 @@ constexpr float kDbPerNeper = 4.34294481903251828f;      // 10 / ln 10: d(10 log
 constexpr int kBwdWarps = 8;     // warps per CTA of the frame pass at most (shared memory decides: extract_bwd.cu)
 
 #ifdef __CUDACC__                // kernel-side helpers of the frame passes (extract_bwd.cu, mfcc_bwd.cu)
-__device__ __forceinline__ int bwd_find_utt(const int32_t* __restrict__ item_off, int n_utts, long long item) {
+// utterance u with off[u] <= x < off[u + 1] (off: item or sample offsets)
+template <class Off>
+__device__ __forceinline__ int bwd_find_utt(const Off* off, int n_utts, long long x) {
     int lo_ = 0, hi_ = n_utts - 1;
     while (lo_ < hi_) {
         const int mid = (lo_ + hi_) >> 1;
-        if (__ldg(item_off + mid + 1) > item) hi_ = mid; else lo_ = mid + 1;
+        if (__ldg(off + mid + 1) > x) hi_ = mid; else lo_ = mid + 1;
     }
     return lo_;
 }

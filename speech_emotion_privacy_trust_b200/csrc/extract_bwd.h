@@ -28,11 +28,7 @@ struct LogmelBwdParams {
 size_t logmel_bwd_workspace_bytes(int n_fft, int hop, long long n_items);
 cudaError_t launch_logmel_bwd(const LogmelBwdParams& prm, int n_fft, int sms, cudaStream_t stream);
 
-// The frame pass alone at n_fft 400 (rows to prm.ws, no gather), with the shared memory and grid of
-// logmel_bwd_frames_kernel<8>.  kernel: a frame-pass kernel with that layout (mfcc_bwd.cu: its np.gradient copy), or
-// nullptr for logmel_bwd_frames_kernel<8> itself.
-using LogmelBwdFramesKernel = void (*)(const LogmelBwdParams);
-cudaError_t launch_logmel_bwd_frames_400(const LogmelBwdParams& prm, LogmelBwdFramesKernel kernel, int sms,
-                                         cudaStream_t stream);
+// The frame pass alone at n_fft 400 (rows to prm.ws, no gather).  deriv: stage np.gradient(x) instead of x.
+cudaError_t launch_logmel_bwd_frames_400(const LogmelBwdParams& prm, int deriv, int sms, cudaStream_t stream);
 
 }  // namespace sept

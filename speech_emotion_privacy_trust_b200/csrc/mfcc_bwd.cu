@@ -7,8 +7,8 @@
 //                                 per-frame sums of what each stream sends to its floor and per-frame argmax bitmasks
 //   mfcc_bwd_route_kernel         one warp per utterance: adds the per-frame sums in frame order and the argmax counts,
 //                                 then adds R_s / count at the argmax positions
-//   logmel_bwd_frames_kernel<8>   (extract_bwd.cu) the waveform stream on G_0
-//   mfcc_bwd_deriv_frames_kernel  the same frame pass on np.gradient(x) and G_1
+//   logmel_bwd_frames_kernel<8, 0>  (extract_bwd.cu) the waveform stream on G_0
+//   logmel_bwd_frames_kernel<8, 1>  the same frame pass on np.gradient(x) and G_1
 //   mfcc_bwd_gather_kernel        one thread per sample: stream 0's rows at the sample plus the np.gradient adjoint of
 //                                 stream 1's per-sample sums, recomputed at the neighbours; each sample written once
 //
@@ -133,90 +133,15 @@ __global__ void __launch_bounds__(kRouteWarps * 32) mfcc_bwd_route_kernel(const 
     }
 }
 
-// logmel_bwd_frames_kernel<8> (extract_bwd.cu) with the items staged as np.gradient(x).  A copy rather than a shared
-// inline body: sharing it changed the code the compiler made for the n_fft 800 / 1600 log-mel instantiations, whose
-// measured times DESIGN.md quotes.  Same shared-memory layout, launched through launch_logmel_bwd_frames_400.
-__global__ void __launch_bounds__(kBwdWarps * 32, 1) mfcc_bwd_deriv_frames_kernel(const LogmelBwdParams prm) {
-    using G = Geo<8>;
-    using B = Bwd<G>;
-    extern __shared__ __align__(16) unsigned char smem_raw[];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, warps = blockDim.x >> 5;
-    const int hop = prm.hop, n_mels = prm.n_mels;
-
-    mel_step* melp = reinterpret_cast<mel_step*>(smem_raw);
-    f2* win2 = reinterpret_cast<f2*>(melp + prm.n_mel_entries);
-    f2* tws = win2 + G::NC;
-    for (int i = threadIdx.x; i < 13 * G::TWS; i += blockDim.x) tws[i] = reinterpret_cast<const f2*>(prm.tws)[i];
-    for (int i = threadIdx.x; i < prm.n_mel_entries; i += blockDim.x)
-        reinterpret_cast<f4*>(melp)[i] = reinterpret_cast<const f4*>(prm.mel_prog)[i];
-    for (int i = threadIdx.x; i < G::NC; i += blockDim.x) win2[i] = reinterpret_cast<const f2*>(prm.window)[i];
-    __syncthreads();
-
-    float* wbase = reinterpret_cast<float*>(smem_raw + bwd_const_bytes(8, prm.n_mel_entries)) + (size_t)warp * B::warp_floats(hop, n_mels);
-    float* stage = wbase;
-    pk2* Y = reinterpret_cast<pk2*>(stage + G::stage_floats(hop));
-    pk2* P = Y + G::Y_PK2;
-    pk2* U = P + G::PPW * G::PP;
-    pk2* D = reinterpret_cast<pk2*>(reinterpret_cast<float*>(U) + B::ud_floats(n_mels));
-    const mel_step* prog = melp;
-    const int row = B::row_floats(hop), span = G::span(hop);
-
-    long long n_items = __ldg(prm.item_off + prm.n_utts);
-    if (n_items > prm.n_items) n_items = prm.n_items;
-    for (long long item = (long long)blockIdx.x * warps + warp; item < n_items; item += (long long)gridDim.x * warps) {
-        const int u = bwd_find_utt(prm.item_off, prm.n_utts, item);
-        const long long s0 = __ldg(prm.utt_off + u), f0 = __ldg(prm.frame_off + u);
-        const int n = (int)(__ldg(prm.utt_off + u + 1) - s0);
-        const int T = (int)(__ldg(prm.frame_off + u + 1) - f0);
-        const int t0 = (int)(item - __ldg(prm.item_off + u)) * G::FPW;
-        __syncwarp();
-        stage_item<G>(lane, prm.wav + s0, n, t0, hop, 1, stage);           // np.gradient(x), reflect padded
-        __syncwarp();
-        pass1<G, false>(lane, stage, hop, WinShared{win2}, Y);
-        __syncwarp();
-#pragma unroll 1
-        for (int task = lane; task < G::P2_TASKS; task += 32) pass2_row<G>(task, Y);
-        __syncwarp();
-        bwd_row0_copy<G>(lane, Y);
-        __syncwarp();
-        bwd_split<G>(lane, Y, tws, P);
-        __syncwarp();
-        bwd_mel_sums<G>(lane, P, prog, prm.n_mel_head, n_mels, prm.fast_dn != 0, U, D);
-        __syncwarp();
-        bwd_dmel<G>(lane, U, D, prm.grad + f0 * n_mels, T, t0, n_mels, P);
-        __syncwarp();
-        bwd_dpower<G>(lane, U, prog, prm.n_mel_head, n_mels, P);
-        __syncwarp();
-        bwd_unsplit<G>(lane, Y, P, tws);
-        __syncwarp();
-#pragma unroll 1
-        for (int task = lane; task < G::P2_TASKS; task += 32) pass2_row<G>(task, Y);
-        __syncwarp();
-        {
-            pk2 gr[25], gi[25];
-            bwd_pass1_load<G>(lane, Y, win2, gr, gi);
-            __syncwarp();
-            bwd_pass1_store<G>(lane, reinterpret_cast<float*>(Y), gr, gi);
-        }
-        __syncwarp();
-        float* out = prm.ws + item * row;
-        for (int j = lane; j < span; j += 32) out[j] = bwd_ola<G>(j, reinterpret_cast<const float*>(Y), hop);
-    }
-}
-
 __global__ void __launch_bounds__(256) mfcc_bwd_gather_kernel(const MfccBwdParams prm) {
     const LogmelBwdParams& fp = prm.frames;
     const int row = Bwd<Geo<8>>::row_floats(200);
     const long long first = __ldg(fp.utt_off), last = __ldg(fp.utt_off + fp.n_utts);
     for (long long i = first + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < last; i += (long long)gridDim.x * blockDim.x) {
-        int lo_ = 0, hi_ = fp.n_utts - 1;                        // utterance of sample i
-        while (lo_ < hi_) {
-            const int mid = (lo_ + hi_) >> 1;
-            if (__ldg(fp.utt_off + mid + 1) > i) hi_ = mid; else lo_ = mid + 1;
-        }
-        const long long s0 = __ldg(fp.utt_off + lo_);
-        const int n = (int)(__ldg(fp.utt_off + lo_ + 1) - s0);
-        const int i0 = __ldg(fp.item_off + lo_), n_items = __ldg(fp.item_off + lo_ + 1) - i0;
+        const int u = bwd_find_utt(fp.utt_off, fp.n_utts, i);
+        const long long s0 = __ldg(fp.utt_off + u);
+        const int n = (int)(__ldg(fp.utt_off + u + 1) - s0);
+        const int i0 = __ldg(fp.item_off + u), n_items = __ldg(fp.item_off + u + 1) - i0;
         prm.dwav[i] = mfcc_bwd_gather(prm.rows0 + (long long)i0 * row, prm.rows1 + (long long)i0 * row, row, n_items, n,
                                       (int)(i - s0));
     }
@@ -252,10 +177,10 @@ cudaError_t launch_mfcc_bwd(const MfccBwdParams& prm, int sms, cudaStream_t stre
     LogmelBwdParams fp = prm.frames;
     fp.grad = prm.power;
     fp.ws = prm.rows0;
-    if ((e = launch_logmel_bwd_frames_400(fp, nullptr, sms, stream)) != cudaSuccess) return e;
+    if ((e = launch_logmel_bwd_frames_400(fp, 0, sms, stream)) != cudaSuccess) return e;
     fp.grad = prm.power + prm.total_frames * kMfccBands;
     fp.ws = prm.rows1;
-    if ((e = launch_logmel_bwd_frames_400(fp, mfcc_bwd_deriv_frames_kernel, sms, stream)) != cudaSuccess) return e;
+    if ((e = launch_logmel_bwd_frames_400(fp, 1, sms, stream)) != cudaSuccess) return e;
     mfcc_bwd_gather_kernel<<<sms * 8, 256, 0, stream>>>(prm);
     return cudaGetLastError();
 }

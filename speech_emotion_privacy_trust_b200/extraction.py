@@ -25,6 +25,7 @@ class Layout:
     frame_off_host: np.ndarray       # int64 [n+1]
     frame_off: torch.Tensor          # device int64 [n+1]
     item_off: torch.Tensor           # device int32 [n+1]
+    n_items: int = 0                 # item_off[n]: work items of the batch (0 with the all-zero item_off of frame layouts)
 
     @property
     def total_frames(self) -> int:
@@ -69,7 +70,8 @@ class RaggedAudio:
             _lib.check(_lib.lib().sept_extract_layout(self.utt_off_host.ctypes.data, n, n_fft, hop,
                                                       frame_off.ctypes.data, item_off.ctypes.data))
             dev = self.wav.device
-            self._layouts[key] = Layout(frame_off, torch.from_numpy(frame_off).to(dev), torch.from_numpy(item_off).to(dev))
+            self._layouts[key] = Layout(frame_off, torch.from_numpy(frame_off).to(dev), torch.from_numpy(item_off).to(dev),
+                                        int(item_off[-1]))
         return self._layouts[key]
 
 
@@ -125,8 +127,6 @@ class LogMelFunction(torch.autograd.Function):
     def forward(ctx, wav, batch, n_fft, n_mels, hop):
         out, lay = logmel(batch, n_fft, n_mels, hop)
         ctx.save_for_backward(wav)
-        fpw = _lib.lib().sept_frames_per_item(n_fft)
-        ctx.n_items = int((-(-np.diff(lay.frame_off_host) // fpw)).sum())   # item_off[n_utts], from host data
         ctx.batch, ctx.lay, ctx.shape = batch, lay, (n_fft, n_mels, hop)
         return out
 
@@ -136,15 +136,14 @@ class LogMelFunction(torch.autograd.Function):
         (wav,) = ctx.saved_tensors
         batch, lay = ctx.batch, ctx.lay
         n_fft, n_mels, hop = ctx.shape
-        n_items = ctx.n_items
         lib = _lib.lib()
         dwav = torch.zeros_like(wav)                              # samples outside every utterance get no gradient
-        ws = torch.empty(max(1, lib.sept_logmel_bwd_workspace_bytes(n_fft, hop, n_items)), dtype=torch.uint8,
+        ws = torch.empty(max(1, lib.sept_logmel_bwd_workspace_bytes(n_fft, hop, lay.n_items)), dtype=torch.uint8,
                          device=wav.device)
         grad = grad.contiguous()
         with torch.cuda.device(wav.device):
             _lib.check(lib.sept_logmel_bwd_f32(wav.data_ptr(), batch.utt_off.data_ptr(), lay.frame_off.data_ptr(),
-                                               lay.item_off.data_ptr(), batch.n_utts, n_items, n_fft, hop, n_mels,
+                                               lay.item_off.data_ptr(), batch.n_utts, lay.n_items, n_fft, hop, n_mels,
                                                grad.data_ptr(), ws.data_ptr(), dwav.data_ptr(), _stream(wav.device)))
         return dwav, None, None, None, None
 
@@ -190,8 +189,6 @@ class MfccFunction(torch.autograd.Function):
     def forward(ctx, wav, batch):
         out, lay = mfcc(batch)
         ctx.save_for_backward(wav)
-        fpw = _lib.lib().sept_frames_per_item(N_FFT_MFCC)
-        ctx.n_items = int((-(-np.diff(lay.frame_off_host) // fpw)).sum())   # item_off[n_utts], from host data
         ctx.batch, ctx.lay = batch, lay
         return out
 
@@ -199,15 +196,15 @@ class MfccFunction(torch.autograd.Function):
     @once_differentiable
     def backward(ctx, grad):
         (wav,) = ctx.saved_tensors
-        batch, lay, n_items = ctx.batch, ctx.lay, ctx.n_items
+        batch, lay = ctx.batch, ctx.lay
         lib = _lib.lib()
         dwav = torch.zeros_like(wav)                              # samples outside every utterance get no gradient
-        ws = torch.empty(max(1, lib.sept_mfcc_bwd_workspace_bytes(batch.n_utts, lay.total_frames, n_items)),
+        ws = torch.empty(max(1, lib.sept_mfcc_bwd_workspace_bytes(batch.n_utts, lay.total_frames, lay.n_items)),
                          dtype=torch.uint8, device=wav.device)
         grad = grad.contiguous()
         with torch.cuda.device(wav.device):
             _lib.check(lib.sept_mfcc_bwd_f32(wav.data_ptr(), batch.utt_off.data_ptr(), lay.frame_off.data_ptr(),
-                                             lay.item_off.data_ptr(), batch.n_utts, lay.total_frames, n_items,
+                                             lay.item_off.data_ptr(), batch.n_utts, lay.total_frames, lay.n_items,
                                              grad.data_ptr(), ws.data_ptr(), dwav.data_ptr(), _stream(wav.device)))
         return dwav, None
 

@@ -1,7 +1,7 @@
 // Host emulation of the MFCC backward (TEST CODE, not a fallback) for ONE utterance: the mel power of both streams with
 // the frame pass's own recompute (extract_bwd.cuh), the head functions of csrc/mfcc_bwd.cuh per (frame, band), the
 // route (floor totals, argmax share), the frame pass of the waveform and of the np.gradient stream (deriv staging) lane
-// by lane as in extract_bwd.cu / mfcc_bwd.cu, then the gather with the np.gradient adjoint sample by sample.
+// by lane (bwd_frame_pass.h), then the gather with the np.gradient adjoint sample by sample.
 //   mfcc_bwd grad <wav.f32> <gbar.f32 (120, T)> <dwav.f32>
 //   mfcc_bwd adjoint <x.f32> <v.f32> <out.f32>     out = [np.gradient(x) as staged (n), its adjoint applied to v (n)]
 #include <cstdio>
@@ -9,8 +9,8 @@
 #include <cstring>
 #include <vector>
 
+#include "bwd_frame_pass.h"
 #include "mfcc_bwd.cuh"
-#include "tables.h"
 
 using namespace sept;
 using G = Geo<8>;
@@ -18,83 +18,11 @@ using B = Bwd<G>;
 
 static constexpr int kHop = 200, kMels = 128;
 
-struct Frames {
-    std::vector<float> win, tws;
-    MelProgram prog;
-    const mel_step* mprog;
-    bool fast_dn;
-    std::vector<float> stage;
-    std::vector<pk4> Ybuf, Pbuf;
-    std::vector<pk2> U, D;
-    pk2 *Y, *P;
-    Frames() {
-        win = make_hann_periodic(400);
-        tws = make_split_twiddles(400);
-        make_mel_program(400, kMels, 16000, prog);
-        mprog = reinterpret_cast<const mel_step*>(prog.entries.data());
-        fast_dn = prog.round_steps.size() == 4 && prog.n_head == FastMel<8>::head && prog.round_steps[0] == FastMel<8>::s0 &&
-                  prog.round_steps[1] == FastMel<8>::s1 && prog.round_steps[2] == FastMel<8>::s2 &&
-                  prog.round_steps[3] == FastMel<8>::s3;
-        stage.assign(G::stage_floats(kHop), 0.f);
-        Ybuf.resize(G::Y_PK4 + 1);
-        Pbuf.resize((G::PPW * G::PP) / 2 + 1);
-        U.resize((size_t)G::PPW * B::ums(kMels));
-        D.resize((size_t)G::PPW * B::ums(kMels));
-        Y = reinterpret_cast<pk2*>(Ybuf.data());
-        P = reinterpret_cast<pk2*>(Pbuf.data());
-    }
-    const f2* win2() const { return reinterpret_cast<const f2*>(win.data()); }
-    const f2* tw2() const { return reinterpret_cast<const f2*>(tws.data()); }
-    // spectrum, split and mel sums of one item (the first half of the frame pass)
-    void front(const std::vector<float>& wav, int t0, int deriv) {
-        const int n = (int)wav.size();
-        for (int lane = 0; lane < 32; ++lane) stage_item<G>(lane, wav.data(), n, t0, kHop, deriv, stage.data());
-        for (int lane = 0; lane < 32; ++lane) pass1<G, false>(lane, stage.data(), kHop, WinShared{win2()}, Y);
-        for (int task = 0; task < G::P2_TASKS; ++task) pass2_row<G>(task, Y);
-        for (int lane = 0; lane < 32; ++lane) bwd_row0_copy<G>(lane, Y);
-        for (int lane = 0; lane < 32; ++lane) bwd_split<G>(lane, Y, tw2(), P);
-        for (int lane = 0; lane < 32; ++lane) bwd_mel_sums<G>(lane, P, mprog, prog.n_head, kMels, fast_dn, U.data(), D.data());
-    }
-    // mel power (T, 128) of the stream
-    std::vector<float> power(const std::vector<float>& wav, int T, int deriv) {
-        std::vector<float> M((size_t)T * kMels, 0.f);
-        const int ums = kMels + 1;
-        for (int t0 = 0; t0 < T; t0 += G::FPW) {
-            front(wav, t0, deriv);
-            for (int p = 0; p < G::PPW; ++p)
-                for (int m = 0; m < kMels; ++m) {
-                    const pk2 acc = U[p * ums + m] + D[p * ums + m + 1];
-                    if (t0 + 2 * p < T) M[(size_t)(t0 + 2 * p) * kMels + m] = lo(acc);
-                    if (t0 + 2 * p + 1 < T) M[(size_t)(t0 + 2 * p + 1) * kMels + m] = hi(acc);
-                }
-        }
-        return M;
-    }
-    // the whole frame pass: span rows of every item for dB gradient grad (T, 128)
-    std::vector<float> rows(const std::vector<float>& wav, int T, int deriv, const std::vector<float>& grad) {
-        const int n_items = (T + G::FPW - 1) / G::FPW, row = B::row_floats(kHop);
-        std::vector<float> ws((size_t)n_items * row, 0.f);
-        static pk2 gr[32][25], gi[32][25];
-        for (int it = 0; it < n_items; ++it) {
-            const int t0 = it * G::FPW;
-            front(wav, t0, deriv);
-            for (int lane = 0; lane < 32; ++lane) bwd_dmel<G>(lane, U.data(), D.data(), grad.data(), T, t0, kMels, P);
-            for (int lane = 0; lane < 32; ++lane) bwd_dpower<G>(lane, U.data(), mprog, prog.n_head, kMels, P);
-            for (int lane = 0; lane < 32; ++lane) bwd_unsplit<G>(lane, Y, P, tw2());
-            for (int task = 0; task < G::P2_TASKS; ++task) pass2_row<G>(task, Y);
-            for (int lane = 0; lane < 32; ++lane) bwd_pass1_load<G>(lane, Y, win2(), gr[lane], gi[lane]);
-            for (int lane = 0; lane < 32; ++lane) bwd_pass1_store<G>(lane, reinterpret_cast<float*>(Y), gr[lane], gi[lane]);
-            for (int j = 0; j < G::span(kHop); ++j) ws[(size_t)it * row + j] = bwd_ola<G>(j, reinterpret_cast<const float*>(Y), kHop);
-        }
-        return ws;
-    }
-};
-
 static unsigned bits(float x) { unsigned u; std::memcpy(&u, &x, 4); return u; }
 
 static std::vector<float> mfcc_grad(const std::vector<float>& wav, const std::vector<float>& gbar) {
     const int n = (int)wav.size(), T = 1 + n / kHop, n_items = (T + G::FPW - 1) / G::FPW;
-    Frames fr;
+    BwdFramePass<8> fr(kHop, kMels);
     const std::vector<float> M0 = fr.power(wav, T, 0), M1 = fr.power(wav, T, 1);
     float max0 = 0.f, max1 = 0.f;                           // the forward's atomicMax over non-negative bits
     for (size_t i = 0; i < M0.size(); ++i) { max0 = M0[i] > max0 ? M0[i] : max0; max1 = M1[i] > max1 ? M1[i] : max1; }
