@@ -313,12 +313,7 @@ int sept_mfcc_f32(const float* wav, const int64_t* utt_off, const int64_t* frame
     sept::MfccDctParams d{};
     d.power = scratch; d.utt_max = utt_max; d.frame_utt = frame_utt; d.frame_off = frame_off; d.dct = dct; d.n_utts = n_utts;
     d.total_frames = total_frames; d.top_db = 80.0f; d.out = out;
-    // Two implementations of the dB + floor + DCT phase, both parity tested.  Default: the packed-FMA kernel (mfcc_dct.cu,
-    // 125 us per audio-hour).  SEPT_MFCC_DCT=tc selects the tcgen05 / tensor-memory kernel (mfcc_tc.cu, 3 x TF32 split,
-    // 197 us): its contraction takes 11 us, the rest is feeding it (DESIGN.md 3.2).  Read per call: tests flip it.
-    const char* which = getenv("SEPT_MFCC_DCT");
-    if (which && which[0] == 't') SEPT_CUDA(sept::launch_mfcc_dct_tc(d, sms, st));
-    else SEPT_CUDA(sept::launch_mfcc_dct(d, st));
+    SEPT_CUDA(sept::launch_mfcc_dct(d, st));
     return SEPT_OK;
 }
 

@@ -6,13 +6,12 @@
 //                             and the finished features.  FAST (the reference's 128-band filterbank): the lane-constant
 //                             tables -- window samples, split twiddles, mel program -- live in tensor memory (tmem.cuh)
 //                             and the mel phase is unrolled; otherwise they are read from shared memory.
-//   (the second phase of MFCC -- per-utterance top_db floor + ortho DCT-II -- lives in mfcc_dct.cu / mfcc_tc.cu)
+//   (the second phase of MFCC -- per-utterance top_db floor + ortho DCT-II -- lives in mfcc_dct.cu)
 //
 // Replaces torchaudio MelSpectrogram/AmplitudeToDB/MFCC as called by
 // feature_extraction/audio_feature_extraction.py:15-46 of the reference.
 #include <cuda_runtime.h>
 #include <cstdint>
-#include <cstdlib>
 #include <type_traits>
 
 #include "extract.h"
@@ -55,14 +54,6 @@ __device__ __forceinline__ void cp_async_f32(float* smem_dst, const float* gmem_
 }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
-
-// ---- optional per-phase cycle counters (diagnostic builds only: -DSEPT_PHASE_CLOCKS, tools/phase_clocks.py) ----------
-#ifdef SEPT_PHASE_CLOCKS
-__device__ unsigned long long g_phase_clk[16];
-#define SEPT_TICK(i) do { const long long now_ = clock64(); if (lane == 0) atomicAdd(&g_phase_clk[i], (unsigned long long)(now_ - tick_last)); tick_last = now_; } while (0)
-#else
-#define SEPT_TICK(i) do { } while (0)
-#endif
 
 struct ItemRef {
     const float* wav;      // utterance start
@@ -379,9 +370,6 @@ __global__ void __launch_bounds__(ExtractWarps<R>::value * 32, 1) extract_kernel
     }
 
     constexpr int n_streams = (MODE == kModeMfccPower) ? 2 : 1;
-#ifdef SEPT_PHASE_CLOCKS
-    long long tick_last = clock64();
-#endif
     for (; item < end; item = kDynamicItems ? item : item + kExtractWarps) {     // dynamic: advanced at the end of the body
         int item_next = end;
 #pragma unroll 1
@@ -401,7 +389,6 @@ __global__ void __launch_bounds__(ExtractWarps<R>::value * 32, 1) extract_kernel
                     stage_item<G>(lane, cur.wav, cur.n, cur.t0, hop, deriv, stage);   // edge items: the stage already holds the stream
                     __syncwarp();
                 }
-                SEPT_TICK(0);
                 const bool diff = cur.interior && deriv != 0;
                 if constexpr (FAST) {
                     WinRegs win;
@@ -422,7 +409,6 @@ __global__ void __launch_bounds__(ExtractWarps<R>::value * 32, 1) extract_kernel
                 };
                 if (cur.interior) {
                     if (stream == 0) { cp_async_wait_all(); __syncwarp(); }
-                    SEPT_TICK(0);
                     if (deriv) run_pass1(std::true_type{});
                     else run_pass1(std::false_type{});
                 } else {
@@ -432,9 +418,7 @@ __global__ void __launch_bounds__(ExtractWarps<R>::value * 32, 1) extract_kernel
                     run_pass1(std::false_type{});
                 }
             }
-            SEPT_TICK(1);
             __syncwarp();                                        // stage is free, Y is complete
-            SEPT_TICK(2);
 
             ItemRef nxt = cur;
             if constexpr (kDynamicItems) {
@@ -450,7 +434,6 @@ __global__ void __launch_bounds__(ExtractWarps<R>::value * 32, 1) extract_kernel
                 if (nxt.interior) prefetch(nxt);                 // overlaps pass 2, split and mel of this item
             }
 
-            SEPT_TICK(3);
             if constexpr (R <= 16) {
                 // fused pass 2 + real split + power: rows j and 25-j stay in registers; the tile is overwritten by P only
                 // after every lane has loaded its rows
@@ -474,12 +457,9 @@ __global__ void __launch_bounds__(ExtractWarps<R>::value * 32, 1) extract_kernel
                         TwShared tw{tws + j * G::TWS};
                         pass2_split<G>(p, j, Y, tw, pu, pv);
                     }
-                    SEPT_TICK(4);
                     __syncwarp();
-                    SEPT_TICK(5);
                     if (G::ps_task(lane, r, p, j)) pass2_split_store<G>(p, j, P, pu, pv);
                 }
-                SEPT_TICK(6);
             } else {
 #pragma unroll 1
                 for (int task = lane; task < G::P2_TASKS; task += 32) pass2_row<G>(task, Y);
@@ -500,7 +480,6 @@ __global__ void __launch_bounds__(ExtractWarps<R>::value * 32, 1) extract_kernel
                 split_store_all<G>(lane, P, a, b, on0);
             }
             __syncwarp();
-            SEPT_TICK(7);
 
             // ---- mel bands (lane = band, all frame pairs of the item) + log + store --------------------------
             {
@@ -508,9 +487,7 @@ __global__ void __launch_bounds__(ExtractWarps<R>::value * 32, 1) extract_kernel
                 if constexpr (FAST) mel_fast<G, MODE>(lane, P, taddr, prm, job);
                 else mel_rounds<G, MODE>(lane, P, melp, n_mels, prm, job);
             }
-            SEPT_TICK(8);
             __syncwarp();                                        // P reads done before the next pass 1 overwrites Y
-            SEPT_TICK(9);
             if (stream == n_streams - 1) cur = nxt;
         }
         if constexpr (kDynamicItems) item = item_next;
@@ -526,20 +503,13 @@ __global__ void __launch_bounds__(ExtractWarps<R>::value * 32, 1) extract_kernel
 // ---- host launchers ----------------------------------------------------------------------------------------
 constexpr size_t kMaxSmem = 232448 - 64;  // 227 KB opt-in limit per CTA minus the static shared memory (TMEM base slot)
 
-// tuning knob (bench experiments only): SEPT_EXTRACT_WARPS lowers the warp count (occupancy-scaling measurements)
-static int warp_cap(int r_max) {
-    static const int env = [] { const char* e = getenv("SEPT_EXTRACT_WARPS"); return e ? atoi(e) : 0; }();
-    return (env > 0 && env < r_max) ? env : r_max;
-}
-
 template <int R>
 static int extract_warps(int hop, int n_mel_entries) {            // warps whose tiles fit beside the constants
     using G = Geo<R>;
     const size_t cb = (size_t)extract_const_bytes(R, n_mel_entries), wb = G::stage_floats(hop) * 4 + G::Y_PK4 * 16;
     if (cb + wb > kMaxSmem) return 0;
     const int fit = (int)((kMaxSmem - cb) / wb);
-    const int cap = warp_cap(ExtractWarps<R>::value);
-    return fit < cap ? fit : cap;
+    return fit < ExtractWarps<R>::value ? fit : ExtractWarps<R>::value;
 }
 
 template <int R>
@@ -615,13 +585,3 @@ size_t extract_smem_bytes_for(int n_fft, int hop, int n_mel_entries) {
 }
 
 }  // namespace sept
-
-#ifdef SEPT_PHASE_CLOCKS
-extern "C" int sept_debug_phase_clocks(unsigned long long* out_host, int reset) {
-    unsigned long long zero[16] = {0};
-    cudaDeviceSynchronize();
-    if (out_host && cudaMemcpyFromSymbol(out_host, sept::g_phase_clk, sizeof(zero)) != cudaSuccess) return -1;
-    if (reset && cudaMemcpyToSymbol(sept::g_phase_clk, zero, sizeof(zero)) != cudaSuccess) return -1;
-    return 0;
-}
-#endif

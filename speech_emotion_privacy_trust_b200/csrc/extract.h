@@ -57,7 +57,6 @@ size_t extract_smem_bytes_for(int n_fft, int hop, int n_mel_entries);
 int extract_frames_per_item(int n_fft);
 // true when a 128-band program with these step counts may run the unrolled mel path
 bool extract_mel_fast_ok(int n_fft, int n_mels, int n_head, const int* round_steps, int n_rounds);
-cudaError_t launch_mfcc_dct(const MfccDctParams& prm, cudaStream_t stream);        // FMA version (extract.cu)
-cudaError_t launch_mfcc_dct_tc(const MfccDctParams& prm, int sms, cudaStream_t stream);   // tcgen05 version (mfcc_tc.cu)
+cudaError_t launch_mfcc_dct(const MfccDctParams& prm, cudaStream_t stream);        // dB + top_db floor + DCT (mfcc_dct.cu)
 
 }  // namespace sept

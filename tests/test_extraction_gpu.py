@@ -68,15 +68,7 @@ def test_logmel_golden_both_layouts(ex, golden_extraction, key, n_fft):
             assert np.max(np.abs(got_bm - exact)) < 0.05
 
 
-@pytest.fixture(params=["fma", "tc"])
-def dct_path(request, monkeypatch):
-    """Both implementations of MFCC's dB + floor + DCT phase: the packed-FMA kernel (default) and the tcgen05 / tensor-memory
-    kernel (csrc/mfcc_tc.cu, 3 x TF32 split); the C ABI reads SEPT_MFCC_DCT on every call."""
-    monkeypatch.setenv("SEPT_MFCC_DCT", request.param)
-    return request.param
-
-
-def test_mfcc_golden(ex, gold_batch, golden_extraction, dct_path):
+def test_mfcc_golden(ex, gold_batch, golden_extraction):
     batch, waves = gold_batch
     flat, lay = ex.mfcc(batch)
     blocks = ex.split_band_major(flat, lay, 120)
@@ -169,7 +161,7 @@ def test_dropin_callables_keep_reference_types(golden_extraction):
         afe.mel_spectrogram(torch.zeros(1, 300), n_fft=800)
 
 
-def test_corpus_scale_properties(ex, monkeypatch):
+def test_corpus_scale_properties(ex):
     """Sizes the oracle cannot cover in seconds: size-independent properties on a 600-utterance, ~1-audio-hour batch."""
     from speech_emotion_privacy_trust_b200 import synth
     wav, off = synth.corpus(600, seed=1234)
@@ -200,12 +192,6 @@ def test_corpus_scale_properties(ex, monkeypatch):
     blk = ex.split_band_major(m, mlay, 120)[u].cpu().numpy()
     refm = restate.mfcc(wav[off[u]:off[u + 1]][None], dtype=np.float64)[0]
     assert np.max(np.abs(blk - refm)) / np.max(np.abs(refm)) < TOL_MFCC_REL
-    # the tensor-core DCT (many 128-frame tiles per persistent CTA, utterance boundaries inside tiles) against the FMA one
-    monkeypatch.setenv("SEPT_MFCC_DCT", "tc")
-    m_tc, _ = ex.mfcc(batch)
-    assert float((m_tc - m).abs().max()) / float(m.abs().max()) < 2e-5
-    blk = ex.split_band_major(m_tc, mlay, 120)[u].cpu().numpy()
-    assert np.max(np.abs(blk - refm)) / np.max(np.abs(refm)) < TOL_MFCC_REL
 
 
 def test_other_hops_and_mel_counts_fuzz(ex):
@@ -234,7 +220,7 @@ def test_other_hops_and_mel_counts_fuzz(ex):
         ex.logmel(ex.RaggedAudio.from_list([np.zeros(4000, np.float32)]), n_fft=800, hop=161)
 
 
-def test_mfcc_fuzz_vs_oracle(ex, dct_path):
+def test_mfcc_fuzz_vs_oracle(ex):
     """MFCC at the one configuration the C ABI accepts (n_fft 400, hop 200, 128 mels, 40 coefficients, three streams), on
     ragged batches that exercise what is special about it: the per-utterance top_db floor (loud + near-silent halves in
     one utterance, whole utterances at the 1e-10 clamp), frame-count boundaries, the shortest legal utterance."""

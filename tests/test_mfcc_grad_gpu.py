@@ -123,11 +123,8 @@ def test_ragged_batch_covers_edges():
     assert torch.count_nonzero(wav.grad[1000:17000]) > 15000
 
 
-@pytest.mark.parametrize("dct", ["default", "tc"])
-def test_forward_bit_identical_and_backward_deterministic(golden_extraction, monkeypatch, dct):
+def test_forward_bit_identical_and_backward_deterministic(golden_extraction):
     from speech_emotion_privacy_trust_b200 import extraction
-    if dct == "tc":
-        monkeypatch.setenv("SEPT_MFCC_DCT", "tc")
     waves = _speech(golden_extraction)
     batch = _batch(waves)
     plain, _ = extraction.mfcc(batch)

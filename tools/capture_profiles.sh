@@ -12,10 +12,7 @@ ncu --metrics gpu__time_duration.sum --clock-control none --nvtx --nvtx-include 
 python tools/run_features.py 600 > /dev/null 2>&1 && \
 ncu --metrics gpu__time_duration.sum --clock-control none --nvtx --nvtx-include "features/" --csv --log-file $out/launches_${tag}_features_1h.csv \
     python tools/run_features.py 600 > /dev/null 2>&1
-SEPT_MFCC_DCT=tc ncu --metrics gpu__time_duration.sum --clock-control none -k regex:mfcc_dct --csv --log-file $out/launches_${tag}_dct_tc.csv \
-    python tools/run_features.py 600 > /dev/null 2>&1
 ncu --set full --clock-control none --import-source on -k regex:extract_kernel -s 3 -c 1 -o $out/prof_${tag}_800 -f python bench.py --steps 2 --warmup 3 --no-extras > /dev/null 2>&1
 ncu --set full --clock-control none --import-source on -k regex:extract_kernel -s 3 -c 1 -o $out/prof_${tag}_1600 -f python bench.py --steps 2 --warmup 3 --no-extras --n-fft 1600 > /dev/null 2>&1
 ncu --set full --clock-control none --import-source on -k regex:"extract_kernel|mfcc_dct" -s 2 -c 2 -o $out/prof_${tag}_mfcc -f python tools/time_features.py mfcc > /dev/null 2>&1
-SEPT_MFCC_DCT=tc ncu --set full --clock-control none --import-source on -k regex:mfcc_dct -s 1 -c 1 -o $out/prof_${tag}_dct_tc -f python tools/time_features.py mfcc > /dev/null 2>&1
 ls -la $out/*${tag}*
