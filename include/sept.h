@@ -146,6 +146,36 @@ int sept_normalize_windows_f32(const float* feat_dev, const int64_t* frame_off_d
                                const float* stats_dev, const int32_t* win_utt_dev, const int32_t* win_t0_dev,
                                int n_windows, int win_len, int n_feat, int mode, float* out_dev, sept_stream_t stream);
 
+/* Backward of sept_normalize_windows_f32 (utt_win_ptr_dev != NULL) or of sept_normalize_f32 (utt_win_ptr_dev == NULL):
+ * what torch autograd gives for sum(grad * out) through the reference's normalisation, padded rows included.
+ * grad_dev is laid out like the forward's out_dev.  Window mode: window w covers frames win_t0[w] .. +win_len of the
+ * utterance whose CSR list holds it: utt_win_dev[utt_win_ptr[u] .. utt_win_ptr[u+1]) are the windows of utterance u
+ * sorted by (win_t0, window index) (any table works: subsets, any order, repeated windows; win_t0 >= 0).
+ * dfeat_dev (total_frames, n_feat) or NULL: every frame is written (0 for frames in no window).
+ * dstats_dev (n_spk, 5, n_feat) or NULL: the gradient of the statistics (count row 0; znorm fills mean and std, min_max
+ * min and max); needs spk_ptr/spk_utts (the CSR of sept_speaker_stats_f32) and workspace_dev of
+ * sept_normalize_bwd_workspace_bytes(n_utts, n_feat) bytes.  Deterministic (no atomics), no allocation, capturable. */
+size_t sept_normalize_bwd_workspace_bytes(int n_utts, int n_feat);
+int sept_normalize_bwd_f32(const float* feat_dev, const int64_t* frame_off_dev, const int32_t* spk_of_utt_dev,
+                           const float* stats_dev, const int32_t* win_t0_dev, const int32_t* utt_win_ptr_dev,
+                           const int32_t* utt_win_dev, int n_windows, int win_len, int n_utts, int n_feat, int mode,
+                           const float* grad_dev, const int32_t* spk_ptr_dev, const int32_t* spk_utts_dev, int n_spk,
+                           void* workspace_dev, float* dfeat_dev, float* dstats_dev, sept_stream_t stream);
+
+/* Backward of sept_speaker_stats_f32 (what torch autograd gives through the reference's stacked-rows mean, ddof-0 std,
+ * min and max): dfeat = d(sum dstats * stats) / d feat for every frame (written, 0 for frames in no training window).
+ * Row 0 (count) of dstats_dev is ignored.  The min / max gradient goes to the frames equal to it in proportion to their
+ * window multiplicity.  Where the forward's std is exactly 0 (every weighted value of that speaker and feature equal, e.g.
+ * digital silence) no gradient flows through the std (sqrt's derivative there is 0 * inf in torch).  stats_dev is the
+ * forward's result; spk_of_utt_dev [n_utts] the speaker row of each utterance.  workspace_dev holds
+ * sept_speaker_stats_bwd_workspace_bytes(n_utts, n_spk, n_feat) bytes, 16-byte aligned.  Deterministic, no allocation,
+ * capturable. */
+size_t sept_speaker_stats_bwd_workspace_bytes(int n_utts, int n_spk, int n_feat);
+int sept_speaker_stats_bwd_f32(const float* feat_dev, const int64_t* frame_off_dev, const uint8_t* whole_dev, int n_utts,
+                               int n_feat, int win_len, int shift_len, const int32_t* spk_of_utt_dev,
+                               const int32_t* spk_ptr_dev, const int32_t* spk_utts_dev, int n_spk, const float* stats_dev,
+                               const float* dstats_dev, void* workspace_dev, float* dfeat_dev, sept_stream_t stream);
+
 /* ---- cloak noise layer + gradient reversal -------------------------------------------------------------------------
  * Forward of cloak_noise (model/cloak_models.py:41-58): out = x*mask + locs + sigma(rhos) * eps*mask with
  * sigma = (1 + tanh rho)/2 * (max_scale - min_scale) + min_scale, broadcast over the batch.  eps_dev != NULL supplies

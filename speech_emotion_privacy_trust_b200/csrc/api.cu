@@ -18,6 +18,7 @@
 #include "extract_bwd.h"
 #include "mfcc_bwd.h"
 #include "norm.h"
+#include "norm_bwd.h"
 #include "resample.h"
 #include "tables.h"
 
@@ -433,6 +434,63 @@ int sept_normalize_windows_f32(const float* feat, const int64_t* frame_off, cons
     p.feat = feat; p.frame_off = frame_off; p.spk_of_utt = spk_of_utt; p.stats = stats; p.n_feat = n_feat;
     p.mode = mode; p.win_utt = win_utt; p.win_t0 = win_t0; p.n_windows = n_windows; p.win_len = win_len; p.out = out;
     SEPT_CUDA(sept::launch_normalize(p, static_cast<cudaStream_t>(stream)));
+    return SEPT_OK;
+}
+
+size_t sept_normalize_bwd_workspace_bytes(int n_utts, int n_feat) {
+    return n_utts > 0 && n_feat > 0 ? sept::normalize_bwd_workspace_bytes(n_utts, n_feat) : 0;
+}
+
+int sept_normalize_bwd_f32(const float* feat, const int64_t* frame_off, const int32_t* spk_of_utt, const float* stats,
+                           const int32_t* win_t0, const int32_t* utt_win_ptr, const int32_t* utt_win, int n_windows,
+                           int win_len, int n_utts, int n_feat, int mode, const float* grad, const int32_t* spk_ptr,
+                           const int32_t* spk_utts, int n_spk, void* workspace, float* dfeat, float* dstats,
+                           sept_stream_t stream) {
+    const bool window = utt_win_ptr != nullptr;
+    if (!feat || !frame_off || !spk_of_utt || !stats || !grad || (!dfeat && !dstats) || n_utts < 0 || n_feat <= 0 ||
+        (window && (!win_t0 || !utt_win || n_windows < 0 || win_len <= 0)) ||
+        (mode != SEPT_NORM_ZNORM && mode != SEPT_NORM_MINMAX))
+        return fail(SEPT_E_BADARG, "sept_normalize_bwd_f32: bad argument");
+    if (dstats && (!spk_ptr || !spk_utts || n_spk < 0 || !workspace))
+        return fail(SEPT_E_BADARG, "sept_normalize_bwd_f32: dstats needs spk_ptr, spk_utts and the workspace");
+    sept::NormalizeBwdParams p{};
+    p.f.feat = feat; p.f.frame_off = frame_off; p.f.spk_of_utt = spk_of_utt; p.f.stats = stats; p.f.n_feat = n_feat;
+    p.f.mode = mode; p.f.n_utts = n_utts;
+    if (window) {
+        p.f.win_utt = utt_win;                                   // non-null selects the window mode, as in the forward
+        p.f.win_t0 = win_t0; p.f.n_windows = n_windows; p.f.win_len = win_len;
+        p.utt_win_ptr = utt_win_ptr; p.utt_win = utt_win;
+    }
+    p.grad = grad; p.dfeat = dfeat;
+    if (dstats) {
+        p.upart = static_cast<float*>(workspace); p.spk_ptr = spk_ptr; p.spk_utts = spk_utts; p.n_spk = n_spk;
+        p.dstats = dstats;
+    }
+    SEPT_CUDA(sept::launch_normalize_bwd(p, static_cast<cudaStream_t>(stream)));
+    return SEPT_OK;
+}
+
+size_t sept_speaker_stats_bwd_workspace_bytes(int n_utts, int n_spk, int n_feat) {
+    return n_utts >= 0 && n_spk >= 0 && n_feat > 0 ? sept::speaker_stats_bwd_workspace_bytes(n_utts, n_spk, n_feat) : 0;
+}
+
+int sept_speaker_stats_bwd_f32(const float* feat, const int64_t* frame_off, const uint8_t* whole, int n_utts, int n_feat,
+                               int win_len, int shift_len, const int32_t* spk_of_utt, const int32_t* spk_ptr,
+                               const int32_t* spk_utts, int n_spk, const float* stats, const float* dstats,
+                               void* workspace, float* dfeat, sept_stream_t stream) {
+    if (!feat || !frame_off || !spk_of_utt || !spk_ptr || !spk_utts || !stats || !dstats || !workspace || !dfeat ||
+        n_utts < 0 || n_spk < 0 || n_feat <= 0 || win_len <= 0 || shift_len <= 0)
+        return fail(SEPT_E_BADARG, "sept_speaker_stats_bwd_f32: bad argument");
+    if (!aligned16(workspace)) return fail(SEPT_E_BADARG, "sept_speaker_stats_bwd_f32: workspace must be 16-byte aligned");
+    sept::SpeakerStatsBwdParams p{};
+    p.f.feat = feat; p.f.frame_off = frame_off; p.f.whole = whole; p.f.n_utts = n_utts; p.f.n_feat = n_feat;
+    p.f.win_len = win_len; p.f.shift_len = shift_len; p.f.spk_ptr = spk_ptr; p.f.spk_utts = spk_utts; p.f.n_spk = n_spk;
+    p.f.stats = const_cast<float*>(stats);
+    p.spk_of_utt = spk_of_utt; p.dstats = dstats; p.dfeat = dfeat;
+    unsigned char* ws = static_cast<unsigned char*>(workspace);
+    p.utt_ties = reinterpret_cast<int32_t*>(ws);
+    p.spk_ties = reinterpret_cast<int32_t*>(ws + sept::speaker_stats_bwd_ties_offset(n_utts, n_feat));
+    SEPT_CUDA(sept::launch_speaker_stats_bwd(p, static_cast<cudaStream_t>(stream)));
     return SEPT_OK;
 }
 

@@ -12,6 +12,8 @@ from typing import Sequence
 import numpy as np
 import torch
 
+from torch.autograd.function import once_differentiable
+
 from . import _lib
 from .extraction import Layout, _stream
 
@@ -24,9 +26,10 @@ class SpeakerStats:
     speakers: list                 # speaker labels, row order of `stats`
     stats: torch.Tensor            # device (n_spk, 5, F): count, mean, std (ddof 0), min, max
     spk_of_utt: torch.Tensor       # device int32 [n_utts] row index per utterance
+    spk_of_utt_host: np.ndarray | None = None   # host copy of spk_of_utt: a backward builds its speaker lists from it
 
     def as_dict(self) -> dict:
-        h = self.stats.cpu().numpy()
+        h = self.stats.detach().cpu().numpy()
         return {s: {"count": h[i, 0], "mean": h[i, 1], "std": h[i, 2], "min": h[i, 3], "max": h[i, 4]}
                 for i, s in enumerate(self.speakers)}
 
@@ -48,20 +51,31 @@ def speaker_stats(feat: torch.Tensor, lay: Layout, speaker_of_utt: Sequence, who
     speakers = list(dict.fromkeys(speaker_of_utt))
     row = {s: i for i, s in enumerate(speakers)}
     spk_idx = np.fromiter((row[s] for s in speaker_of_utt), dtype=np.int32, count=n_utts)
-    order = np.argsort(spk_idx, kind="stable").astype(np.int32)
-    ptr = np.zeros(len(speakers) + 1, dtype=np.int32)
-    np.cumsum(np.bincount(spk_idx, minlength=len(speakers)), out=ptr[1:])
     dev = feat.device
-    F = feat.shape[1]
-    d_ptr, d_order = torch.from_numpy(ptr).to(dev), torch.from_numpy(order).to(dev)
+    d_ptr, d_order = _speaker_lists(spk_idx, len(speakers), dev)
     d_whole = None if whole_utterance is None else torch.from_numpy(np.asarray(whole_utterance, dtype=np.uint8)).to(dev)
+    stats = _launch_speaker_stats(feat, lay, d_whole, win_len, shift_len, d_ptr, d_order, len(speakers))
+    return SpeakerStats(speakers, stats, torch.from_numpy(spk_idx).to(dev), spk_idx)
+
+
+def _speaker_lists(spk_idx: np.ndarray, n_spk: int, dev):
+    """Device CSR (ptr [n_spk + 1], utterance ids grouped by speaker in utterance order) of a host speaker index."""
+    order = np.argsort(spk_idx, kind="stable").astype(np.int32)
+    ptr = np.zeros(n_spk + 1, dtype=np.int32)
+    np.cumsum(np.bincount(spk_idx, minlength=n_spk), out=ptr[1:])
+    return torch.from_numpy(ptr).to(dev), torch.from_numpy(order).to(dev)
+
+
+def _launch_speaker_stats(feat, lay, d_whole, win_len, shift_len, d_ptr, d_order, n_spk) -> torch.Tensor:
+    dev = feat.device
+    n_utts, F = len(lay.frame_off_host) - 1, feat.shape[1]
     partial = torch.empty((n_utts, 5, F), dtype=torch.float32, device=dev)
-    stats = torch.empty((len(speakers), 5, F), dtype=torch.float32, device=dev)
+    stats = torch.empty((n_spk, 5, F), dtype=torch.float32, device=dev)
     with torch.cuda.device(dev):
         _lib.check(_lib.lib().sept_speaker_stats_f32(
             feat.data_ptr(), lay.frame_off.data_ptr(), 0 if d_whole is None else d_whole.data_ptr(), n_utts, F, win_len,
-            shift_len, d_ptr.data_ptr(), d_order.data_ptr(), len(speakers), partial.data_ptr(), stats.data_ptr(), _stream(dev)))
-    return SpeakerStats(speakers, stats, torch.from_numpy(spk_idx).to(dev))
+            shift_len, d_ptr.data_ptr(), d_order.data_ptr(), n_spk, partial.data_ptr(), stats.data_ptr(), _stream(dev)))
+    return stats
 
 
 def normalize(feat: torch.Tensor, lay: Layout, st: SpeakerStats, mode: str = "znorm") -> torch.Tensor:
@@ -130,5 +144,149 @@ def speaker_stats_distributed(feat: torch.Tensor, lay: Layout, speaker_of_utt: S
         mn[idx], mx[idx] = st[:, 3], st[:, 4]
     n, mu, sd, lo, hi = parallel.merge_speaker_partials(cnt, mean, m2, mn, mx, group=group)
     stats = torch.stack([n, mu, sd, lo, hi], dim=1).contiguous()
-    spk_idx = torch.tensor([row[s] for s in speaker_of_utt], dtype=torch.int32, device=dev)
-    return SpeakerStats(list(all_speakers), stats, spk_idx)
+    spk_idx = np.array([row[s] for s in speaker_of_utt], dtype=np.int32)
+    return SpeakerStats(list(all_speakers), stats, torch.from_numpy(spk_idx).to(dev), spk_idx)
+
+
+# ---- gradients: the same forward launches, with a grad_fn to feat (and to the statistics) ------------------------
+class SpeakerStatsFunction(torch.autograd.Function):
+    """speaker_stats() with a gradient to feat: forward is the sept_speaker_stats_f32 launch of speaker_stats(), backward
+    one sept_speaker_stats_bwd_f32 call (the count row gets no gradient; no double backward)."""
+
+    @staticmethod
+    def forward(ctx, feat, lay, d_whole, win_len, shift_len, spk_of_utt, d_ptr, d_order, n_spk):
+        stats = _launch_speaker_stats(feat, lay, d_whole, win_len, shift_len, d_ptr, d_order, n_spk)
+        ctx.save_for_backward(feat, stats)
+        ctx.cfg = (lay, d_whole, win_len, shift_len, spk_of_utt, d_ptr, d_order, n_spk)
+        return stats
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, dstats):
+        feat, stats = ctx.saved_tensors
+        lay, d_whole, win_len, shift_len, spk_of_utt, d_ptr, d_order, n_spk = ctx.cfg
+        lib = _lib.lib()
+        dev, n_utts, F = feat.device, len(lay.frame_off_host) - 1, feat.shape[1]
+        dfeat = torch.empty_like(feat)
+        ws = torch.empty(max(16, lib.sept_speaker_stats_bwd_workspace_bytes(n_utts, n_spk, F)), dtype=torch.uint8, device=dev)
+        dstats = dstats.contiguous()
+        with torch.cuda.device(dev):
+            _lib.check(lib.sept_speaker_stats_bwd_f32(
+                feat.data_ptr(), lay.frame_off.data_ptr(), 0 if d_whole is None else d_whole.data_ptr(), n_utts, F, win_len,
+                shift_len, spk_of_utt.data_ptr(), d_ptr.data_ptr(), d_order.data_ptr(), n_spk, stats.data_ptr(),
+                dstats.data_ptr(), ws.data_ptr(), dfeat.data_ptr(), _stream(dev)))
+        return dfeat, None, None, None, None, None, None, None, None
+
+
+def speaker_stats_grad(feat: torch.Tensor, lay: Layout, speaker_of_utt: Sequence,
+                       whole_utterance: Sequence[bool] | None = None, win_len: int = WIN_LEN,
+                       shift_len: int = SHIFT_LEN) -> SpeakerStats:
+    """speaker_stats() with a gradient: `.stats` is bit-identical and carries a grad_fn to feat.
+
+    The gradient is what torch autograd gives through the reference's stacked rows (a frame in k windows is k rows):
+    mean and ddof-0 std of the weighted frames, min / max split over tied frames in proportion to their multiplicity.
+    The count row gets none; where the std is exactly 0 (a constant feature column) none flows through the std.
+    Deterministic (no atomics)."""
+    _lib.require_cuda(feat)
+    if feat.dtype != torch.float32 or feat.dim() != 2 or not feat.is_contiguous():
+        raise ValueError("feat must be a contiguous (total_frames, F) float32 tensor")
+    n_utts = len(lay.frame_off_host) - 1
+    if len(speaker_of_utt) != n_utts:
+        raise ValueError("one speaker label per utterance is required")
+    speakers = list(dict.fromkeys(speaker_of_utt))
+    row = {s: i for i, s in enumerate(speakers)}
+    spk_idx = np.fromiter((row[s] for s in speaker_of_utt), dtype=np.int32, count=n_utts)
+    dev = feat.device
+    d_ptr, d_order = _speaker_lists(spk_idx, len(speakers), dev)
+    d_whole = None if whole_utterance is None else torch.from_numpy(np.asarray(whole_utterance, dtype=np.uint8)).to(dev)
+    d_spk = torch.from_numpy(spk_idx).to(dev)
+    stats = SpeakerStatsFunction.apply(feat, lay, d_whole, win_len, shift_len, d_spk, d_ptr, d_order, len(speakers))
+    return SpeakerStats(speakers, stats, d_spk, spk_idx)
+
+
+class NormalizeFunction(torch.autograd.Function):
+    """normalize() (win is None) or normalized_windows() with gradients to feat and to the statistics: forward is the
+    existing launch, backward one sept_normalize_bwd_f32 call.  The host tables the backward needs (each utterance's
+    windows sorted by start, each speaker's utterances) are built here, so the backward launches kernels only."""
+
+    @staticmethod
+    def forward(ctx, feat, stats, lay, st, win, mode):
+        st_fwd = SpeakerStats(st.speakers, stats, st.spk_of_utt, st.spk_of_utt_host)
+        n_utts = len(lay.frame_off_host) - 1
+        dev = feat.device
+        if win is None:
+            out = normalize(feat, lay, st_fwd, mode)
+            tables = None
+        else:
+            wu, wt, win_len = win
+            out = normalized_windows(feat, lay, st_fwd, wu, wt, mode, win_len)
+            order = np.lexsort((np.arange(len(wu)), wt, wu)).astype(np.int32)     # by utterance, start, window id
+            ptr = np.zeros(n_utts + 1, dtype=np.int32)
+            np.cumsum(np.bincount(wu, minlength=n_utts), out=ptr[1:])
+            tables = (torch.from_numpy(wt).to(dev), torch.from_numpy(ptr).to(dev), torch.from_numpy(order).to(dev),
+                      len(wu), win_len)
+        spk_lists = None
+        if ctx.needs_input_grad[1]:
+            spk_idx = st.spk_of_utt_host if st.spk_of_utt_host is not None else st.spk_of_utt.cpu().numpy()
+            spk_lists = _speaker_lists(np.asarray(spk_idx, dtype=np.int32), stats.shape[0], dev)
+        ctx.save_for_backward(feat, stats)
+        ctx.cfg = (lay, st.spk_of_utt, tables, spk_lists, MODES[mode])
+        return out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, grad):
+        feat, stats = ctx.saved_tensors
+        lay, spk_of_utt, tables, spk_lists, mode = ctx.cfg
+        need_feat, need_stats = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+        if not (need_feat or need_stats):
+            return None, None, None, None, None, None
+        lib = _lib.lib()
+        dev, n_utts, F = feat.device, len(lay.frame_off_host) - 1, feat.shape[1]
+        dfeat = torch.empty_like(feat) if need_feat else None
+        dstats = torch.empty_like(stats) if need_stats else None
+        ws = (torch.empty(max(16, lib.sept_normalize_bwd_workspace_bytes(n_utts, F)), dtype=torch.uint8, device=dev)
+              if need_stats else None)
+        d_wt, d_ptr, d_list, n_win, win_len = tables if tables is not None else (None, None, None, 0, 0)
+        s_ptr, s_list = spk_lists if need_stats else (None, None)
+        grad = grad.contiguous()
+
+        def ptr(t):
+            return 0 if t is None else t.data_ptr()
+
+        with torch.cuda.device(dev):
+            _lib.check(lib.sept_normalize_bwd_f32(
+                feat.data_ptr(), lay.frame_off.data_ptr(), spk_of_utt.data_ptr(), stats.data_ptr(), ptr(d_wt), ptr(d_ptr),
+                ptr(d_list), n_win, win_len, n_utts, F, mode, grad.data_ptr(), ptr(s_ptr), ptr(s_list), stats.shape[0],
+                ptr(ws), ptr(dfeat), ptr(dstats), _stream(dev)))
+        return dfeat, dstats, None, None, None, None
+
+
+def normalize_grad(feat: torch.Tensor, lay: Layout, st: SpeakerStats, mode: str = "znorm") -> torch.Tensor:
+    """normalize() with a gradient: bit-identical values with a grad_fn to feat and, when st.stats requires grad (from
+    speaker_stats_grad), to the statistics.  Deterministic."""
+    _lib.require_cuda(feat)
+    if mode not in MODES:
+        raise ValueError(f"mode must be one of {sorted(MODES)}")
+    return NormalizeFunction.apply(feat, st.stats, lay, st, None, mode)
+
+
+def normalized_windows_grad(feat: torch.Tensor, lay: Layout, st: SpeakerStats, win_utt: np.ndarray, win_t0: np.ndarray,
+                            mode: str = "znorm", win_len: int = WIN_LEN) -> torch.Tensor:
+    """normalized_windows() with a gradient: bit-identical (n_windows, 1, win_len, F) windows with a grad_fn to feat and,
+    when st.stats requires grad (from speaker_stats_grad), to the statistics, padded rows included (they depend on the
+    statistics).  Any window table works (subsets, any order, repeated windows); win_t0 < 0 or win_utt outside
+    [0, n_utts) raises ValueError.  Deterministic (no atomics)."""
+    _lib.require_cuda(feat)
+    if mode not in MODES:
+        raise ValueError(f"mode must be one of {sorted(MODES)}")
+    wu = np.ascontiguousarray(win_utt, dtype=np.int32).reshape(-1)
+    wt = np.ascontiguousarray(win_t0, dtype=np.int32).reshape(-1)
+    n_utts = len(lay.frame_off_host) - 1
+    if len(wu) != len(wt):
+        raise ValueError("win_utt and win_t0 must have the same length")
+    if len(wt) and wt.min() < 0:
+        raise ValueError("win_t0 must be >= 0")
+    if len(wu) and (wu.min() < 0 or wu.max() >= n_utts):
+        raise ValueError(f"win_utt must lie in [0, {n_utts})")
+    return NormalizeFunction.apply(feat, st.stats, lay, st, (wu, wt, win_len), mode)
