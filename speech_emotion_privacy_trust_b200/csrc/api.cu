@@ -16,6 +16,7 @@
 #include "cloak.h"
 #include "extract.h"
 #include "extract_bwd.h"
+#include "extract_core.cuh"
 #include "mfcc_bwd.h"
 #include "norm.h"
 #include "norm_bwd.h"
@@ -158,13 +159,23 @@ int check_extract_shape(int n_fft, int hop, int n_mels, int n_mel_entries) {
     if (hop <= 0 || (hop & 1) || hop > n_fft)
         return fail(SEPT_E_UNSUPPORTED, "hop=%d unsupported: must be even and in (0, n_fft]", hop);
     if (n_mels <= 0 || n_mels > 512) return fail(SEPT_E_UNSUPPORTED, "n_mels=%d unsupported (1..512)", n_mels);
-    if (n_mel_entries >= 0 && sept::extract_smem_bytes_for(n_fft, hop, n_mel_entries) > 232448)
+    if (n_mel_entries >= 0 && sept::extract_smem_bytes_for(n_fft, hop, n_mel_entries) > sept::kMaxDynSmem)
         return fail(SEPT_E_UNSUPPORTED, "n_fft=%d hop=%d n_mels=%d does not fit the 227 KB of shared memory", n_fft, hop,
                     n_mels);
     return SEPT_OK;
 }
 
-// launch parameters shared by every extraction launch: the batch, its layout and the (n_fft, n_mels) constants
+// the set-up of every extraction entry, forward or backward: the shape checks and the (n_fft, n_mels) constants
+int extract_setup(int n_fft, int hop, int n_mels, ExtractConsts* c, int* sms) {
+    int rc = check_extract_shape(n_fft, hop, n_mels, -1);
+    if (rc) return rc;
+    rc = get_consts(n_fft, n_mels, c, sms);
+    if (rc) return rc;
+    return check_extract_shape(n_fft, hop, n_mels, c->n_mel_entries);
+}
+
+// launch parameters shared by every extraction launch: the batch, its layout and the (n_fft, n_mels) constants.  A
+// backward recomputes the forward with the same struct.
 sept::ExtractParams extract_params(const ExtractConsts& c, const float* wav, const int64_t* utt_off,
                                    const int64_t* frame_off, const int32_t* item_off, int n_utts, int hop, int n_mels) {
     sept::ExtractParams p{};
@@ -174,26 +185,12 @@ sept::ExtractParams extract_params(const ExtractConsts& c, const float* wav, con
     return p;
 }
 
-// ... and of every frame pass of a backward
-sept::LogmelBwdParams logmel_bwd_params(const ExtractConsts& c, const float* wav, const int64_t* utt_off,
-                                        const int64_t* frame_off, const int32_t* item_off, int n_utts, long long n_items,
-                                        int hop, int n_mels) {
-    sept::LogmelBwdParams p{};
-    p.wav = wav; p.utt_off = utt_off; p.frame_off = frame_off; p.item_off = item_off; p.n_utts = n_utts; p.n_items = n_items;
-    p.hop = hop; p.n_mels = n_mels; p.n_mel_entries = c.n_mel_entries; p.n_mel_head = c.n_mel_head; p.fast_dn = c.mel_fast;
-    p.window = c.window; p.tws = c.tws; p.mel_prog = c.mel_prog;
-    return p;
-}
-
-// The MFCC forward's power launch: mel power of x and np.gradient(x) to power [2][total_frames][128], the bits of each
-// utterance's largest value to utt_max [2][n_utts], the utterance of every frame to frame_utt.  It is deterministic, so
-// the backward, which runs this same launch, recomputes the forward's values bit for bit.
-int launch_mfcc_power(const ExtractConsts& c, int sms, const float* wav, const int64_t* utt_off, const int64_t* frame_off,
-                      const int32_t* item_off, int n_utts, int64_t total_frames, float* power, int32_t* utt_max,
-                      int* frame_utt, cudaStream_t st) {
-    SEPT_CUDA(cudaMemsetAsync(utt_max, 0, sizeof(int32_t) * 2 * (size_t)n_utts, st));
-    sept::ExtractParams p = extract_params(c, wav, utt_off, frame_off, item_off, n_utts, 200, 128);
-    p.total_frames = total_frames; p.out = power; p.utt_max = utt_max; p.frame_utt = frame_utt;
+// The MFCC forward's power launch (p: extract_params at n_fft 400, hop 200, 128 mels): mel power of x and
+// np.gradient(x) to p.out [2][total_frames][128], the bits of each utterance's largest value to p.utt_max [2][n_utts],
+// the utterance of every frame to p.frame_utt.  It is deterministic, so the backward, which runs this same launch,
+// recomputes the forward's values bit for bit.
+int launch_mfcc_power(const sept::ExtractParams& p, int sms, cudaStream_t st) {
+    SEPT_CUDA(cudaMemsetAsync(p.utt_max, 0, sizeof(int32_t) * 2 * (size_t)p.n_utts, st));
     SEPT_CUDA(sept::launch_extract(p, 400, sept::kModeMfccPower, sms, st));
     return SEPT_OK;
 }
@@ -254,13 +251,9 @@ int sept_logmel_f32(const float* wav, const int64_t* utt_off, const int64_t* fra
         return fail(SEPT_E_BADARG, "sept_logmel_f32: null pointer or negative n_utts");
     if (layout != SEPT_LAYOUT_FRAME_MAJOR && layout != SEPT_LAYOUT_BAND_MAJOR)
         return fail(SEPT_E_BADARG, "sept_logmel_f32: layout %d", layout);
-    int rc = check_extract_shape(n_fft, hop, n_mels, -1);
-    if (rc) return rc;
     ExtractConsts c;
     int sms = 0;
-    rc = get_consts(n_fft, n_mels, &c, &sms);
-    if (rc) return rc;
-    rc = check_extract_shape(n_fft, hop, n_mels, c.n_mel_entries);
+    int rc = extract_setup(n_fft, hop, n_mels, &c, &sms);
     if (rc) return rc;
     sept::ExtractParams p = extract_params(c, wav, utt_off, frame_off, item_off, n_utts, hop, n_mels);
     p.deriv = deriv ? 1 : 0;
@@ -281,16 +274,13 @@ int sept_logmel_bwd_f32(const float* wav, const int64_t* utt_off, const int64_t*
     if (!wav || !utt_off || !frame_off || !item_off || !grad || !workspace || !dwav || n_utts < 0 || n_items < 0)
         return fail(SEPT_E_BADARG, "sept_logmel_bwd_f32: null pointer or negative size");
     if (!aligned16(workspace)) return fail(SEPT_E_BADARG, "sept_logmel_bwd_f32: workspace must be 16-byte aligned");
-    int rc = check_extract_shape(n_fft, hop, n_mels, -1);
-    if (rc) return rc;
     ExtractConsts c;
     int sms = 0;
-    rc = get_consts(n_fft, n_mels, &c, &sms);
+    int rc = extract_setup(n_fft, hop, n_mels, &c, &sms);
     if (rc) return rc;
-    rc = check_extract_shape(n_fft, hop, n_mels, c.n_mel_entries);   // what the forward accepts, the backward takes
-    if (rc) return rc;
-    sept::LogmelBwdParams p = logmel_bwd_params(c, wav, utt_off, frame_off, item_off, n_utts, n_items, hop, n_mels);
-    p.grad = grad; p.ws = static_cast<float*>(workspace); p.dwav = dwav;
+    sept::LogmelBwdParams p{};
+    p.f = extract_params(c, wav, utt_off, frame_off, item_off, n_utts, hop, n_mels);
+    p.n_items = n_items; p.grad = grad; p.ws = static_cast<float*>(workspace); p.dwav = dwav;
     SEPT_CUDA(sept::launch_logmel_bwd(p, n_fft, sms, static_cast<cudaStream_t>(stream)));
     return SEPT_OK;
 }
@@ -302,17 +292,19 @@ int sept_mfcc_f32(const float* wav, const int64_t* utt_off, const int64_t* frame
         return fail(SEPT_E_BADARG, "sept_mfcc_f32: null pointer or bad size");
     ExtractConsts c;
     int sms = 0;
-    int rc = get_consts(400, 128, &c, &sms);
+    int rc = extract_setup(400, 200, 128, &c, &sms);
     if (rc) return rc;
     float* dct = nullptr;
     rc = get_dct(&dct);
     if (rc) return rc;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    int* frame_utt = reinterpret_cast<int*>(scratch + 2 * (size_t)total_frames * 128);
-    rc = launch_mfcc_power(c, sms, wav, utt_off, frame_off, item_off, n_utts, total_frames, scratch, utt_max, frame_utt, st);
+    sept::ExtractParams p = extract_params(c, wav, utt_off, frame_off, item_off, n_utts, 200, 128);
+    p.total_frames = total_frames; p.out = scratch; p.utt_max = utt_max;
+    p.frame_utt = reinterpret_cast<int*>(scratch + 2 * (size_t)total_frames * 128);
+    rc = launch_mfcc_power(p, sms, st);
     if (rc) return rc;
     sept::MfccDctParams d{};
-    d.power = scratch; d.utt_max = utt_max; d.frame_utt = frame_utt; d.frame_off = frame_off; d.dct = dct; d.n_utts = n_utts;
+    d.power = scratch; d.utt_max = utt_max; d.frame_utt = p.frame_utt; d.frame_off = frame_off; d.dct = dct; d.n_utts = n_utts;
     d.total_frames = total_frames; d.top_db = 80.0f; d.out = out;
     SEPT_CUDA(sept::launch_mfcc_dct(d, st));
     return SEPT_OK;
@@ -332,7 +324,7 @@ int sept_mfcc_bwd_f32(const float* wav, const int64_t* utt_off, const int64_t* f
     if (!aligned16(workspace)) return fail(SEPT_E_BADARG, "sept_mfcc_bwd_f32: workspace must be 16-byte aligned");
     ExtractConsts c;
     int sms = 0;
-    int rc = get_consts(400, 128, &c, &sms);
+    int rc = extract_setup(400, 200, 128, &c, &sms);
     if (rc) return rc;
     float* dct = nullptr;
     rc = get_dct(&dct);
@@ -340,15 +332,16 @@ int sept_mfcc_bwd_f32(const float* wav, const int64_t* utt_off, const int64_t* f
     const sept::MfccBwdLayout l = sept::mfcc_bwd_layout(n_utts, total_frames, n_items);
     unsigned char* ws = static_cast<unsigned char*>(workspace);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    float* power = reinterpret_cast<float*>(ws + l.power);
-    int32_t* utt_max = reinterpret_cast<int32_t*>(ws + l.utt_max);
-    int* frame_utt = reinterpret_cast<int*>(ws + l.frame_utt);
-    rc = launch_mfcc_power(c, sms, wav, utt_off, frame_off, item_off, n_utts, total_frames, power, utt_max, frame_utt, st);
-    if (rc) return rc;
     sept::MfccBwdParams b{};
-    b.frames = logmel_bwd_params(c, wav, utt_off, frame_off, item_off, n_utts, n_items, 200, 128);
-    b.grad = grad; b.dct = dct; b.frame_utt = frame_utt; b.utt_max = utt_max; b.total_frames = total_frames;
-    b.power = power; b.part = reinterpret_cast<float*>(ws + l.part); b.amask = reinterpret_cast<uint32_t*>(ws + l.amask);
+    sept::ExtractParams& p = b.frames.f;                         // the power launch, then the frame passes' recompute
+    p = extract_params(c, wav, utt_off, frame_off, item_off, n_utts, 200, 128);
+    p.total_frames = total_frames; p.out = reinterpret_cast<float*>(ws + l.power);
+    p.utt_max = reinterpret_cast<int32_t*>(ws + l.utt_max); p.frame_utt = reinterpret_cast<int*>(ws + l.frame_utt);
+    rc = launch_mfcc_power(p, sms, st);
+    if (rc) return rc;
+    b.frames.n_items = n_items;
+    b.grad = grad; b.dct = dct; b.frame_utt = p.frame_utt; b.utt_max = p.utt_max; b.total_frames = total_frames;
+    b.power = p.out; b.part = reinterpret_cast<float*>(ws + l.part); b.amask = reinterpret_cast<uint32_t*>(ws + l.amask);
     b.rows0 = reinterpret_cast<float*>(ws + l.rows0); b.rows1 = reinterpret_cast<float*>(ws + l.rows1); b.dwav = dwav;
     SEPT_CUDA(sept::launch_mfcc_bwd(b, sms, st));
     return SEPT_OK;

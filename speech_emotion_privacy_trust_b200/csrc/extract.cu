@@ -23,27 +23,12 @@ namespace sept {
 constexpr float kDbPerLog2 = 3.01029995663981195f;   // 10*log10(2)
 constexpr float kAmin = 1e-10f;                        // amplitude_to_DB amin (functional.py:390)
 
-// bytes of the CTA-shared constants: mel gather program, window, split twiddles
-__host__ __device__ inline int extract_const_bytes(int R, int n_mel_entries) {
-    return (n_mel_entries * 16 + R * 25 * 8 + 13 * (R + 1) * 8 + 15) & ~15;
-}
-
 // 10*log10(max(p, 1e-10)) through MUFU.LG2 (abs. error ~1e-6 in log2 => ~1e-5 dB); the clamp keeps the argument normal,
 // so the flush-to-zero form needs no denormal branch
 __device__ __forceinline__ float power_to_db(float p) {
     float l;
     asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(l) : "f"(fmaxf(p, kAmin)));
     return kDbPerLog2 * l;
-}
-
-// first utterance u with item_off[u+1] > item
-__device__ __forceinline__ int find_utt(const int32_t* __restrict__ item_off, int n_utts, int item) {
-    int lo_ = 0, hi_ = n_utts - 1;
-    while (lo_ < hi_) {
-        const int mid = (lo_ + hi_) >> 1;
-        if (__ldg(item_off + mid + 1) > item) hi_ = mid; else lo_ = mid + 1;
-    }
-    return lo_;
 }
 
 // ---- asynchronous staging (LDGSTS): the next item's waveform span lands in shared memory while the current item is
@@ -278,15 +263,10 @@ __global__ void __launch_bounds__(ExtractWarps<R>::value * 32, 1) extract_kernel
     const int hop = prm.hop, n_mels = prm.n_mels;
     const int stage_floats = G::stage_floats(hop);
 
-    // ---- CTA-shared constants -----------------------------------------------------------------------------
-    mel_step* melp = reinterpret_cast<mel_step*>(smem_raw);                      // [n_mel_entries]
-    f2* win2 = reinterpret_cast<f2*>(melp + prm.n_mel_entries);                  // [NC]
-    f2* tws = win2 + G::NC;                                                      // [13][R + 1]
-    const int const_bytes = extract_const_bytes(R, prm.n_mel_entries);
-    for (int i = threadIdx.x; i < 13 * G::TWS; i += blockDim.x) tws[i] = reinterpret_cast<const f2*>(prm.tws)[i];
-    for (int i = threadIdx.x; i < prm.n_mel_entries; i += blockDim.x)
-        reinterpret_cast<f4*>(melp)[i] = reinterpret_cast<const f4*>(prm.mel_prog)[i];
-    for (int i = threadIdx.x; i < G::NC; i += blockDim.x) win2[i] = reinterpret_cast<const f2*>(prm.window)[i];
+    const CtaConsts cc = load_cta_consts<G>(threadIdx.x, blockDim.x, smem_raw, prm);
+    mel_step* melp = cc.mel;
+    f2* win2 = cc.win2;
+    f2* tws = cc.tws;
     uint32_t taddr = 0;                                           // this warp's quarter of the CTA's tensor memory
     __shared__ uint32_t tmem_base;
     // ---- this CTA's contiguous item range.  kDynamicItems: its warps draw items from a shared counter instead of
@@ -321,7 +301,7 @@ __global__ void __launch_bounds__(ExtractWarps<R>::value * 32, 1) extract_kernel
 
     // ---- warp-private tiles -------------------------------------------------------------------------------
     const int warp_bytes = stage_floats * 4 + G::Y_PK4 * 16;
-    unsigned char* wbase = smem_raw + const_bytes + warp * warp_bytes;
+    unsigned char* wbase = smem_raw + extract_const_bytes(R, prm.n_mel_entries) + warp * warp_bytes;
     float* stage = reinterpret_cast<float*>(wbase);
     pk2* Y = reinterpret_cast<pk2*>(wbase + stage_floats * 4);
     pk2* P = Y;
@@ -501,15 +481,13 @@ __global__ void __launch_bounds__(ExtractWarps<R>::value * 32, 1) extract_kernel
 
 
 // ---- host launchers ----------------------------------------------------------------------------------------
-constexpr size_t kMaxSmem = 232448 - 64;  // 227 KB opt-in limit per CTA minus the static shared memory (TMEM base slot)
+constexpr size_t kMaxSmem = kMaxDynSmem - 64;  // minus the static shared memory (tmem_base, cta_next)
 
 template <int R>
-static int extract_warps(int hop, int n_mel_entries) {            // warps whose tiles fit beside the constants
+static int extract_warps(int hop, int n_mel_entries) {
     using G = Geo<R>;
-    const size_t cb = (size_t)extract_const_bytes(R, n_mel_entries), wb = G::stage_floats(hop) * 4 + G::Y_PK4 * 16;
-    if (cb + wb > kMaxSmem) return 0;
-    const int fit = (int)((kMaxSmem - cb) / wb);
-    return fit < ExtractWarps<R>::value ? fit : ExtractWarps<R>::value;
+    return warps_that_fit(extract_const_bytes(R, n_mel_entries), G::stage_floats(hop) * 4 + G::Y_PK4 * 16,
+                          ExtractWarps<R>::value, kMaxSmem);
 }
 
 template <int R>
@@ -557,22 +535,6 @@ int extract_frames_per_item(int n_fft) {
         case 1600: return Geo<32>::FPW;
     }
     return 0;
-}
-
-template <int R>
-static bool fast_ok(int n_head, const int* st) {
-    using F = FastMel<R>;
-    return n_head == F::head && st[0] == F::s0 && st[1] == F::s1 && st[2] == F::s2 && st[3] == F::s3;
-}
-
-bool extract_mel_fast_ok(int n_fft, int n_mels, int n_head, const int* round_steps, int n_rounds) {
-    if (n_mels != 128 || n_rounds != 4) return false;
-    switch (n_fft) {
-        case 400: return fast_ok<8>(n_head, round_steps);
-        case 800: return fast_ok<16>(n_head, round_steps);
-        case 1600: return fast_ok<32>(n_head, round_steps);
-    }
-    return false;
 }
 
 size_t extract_smem_bytes_for(int n_fft, int hop, int n_mel_entries) {

@@ -19,6 +19,15 @@ enum : int {
 // with ten warps and items drawn from a counter: 7.11 vs 6.95 ms).
 template <int R> struct ExtractWarps { static constexpr int value = 8; };
 
+constexpr size_t kMaxDynSmem = 232448;   // 227 KB: the opt-in limit of a CTA's dynamic shared memory
+
+// warps (at most cap) whose tiles of warp_bytes fit beside const_bytes of CTA constants in limit bytes; 0: none fits
+inline int warps_that_fit(size_t const_bytes, size_t warp_bytes, int cap, size_t limit) {
+    if (const_bytes + warp_bytes > limit) return 0;
+    const int fit = (int)((limit - const_bytes) / warp_bytes);
+    return fit < cap ? fit : cap;
+}
+
 struct ExtractParams {
     const float* wav;            // all utterances back to back
     const int64_t* utt_off;      // [n_utts + 1] sample offsets
@@ -55,8 +64,6 @@ struct MfccDctParams {
 cudaError_t launch_extract(const ExtractParams& prm, int n_fft, int mode, int grid, cudaStream_t stream);
 size_t extract_smem_bytes_for(int n_fft, int hop, int n_mel_entries);
 int extract_frames_per_item(int n_fft);
-// true when a 128-band program with these step counts may run the unrolled mel path
-bool extract_mel_fast_ok(int n_fft, int n_mels, int n_head, const int* round_steps, int n_rounds);
 cudaError_t launch_mfcc_dct(const MfccDctParams& prm, cudaStream_t stream);        // dB + top_db floor + DCT (mfcc_dct.cu)
 
 }  // namespace sept

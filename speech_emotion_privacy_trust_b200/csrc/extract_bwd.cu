@@ -22,36 +22,33 @@ __global__ void __launch_bounds__(kBwdWarps * 32, 1) logmel_bwd_frames_kernel(co
     using B = Bwd<G>;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, warps = blockDim.x >> 5;
-    const int hop = prm.hop, n_mels = prm.n_mels;
+    const ExtractParams& f = prm.f;
+    const int hop = f.hop, n_mels = f.n_mels;
 
-    mel_step* melp = reinterpret_cast<mel_step*>(smem_raw);
-    f2* win2 = reinterpret_cast<f2*>(melp + prm.n_mel_entries);
-    f2* tws = win2 + G::NC;
-    for (int i = threadIdx.x; i < 13 * G::TWS; i += blockDim.x) tws[i] = reinterpret_cast<const f2*>(prm.tws)[i];
-    for (int i = threadIdx.x; i < prm.n_mel_entries; i += blockDim.x)
-        reinterpret_cast<f4*>(melp)[i] = reinterpret_cast<const f4*>(prm.mel_prog)[i];
-    for (int i = threadIdx.x; i < G::NC; i += blockDim.x) win2[i] = reinterpret_cast<const f2*>(prm.window)[i];
+    const CtaConsts cc = load_cta_consts<G>(threadIdx.x, blockDim.x, smem_raw, f);
+    const f2* win2 = cc.win2;
+    const f2* tws = cc.tws;
     __syncthreads();
 
-    float* wbase = reinterpret_cast<float*>(smem_raw + bwd_const_bytes(R, prm.n_mel_entries)) + (size_t)warp * B::warp_floats(hop, n_mels);
+    float* wbase = reinterpret_cast<float*>(smem_raw + extract_const_bytes(R, f.n_mel_entries)) + (size_t)warp * B::warp_floats(hop, n_mels);
     float* stage = wbase;
     pk2* Y = reinterpret_cast<pk2*>(stage + G::stage_floats(hop));
     pk2* P = Y + G::Y_PK2;
     pk2* U = P + G::PPW * G::PP;
     pk2* D = reinterpret_cast<pk2*>(reinterpret_cast<float*>(U) + B::ud_floats(n_mels));
-    const mel_step* prog = melp;
+    const mel_step* prog = cc.mel;
     const int row = B::row_floats(hop), span = G::span(hop);
 
-    long long n_items = __ldg(prm.item_off + prm.n_utts);
+    long long n_items = __ldg(f.item_off + f.n_utts);
     if (n_items > prm.n_items) n_items = prm.n_items;
     for (long long item = (long long)blockIdx.x * warps + warp; item < n_items; item += (long long)gridDim.x * warps) {
-        const int u = bwd_find_utt(prm.item_off, prm.n_utts, item);
-        const long long s0 = __ldg(prm.utt_off + u), f0 = __ldg(prm.frame_off + u);
-        const int n = (int)(__ldg(prm.utt_off + u + 1) - s0);
-        const int T = (int)(__ldg(prm.frame_off + u + 1) - f0);
-        const int t0 = (int)(item - __ldg(prm.item_off + u)) * G::FPW;
+        const int u = find_utt(f.item_off, f.n_utts, item);
+        const long long s0 = __ldg(f.utt_off + u), f0 = __ldg(f.frame_off + u);
+        const int n = (int)(__ldg(f.utt_off + u + 1) - s0);
+        const int T = (int)(__ldg(f.frame_off + u + 1) - f0);
+        const int t0 = (int)(item - __ldg(f.item_off + u)) * G::FPW;
         __syncwarp();                                            // previous item's frame tile reads are done
-        stage_item<G>(lane, prm.wav + s0, n, t0, hop, DERIV, stage);
+        stage_item<G>(lane, f.wav + s0, n, t0, hop, DERIV, stage);
         __syncwarp();
         pass1<G, false>(lane, stage, hop, WinShared{win2}, Y);
         __syncwarp();
@@ -62,11 +59,11 @@ __global__ void __launch_bounds__(kBwdWarps * 32, 1) logmel_bwd_frames_kernel(co
         __syncwarp();
         bwd_split<G>(lane, Y, tws, P);
         __syncwarp();
-        bwd_mel_sums<G>(lane, P, prog, prm.n_mel_head, n_mels, prm.fast_dn != 0, U, D);
+        bwd_mel_sums<G>(lane, P, prog, f.n_mel_head, n_mels, f.mel_fast != 0, U, D);
         __syncwarp();
         bwd_dmel<G>(lane, U, D, prm.grad + f0 * n_mels, T, t0, n_mels, P);
         __syncwarp();
-        bwd_dpower<G>(lane, U, prog, prm.n_mel_head, n_mels, P);
+        bwd_dpower<G>(lane, U, prog, f.n_mel_head, n_mels, P);
         __syncwarp();
         bwd_unsplit<G>(lane, Y, P, tws);
         __syncwarp();
@@ -88,34 +85,25 @@ __global__ void __launch_bounds__(kBwdWarps * 32, 1) logmel_bwd_frames_kernel(co
 template <int R>
 __global__ void __launch_bounds__(256) logmel_bwd_gather_kernel(const LogmelBwdParams prm) {
     using G = Geo<R>;
-    const int row = Bwd<G>::row_floats(prm.hop);
-    const long long first = __ldg(prm.utt_off), last = __ldg(prm.utt_off + prm.n_utts);
+    const ExtractParams& f = prm.f;
+    const int row = Bwd<G>::row_floats(f.hop);
+    const long long first = __ldg(f.utt_off), last = __ldg(f.utt_off + f.n_utts);
     for (long long i = first + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < last; i += (long long)gridDim.x * blockDim.x) {
-        const int u = bwd_find_utt(prm.utt_off, prm.n_utts, i);
-        const long long s0 = __ldg(prm.utt_off + u);
-        const int n = (int)(__ldg(prm.utt_off + u + 1) - s0);
-        const int i0 = __ldg(prm.item_off + u), n_items = __ldg(prm.item_off + u + 1) - i0;
-        prm.dwav[i] = bwd_gather<G>(prm.ws + (long long)i0 * row, row, n_items, n, (int)(i - s0), prm.hop);
+        const int u = find_utt(f.utt_off, f.n_utts, i);
+        const long long s0 = __ldg(f.utt_off + u);
+        const int n = (int)(__ldg(f.utt_off + u + 1) - s0);
+        const int i0 = __ldg(f.item_off + u), n_items = __ldg(f.item_off + u + 1) - i0;
+        prm.dwav[i] = bwd_gather<G>(prm.ws + (long long)i0 * row, row, n_items, n, (int)(i - s0), f.hop);
     }
-}
-
-constexpr size_t kBwdMaxSmem = 232448;
-
-template <int R>
-static int bwd_warps(int hop, int n_mels, int n_mel_entries) {
-    const size_t cb = (size_t)bwd_const_bytes(R, n_mel_entries), wb = (size_t)Bwd<Geo<R>>::warp_floats(hop, n_mels) * 4;
-    if (cb + wb > kBwdMaxSmem) return 0;
-    const int fit = (int)((kBwdMaxSmem - cb) / wb);
-    return fit < kBwdWarps ? fit : kBwdWarps;
 }
 
 template <int R, int DERIV>
 static cudaError_t launch_frames(const LogmelBwdParams& prm, int sms, cudaStream_t stream) {
     const auto kernel = logmel_bwd_frames_kernel<R, DERIV>;
-    const int warps = bwd_warps<R>(prm.hop, prm.n_mels, prm.n_mel_entries);
+    const size_t cb = extract_const_bytes(R, prm.f.n_mel_entries), wb = Bwd<Geo<R>>::warp_floats(prm.f.hop, prm.f.n_mels) * 4;
+    const int warps = warps_that_fit(cb, wb, kBwdWarps, kMaxDynSmem);
     if (warps == 0) return cudaErrorInvalidConfiguration;
-    const size_t smem = (size_t)bwd_const_bytes(R, prm.n_mel_entries) +
-                        (size_t)warps * Bwd<Geo<R>>::warp_floats(prm.hop, prm.n_mels) * 4;
+    const size_t smem = cb + warps * wb;
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     kernel<<<sms, warps * 32, smem, stream>>>(prm);

@@ -34,24 +34,6 @@ constexpr float kDbPerNeper = 4.34294481903251828f;      // 10 / ln 10: d(10 log
 
 constexpr int kBwdWarps = 8;     // warps per CTA of the frame pass at most (shared memory decides: extract_bwd.cu)
 
-#ifdef __CUDACC__                // kernel-side helpers of the frame passes (extract_bwd.cu, mfcc_bwd.cu)
-// utterance u with off[u] <= x < off[u + 1] (off: item or sample offsets)
-template <class Off>
-__device__ __forceinline__ int bwd_find_utt(const Off* off, int n_utts, long long x) {
-    int lo_ = 0, hi_ = n_utts - 1;
-    while (lo_ < hi_) {
-        const int mid = (lo_ + hi_) >> 1;
-        if (__ldg(off + mid + 1) > x) hi_ = mid; else lo_ = mid + 1;
-    }
-    return lo_;
-}
-
-// bytes of the frame pass's shared constants (mel program, window, split twiddles) in front of the warp tiles
-__host__ __device__ inline int bwd_const_bytes(int R, int n_mel_entries) {
-    return (n_mel_entries * 16 + R * 25 * 8 + 13 * (R + 1) * 8 + 15) & ~15;
-}
-#endif
-
 template <class G>
 struct Bwd {
     static SEPT_HD int ums(int n_mels) { return n_mels + 1; }                 // pk2 per frame pair of U and D

@@ -4,22 +4,13 @@
 #include <cstddef>
 #include <cstdint>
 
+#include "extract.h"
+
 namespace sept {
 
 struct LogmelBwdParams {
-    const float* wav;            // all utterances back to back
-    const int64_t* utt_off;      // [n_utts + 1] sample offsets
-    const int64_t* frame_off;    // [n_utts + 1] frame offsets
-    const int32_t* item_off;     // [n_utts + 1] item offsets
-    int n_utts;
+    ExtractParams f;             // the forward's launch, which the frame pass recomputes (its outputs are unused)
     long long n_items;           // items the workspace holds rows for
-    int hop;
-    int n_mels;
-    int n_mel_entries, n_mel_head;
-    int fast_dn;                 // the forward runs its compiled-in 128-band path: falling weight = 1/4 - rising
-    const float* window;         // [n_fft] periodic Hann
-    const float* tws;            // split twiddles (tables.h: make_split_twiddles)
-    const void* mel_prog;        // gather program (tables.h: make_mel_program)
     const float* grad;           // (total_frames, n_mels) upstream gradient of the frame-major log-mel
     float* ws;                   // [n_items][row] span rows
     float* dwav;                 // gradient w.r.t. wav

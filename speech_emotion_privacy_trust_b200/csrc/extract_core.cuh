@@ -23,6 +23,9 @@
 // and MelScale's matmul (transforms/_transforms.py:417).
 #pragma once
 #include "dft.cuh"
+#ifdef __CUDACC__
+#include "extract.h"
+#endif
 
 namespace sept {
 
@@ -359,5 +362,65 @@ SEPT_HD void mel_head(const pk2* P, const mel_step* head, int n_head, pk2 (&U)[G
             U[p] = fma2(*reinterpret_cast<const pk2*>(base + st.off + p * (G::PP * 8)), splat(st.up), U[p]);
     }
 }
+
+// true when the program has the step counts of FastMel<R>: the forward then runs its unrolled path, which takes the
+// falling weight as 1/4 - rising, and the backward must do the same to recompute the forward's mel power
+template <int R>
+inline bool fast_ok(int n_head, const int* st) {
+    using F = FastMel<R>;
+    return n_head == F::head && st[0] == F::s0 && st[1] == F::s1 && st[2] == F::s2 && st[3] == F::s3;
+}
+
+inline bool extract_mel_fast_ok(int n_fft, int n_mels, int n_head, const int* round_steps, int n_rounds) {
+    if (n_mels != 128 || n_rounds != 4) return false;
+    switch (n_fft) {
+        case 400: return fast_ok<8>(n_head, round_steps);
+        case 800: return fast_ok<16>(n_head, round_steps);
+        case 1600: return fast_ok<32>(n_head, round_steps);
+    }
+    return false;
+}
+
+// ---- CTA-shared constants of the extraction kernel and its backward, in front of the warp tiles: mel gather program
+// [n_mel_entries], window [NC] f2, split twiddles [13][R + 1] f2
+SEPT_HD int extract_const_bytes(int R, int n_mel_entries) {
+    return (n_mel_entries * 16 + R * 25 * 8 + 13 * (R + 1) * 8 + 15) & ~15;
+}
+
+#ifdef __CUDACC__
+struct CtaConsts {
+    mel_step* mel;
+    f2* win2;
+    f2* tws;
+};
+
+// thread tid of the CTA's n_threads copies its share of the constants of prm to the front of shared memory; a
+// __syncthreads() must precede any read.  The kernel passes threadIdx.x and blockDim.x: read there, they carry the
+// ranges of its launch bounds, which spare the loops a guard.
+template <class G>
+__device__ __forceinline__ CtaConsts load_cta_consts(unsigned tid, unsigned n_threads, unsigned char* smem,
+                                                     const ExtractParams& prm) {
+    CtaConsts c;
+    c.mel = reinterpret_cast<mel_step*>(smem);
+    c.win2 = reinterpret_cast<f2*>(c.mel + prm.n_mel_entries);
+    c.tws = c.win2 + G::NC;
+    for (int i = tid; i < 13 * G::TWS; i += n_threads) c.tws[i] = reinterpret_cast<const f2*>(prm.tws)[i];
+    for (int i = tid; i < prm.n_mel_entries; i += n_threads)
+        reinterpret_cast<f4*>(c.mel)[i] = reinterpret_cast<const f4*>(prm.mel_prog)[i];
+    for (int i = tid; i < G::NC; i += n_threads) c.win2[i] = reinterpret_cast<const f2*>(prm.window)[i];
+    return c;
+}
+
+// utterance u with off[u] <= x < off[u + 1] (off: item or sample offsets)
+template <class Off, class Key>
+__device__ __forceinline__ int find_utt(const Off* off, int n_utts, Key x) {
+    int lo_ = 0, hi_ = n_utts - 1;
+    while (lo_ < hi_) {
+        const int mid = (lo_ + hi_) >> 1;
+        if (__ldg(off + mid + 1) > x) hi_ = mid; else lo_ = mid + 1;
+    }
+    return lo_;
+}
+#endif
 
 }  // namespace sept

@@ -38,10 +38,10 @@ __global__ void __launch_bounds__(kHeadThreads) mfcc_bwd_head_kernel(const MfccB
     // every warp needs the utterance of the lane's frame for the Gbar loads; warp 0 also keeps its floors and maxima
     const bool live = lane < nf;
     const int u = live ? __ldg(prm.frame_utt + g0 + lane) : 0;
-    const long long f0 = live ? __ldg(prm.frames.frame_off + u) : 0;
-    const long long T = live ? __ldg(prm.frames.frame_off + u + 1) - f0 : 0;
+    const long long f0 = live ? __ldg(prm.frames.f.frame_off + u) : 0;
+    const long long T = live ? __ldg(prm.frames.f.frame_off + u + 1) - f0 : 0;
     if (warp == 0 && live) {
-        const int b0 = __ldg(prm.utt_max + u), b1 = __ldg(prm.utt_max + prm.frames.n_utts + u);
+        const int b0 = __ldg(prm.utt_max + u), b1 = __ldg(prm.utt_max + prm.frames.f.n_utts + u);
         mx[0][lane] = b0;
         mx[1][lane] = b1;
         fl[lane] = mfcc_floors(__int_as_float(b0), __int_as_float(b1));
@@ -97,8 +97,8 @@ __global__ void __launch_bounds__(kHeadThreads) mfcc_bwd_head_kernel(const MfccB
 
 __global__ void __launch_bounds__(kRouteWarps * 32) mfcc_bwd_route_kernel(const MfccBwdParams prm) {
     const int lane = threadIdx.x & 31, u = blockIdx.x * kRouteWarps + (threadIdx.x >> 5);
-    if (u >= prm.frames.n_utts) return;
-    const long long f0 = __ldg(prm.frames.frame_off + u), f1 = __ldg(prm.frames.frame_off + u + 1);
+    if (u >= prm.frames.f.n_utts) return;
+    const long long f0 = __ldg(prm.frames.f.frame_off + u), f1 = __ldg(prm.frames.f.frame_off + u + 1);
     float r0 = 0.f, r1 = 0.f, r2 = 0.f;
     int c0 = 0, c1 = 0;
     for (long long f = f0 + lane; f < f1; f += 32) {
@@ -119,7 +119,7 @@ __global__ void __launch_bounds__(kRouteWarps * 32) mfcc_bwd_route_kernel(const 
     }
     const float s0 = c0 ? r0 / (float)c0 : 0.f, s1 = c1 ? r1 / (float)c1 : 0.f, s2 = c1 ? r2 / (float)c1 : 0.f;
     if (s0 == 0.f && s1 == 0.f && s2 == 0.f) return;        // nothing was floored (the usual case: no write at all)
-    const float max1 = __int_as_float(__ldg(prm.utt_max + prm.frames.n_utts + u));
+    const float max1 = __int_as_float(__ldg(prm.utt_max + prm.frames.f.n_utts + u));
     float* G0 = prm.power;
     float* G1 = prm.power + prm.total_frames * kMfccBands;
     for (long long f = f0 + lane; f < f1; f += 32) {
@@ -134,11 +134,11 @@ __global__ void __launch_bounds__(kRouteWarps * 32) mfcc_bwd_route_kernel(const 
 }
 
 __global__ void __launch_bounds__(256) mfcc_bwd_gather_kernel(const MfccBwdParams prm) {
-    const LogmelBwdParams& fp = prm.frames;
+    const ExtractParams& fp = prm.frames.f;
     const int row = Bwd<Geo<8>>::row_floats(200);
     const long long first = __ldg(fp.utt_off), last = __ldg(fp.utt_off + fp.n_utts);
     for (long long i = first + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < last; i += (long long)gridDim.x * blockDim.x) {
-        const int u = bwd_find_utt(fp.utt_off, fp.n_utts, i);
+        const int u = find_utt(fp.utt_off, fp.n_utts, i);
         const long long s0 = __ldg(fp.utt_off + u);
         const int n = (int)(__ldg(fp.utt_off + u + 1) - s0);
         const int i0 = __ldg(fp.item_off + u), n_items = __ldg(fp.item_off + u + 1) - i0;
@@ -172,7 +172,7 @@ cudaError_t launch_mfcc_bwd(const MfccBwdParams& prm, int sms, cudaStream_t stre
     mfcc_bwd_head_kernel<<<(unsigned)head_blocks, kHeadThreads, 0, stream>>>(prm);
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
-    mfcc_bwd_route_kernel<<<(prm.frames.n_utts + kRouteWarps - 1) / kRouteWarps, kRouteWarps * 32, 0, stream>>>(prm);
+    mfcc_bwd_route_kernel<<<(prm.frames.f.n_utts + kRouteWarps - 1) / kRouteWarps, kRouteWarps * 32, 0, stream>>>(prm);
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
     LogmelBwdParams fp = prm.frames;
     fp.grad = prm.power;

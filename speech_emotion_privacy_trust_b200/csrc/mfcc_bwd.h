@@ -23,7 +23,7 @@ struct MfccBwdLayout {
 MfccBwdLayout mfcc_bwd_layout(int n_utts, long long total_frames, long long n_items);
 
 struct MfccBwdParams {
-    LogmelBwdParams frames;      // wav, offsets, n_fft 400 constants and n_items of both frame passes (grad, ws per pass)
+    LogmelBwdParams frames;      // the forward's power launch (frames.f) and n_items of both frame passes (grad, ws per pass)
     const float* grad;           // (120, T_u) blocks of sept_mfcc_f32's layout
     const float* dct;            // [128][40] orthonormal DCT-II basis
     const int32_t* frame_utt;

@@ -17,7 +17,7 @@ struct BwdFramePass {
     std::vector<float> win, tws;
     MelProgram prog;
     const mel_step* mprog;
-    bool fast_dn;                // what api.cu passes as fast_dn: the forward runs its compiled-in 128-band path
+    bool fast_dn;                // the forward runs its compiled-in 128-band path (ExtractParams::mel_fast)
     std::vector<float> stage;
     std::vector<pk4> Ybuf, Pbuf;
     std::vector<pk2> U, D;
@@ -29,9 +29,7 @@ struct BwdFramePass {
           U((size_t)G::PPW * B::ums(n_mels)), D((size_t)G::PPW * B::ums(n_mels)) {
         make_mel_program(G::NFFT, n_mels, 16000, prog);
         mprog = reinterpret_cast<const mel_step*>(prog.entries.data());
-        fast_dn = n_mels == 128 && prog.round_steps.size() == 4 && prog.n_head == FastMel<R>::head &&
-                  prog.round_steps[0] == FastMel<R>::s0 && prog.round_steps[1] == FastMel<R>::s1 &&
-                  prog.round_steps[2] == FastMel<R>::s2 && prog.round_steps[3] == FastMel<R>::s3;
+        fast_dn = extract_mel_fast_ok(G::NFFT, n_mels, prog.n_head, prog.round_steps.data(), (int)prog.round_steps.size());
         Y = reinterpret_cast<pk2*>(Ybuf.data());
         P = reinterpret_cast<pk2*>(Pbuf.data());
     }
