@@ -176,6 +176,24 @@ int sept_speaker_stats_bwd_f32(const float* feat_dev, const int64_t* frame_off_d
                                const int32_t* spk_ptr_dev, const int32_t* spk_utts_dev, int n_spk, const float* stats_dev,
                                const float* dstats_dev, void* workspace_dev, float* dfeat_dev, sept_stream_t stream);
 
+/* sept_speaker_stats_bwd_f32 in its two halves, for statistics merged over several ranks (each rank holds some of a
+ * speaker's utterances).  Every rank passes the merged (global) stats_dev with the same n_spk speaker rows and the CSR
+ * of its own utterances over those rows (a speaker the rank does not hold is an empty range and gets tie weight 0).
+ * _ties_i32 writes ties_dev (n_spk, 2, n_feat) int32: the summed window multiplicity of the rank's frames equal to each
+ * speaker's min (row 0) and max (row 1).  workspace_dev holds sept_speaker_stats_bwd_ties_workspace_bytes(n_utts, n_feat)
+ * bytes, 16-byte aligned.  Sum ties_dev over the ranks (exact in int32) and dstats_dev over the ranks, then
+ * _frames_f32 writes dfeat_dev (total_frames, n_feat) like sept_speaker_stats_bwd_f32.  On one rank the two calls give
+ * what sept_speaker_stats_bwd_f32 gives, bit for bit.  Deterministic, no allocation, capturable. */
+size_t sept_speaker_stats_bwd_ties_workspace_bytes(int n_utts, int n_feat);
+int sept_speaker_stats_bwd_ties_i32(const float* feat_dev, const int64_t* frame_off_dev, const uint8_t* whole_dev,
+                                    int n_utts, int n_feat, int win_len, int shift_len, const int32_t* spk_of_utt_dev,
+                                    const int32_t* spk_ptr_dev, const int32_t* spk_utts_dev, int n_spk,
+                                    const float* stats_dev, void* workspace_dev, int32_t* ties_dev, sept_stream_t stream);
+int sept_speaker_stats_bwd_frames_f32(const float* feat_dev, const int64_t* frame_off_dev, const uint8_t* whole_dev,
+                                      int n_utts, int n_feat, int win_len, int shift_len, const int32_t* spk_of_utt_dev,
+                                      const float* stats_dev, const float* dstats_dev, const int32_t* ties_dev,
+                                      float* dfeat_dev, sept_stream_t stream);
+
 /* ---- cloak noise layer + gradient reversal -------------------------------------------------------------------------
  * Forward of cloak_noise (model/cloak_models.py:41-58): out = x*mask + locs + sigma(rhos) * eps*mask with
  * sigma = (1 + tanh rho)/2 * (max_scale - min_scale) + min_scale, broadcast over the batch.  eps_dev != NULL supplies

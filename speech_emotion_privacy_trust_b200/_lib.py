@@ -38,6 +38,11 @@ _SIGNATURES = {
     "sept_speaker_stats_bwd_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
     "sept_speaker_stats_bwd_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr, C.c_int,
                                              c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
+    "sept_speaker_stats_bwd_ties_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
+    "sept_speaker_stats_bwd_ties_i32": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr,
+                                                  C.c_int, c_ptr, c_ptr, c_ptr, c_ptr]),
+    "sept_speaker_stats_bwd_frames_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr,
+                                                    c_ptr, c_ptr, c_ptr]),
     "sept_counter_add_u64": (C.c_int, [c_ptr, C.c_uint64, c_ptr]),
     "sept_cloak_fwd_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, C.c_uint64, C.c_uint64, c_ptr, C.c_int, C.c_float, C.c_float, C.c_float,
                                      C.c_int, C.c_int, c_ptr, c_ptr, c_ptr, c_ptr]),

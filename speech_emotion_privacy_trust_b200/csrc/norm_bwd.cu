@@ -359,18 +359,32 @@ cudaError_t launch_normalize_bwd(const NormalizeBwdParams& p, cudaStream_t strea
     return cudaGetLastError();
 }
 
-cudaError_t launch_speaker_stats_bwd(const SpeakerStatsBwdParams& p, cudaStream_t stream) {
-    const bool vec = p.f.n_feat % 4 == 0 && aligned(p.f.feat) && aligned(p.f.stats) && aligned(p.dfeat);
+// Both halves pick the vector width from the pointers they touch (the frames half also writes dfeat); the tie weights
+// are exact integers, so the width does not change a bit of either result.
+static bool stats_bwd_vec(const SpeakerStatsBwdParams& p) {
+    return p.f.n_feat % 4 == 0 && aligned(p.f.feat) && aligned(p.f.stats) && (!p.dfeat || aligned(p.dfeat));
+}
+
+cudaError_t launch_speaker_stats_bwd_ties(const SpeakerStatsBwdParams& p, cudaStream_t stream) {
     if (p.f.n_utts > 0) {
-        if (vec) stats_bwd_ties_kernel<4><<<p.f.n_utts, kBwdThreads, 0, stream>>>(p);
+        if (stats_bwd_vec(p)) stats_bwd_ties_kernel<4><<<p.f.n_utts, kBwdThreads, 0, stream>>>(p);
         else stats_bwd_ties_kernel<1><<<p.f.n_utts, kBwdThreads, 0, stream>>>(p);
     }
     if (p.f.n_spk > 0) stats_bwd_tie_merge_kernel<<<p.f.n_spk, 128 * kBwdMergeSlices, 0, stream>>>(p);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_speaker_stats_bwd_frames(const SpeakerStatsBwdParams& p, cudaStream_t stream) {
     if (p.f.n_utts > 0) {
-        if (vec) stats_bwd_frames_kernel<4><<<p.f.n_utts, kBwdThreads, 0, stream>>>(p);
+        if (stats_bwd_vec(p)) stats_bwd_frames_kernel<4><<<p.f.n_utts, kBwdThreads, 0, stream>>>(p);
         else stats_bwd_frames_kernel<1><<<p.f.n_utts, kBwdThreads, 0, stream>>>(p);
     }
     return cudaGetLastError();
+}
+
+cudaError_t launch_speaker_stats_bwd(const SpeakerStatsBwdParams& p, cudaStream_t stream) {
+    const cudaError_t e = launch_speaker_stats_bwd_ties(p, stream);
+    return e != cudaSuccess ? e : launch_speaker_stats_bwd_frames(p, stream);
 }
 
 }  // namespace sept

@@ -29,7 +29,7 @@ struct SpeakerStatsBwdParams {
     const int32_t* spk_of_utt;   // [n_utts]
     const float* dstats;         // (n_spk, 5, F); row 0 (count) is ignored
     int32_t* utt_ties;           // workspace (n_utts, 2, F): tie weight of the speaker's min / max in the utterance
-    int32_t* spk_ties;           // workspace (n_spk, 2, F)
+    int32_t* spk_ties;           // workspace (n_spk, 2, F), or the caller's buffer when the two halves run apart
     float* dfeat;                // (total_frames, F)
 };
 
@@ -45,6 +45,10 @@ inline size_t speaker_stats_bwd_workspace_bytes(int n_utts, int n_spk, int n_fea
 }
 
 cudaError_t launch_normalize_bwd(const NormalizeBwdParams& p, cudaStream_t stream);
-cudaError_t launch_speaker_stats_bwd(const SpeakerStatsBwdParams& p, cudaStream_t stream);
+// the statistics backward in two halves, so that data-parallel callers can sum spk_ties over the ranks in between:
+// ties (passes 1 and 2: utt_ties -> spk_ties; dstats and dfeat unused) and frames (pass 3: spk_ties -> dfeat)
+cudaError_t launch_speaker_stats_bwd_ties(const SpeakerStatsBwdParams& p, cudaStream_t stream);
+cudaError_t launch_speaker_stats_bwd_frames(const SpeakerStatsBwdParams& p, cudaStream_t stream);
+cudaError_t launch_speaker_stats_bwd(const SpeakerStatsBwdParams& p, cudaStream_t stream);   // ties, then frames
 
 }  // namespace sept

@@ -129,9 +129,22 @@ def speaker_stats_distributed(feat: torch.Tensor, lay: Layout, speaker_of_utt: S
     sharding, SURVEY 8e): every rank reduces its own utterances with the kernels, then ONE all-gather of the
     (count, mean, M2, min, max) partials and a Chan merge in rank order give every rank the global statistics.
     `all_speakers` fixes the row order on every rank (speakers a rank does not hold contribute empty partials)."""
-    from . import parallel
     local = speaker_stats(feat, lay, speaker_of_utt, whole_utterance, win_len, shift_len)
-    dev, F = feat.device, feat.shape[1]
+    stats = _merge_ranks(local, all_speakers, group)
+    spk_idx = _rows_of(speaker_of_utt, all_speakers)
+    return SpeakerStats(list(all_speakers), stats, torch.from_numpy(spk_idx).to(feat.device), spk_idx)
+
+
+def _rows_of(speaker_of_utt: Sequence, all_speakers: Sequence) -> np.ndarray:
+    row = {s: i for i, s in enumerate(all_speakers)}
+    return np.array([row[s] for s in speaker_of_utt], dtype=np.int32)
+
+
+def _merge_ranks(local: SpeakerStats, all_speakers: Sequence, group) -> torch.Tensor:
+    """The rank's own statistics -> the global (len(all_speakers), 5, F) ones: one all-gather and a Chan merge in rank
+    order (parallel.merge_speaker_partials)."""
+    from . import parallel
+    dev, F = local.stats.device, local.stats.shape[2]
     row = {s: i for i, s in enumerate(all_speakers)}
     n_spk = len(all_speakers)
     cnt = torch.zeros((n_spk, F), dtype=torch.float32, device=dev)
@@ -143,9 +156,7 @@ def speaker_stats_distributed(feat: torch.Tensor, lay: Layout, speaker_of_utt: S
         cnt[idx], mean[idx], m2[idx] = st[:, 0], st[:, 1], st[:, 2] * st[:, 2] * st[:, 0]
         mn[idx], mx[idx] = st[:, 3], st[:, 4]
     n, mu, sd, lo, hi = parallel.merge_speaker_partials(cnt, mean, m2, mn, mx, group=group)
-    stats = torch.stack([n, mu, sd, lo, hi], dim=1).contiguous()
-    spk_idx = np.array([row[s] for s in speaker_of_utt], dtype=np.int32)
-    return SpeakerStats(list(all_speakers), stats, torch.from_numpy(spk_idx).to(dev), spk_idx)
+    return torch.stack([n, mu, sd, lo, hi], dim=1).contiguous()
 
 
 # ---- gradients: the same forward launches, with a grad_fn to feat (and to the statistics) ------------------------
@@ -202,6 +213,74 @@ def speaker_stats_grad(feat: torch.Tensor, lay: Layout, speaker_of_utt: Sequence
     d_spk = torch.from_numpy(spk_idx).to(dev)
     stats = SpeakerStatsFunction.apply(feat, lay, d_whole, win_len, shift_len, d_spk, d_ptr, d_order, len(speakers))
     return SpeakerStats(speakers, stats, d_spk, spk_idx)
+
+
+class SpeakerStatsDistributedFunction(torch.autograd.Function):
+    """speaker_stats_distributed() with a gradient to this rank's feat.  Forward: the local launch, all-gather and Chan
+    merge of speaker_stats_distributed().  Backward: dstats summed over the ranks in rank order (one all-gather), the
+    rank's min / max tie weights against the global statistics (sept_speaker_stats_bwd_ties_i32), one exact int32 SUM
+    all-reduce of them, then sept_speaker_stats_bwd_frames_f32 (no double backward)."""
+
+    @staticmethod
+    def forward(ctx, feat, lay, speaker_of_utt, all_speakers, whole_utterance, group, win_len, shift_len, d_whole, d_spk,
+                d_ptr, d_order):
+        local = speaker_stats(feat, lay, speaker_of_utt, whole_utterance, win_len, shift_len)
+        stats = _merge_ranks(local, all_speakers, group)
+        ctx.save_for_backward(feat, stats)
+        ctx.cfg = (lay, group, win_len, shift_len, d_whole, d_spk, d_ptr, d_order)
+        return stats
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, dstats):
+        from . import parallel
+        feat, stats = ctx.saved_tensors
+        lay, group, win_len, shift_len, d_whole, d_spk, d_ptr, d_order = ctx.cfg
+        lib = _lib.lib()
+        dev, n_utts, n_spk, F = feat.device, len(lay.frame_off_host) - 1, stats.shape[0], feat.shape[1]
+        dstats = parallel.sum_in_rank_order(dstats.contiguous(), group)
+        ties = torch.empty((n_spk, 2, F), dtype=torch.int32, device=dev)
+        ws = torch.empty(max(16, lib.sept_speaker_stats_bwd_ties_workspace_bytes(n_utts, F)), dtype=torch.uint8, device=dev)
+        dfeat = torch.empty_like(feat)
+        whole = 0 if d_whole is None else d_whole.data_ptr()
+        with torch.cuda.device(dev):
+            _lib.check(lib.sept_speaker_stats_bwd_ties_i32(
+                feat.data_ptr(), lay.frame_off.data_ptr(), whole, n_utts, F, win_len, shift_len, d_spk.data_ptr(),
+                d_ptr.data_ptr(), d_order.data_ptr(), n_spk, stats.data_ptr(), ws.data_ptr(), ties.data_ptr(), _stream(dev)))
+            parallel.allreduce_exact_sum(ties, group)
+            _lib.check(lib.sept_speaker_stats_bwd_frames_f32(
+                feat.data_ptr(), lay.frame_off.data_ptr(), whole, n_utts, F, win_len, shift_len, d_spk.data_ptr(),
+                stats.data_ptr(), dstats.data_ptr(), ties.data_ptr(), dfeat.data_ptr(), _stream(dev)))
+        return dfeat, None, None, None, None, None, None, None, None, None, None, None
+
+
+def speaker_stats_distributed_grad(feat: torch.Tensor, lay: Layout, speaker_of_utt: Sequence, all_speakers: Sequence,
+                                   whole_utterance: Sequence[bool] | None = None, group=None, win_len: int = WIN_LEN,
+                                   shift_len: int = SHIFT_LEN) -> SpeakerStats:
+    """speaker_stats_distributed() with a gradient: `.stats` is bit-identical and carries a grad_fn to this rank's feat.
+
+    With the ranks' losses summed, the gradient each rank gets is what speaker_stats_grad() gives on one GPU over the
+    union of every rank's utterances, restricted to this rank's frames: the statistics, the min / max tie multiplicities
+    and the upstream dstats are all global.  The backward is collective (one all-gather of dstats, one int32 all-reduce),
+    so every rank of `group` must run it, as with any data-parallel backward.  Without an initialised process group, or
+    with one rank, no collective runs.  Deterministic: every rank adds dstats in rank order."""
+    _lib.require_cuda(feat)
+    if feat.dtype != torch.float32 or feat.dim() != 2 or not feat.is_contiguous():
+        raise ValueError("feat must be a contiguous (total_frames, F) float32 tensor")
+    n_utts = len(lay.frame_off_host) - 1
+    if len(speaker_of_utt) != n_utts:
+        raise ValueError("one speaker label per utterance is required")
+    missing = set(speaker_of_utt) - set(all_speakers)
+    if missing:
+        raise ValueError(f"speakers missing from all_speakers: {sorted(map(str, missing))}")
+    spk_idx = _rows_of(speaker_of_utt, all_speakers)
+    dev = feat.device
+    d_ptr, d_order = _speaker_lists(spk_idx, len(all_speakers), dev)
+    d_whole = None if whole_utterance is None else torch.from_numpy(np.asarray(whole_utterance, dtype=np.uint8)).to(dev)
+    d_spk = torch.from_numpy(spk_idx).to(dev)
+    stats = SpeakerStatsDistributedFunction.apply(feat, lay, speaker_of_utt, all_speakers, whole_utterance, group, win_len,
+                                                  shift_len, d_whole, d_spk, d_ptr, d_order)
+    return SpeakerStats(list(all_speakers), stats, d_spk, spk_idx)
 
 
 class NormalizeFunction(torch.autograd.Function):

@@ -1,7 +1,8 @@
 """Multi-GPU plumbing: one process per GPU, torch.distributed (NCCL on the B200 box, gloo in CPU tests).
 
 Extraction shards by utterance and needs no collective (SURVEY 8e).  Cloak + GRL training is data parallel with one
-flat-bucket gradient all-reduce per step; per-speaker statistics need one all-gather of the utterance partials' merge.
+flat-bucket gradient all-reduce per step; per-speaker statistics need one all-gather of the utterance partials' merge,
+and their gradient one all-gather of dstats and one integer all-reduce of the min / max tie weights.
 """
 from __future__ import annotations
 
@@ -151,6 +152,26 @@ def merge_speaker_partials(count: torch.Tensor, mean: torch.Tensor, m2: torch.Te
         lo, hi = torch.minimum(lo, lb), torch.maximum(hi, hb)
     std = torch.sqrt(s2 / torch.where(n > 0, n, torch.ones_like(n)))
     return n, mu, std, lo, hi
+
+
+def sum_in_rank_order(t: torch.Tensor, group=None) -> torch.Tensor:
+    """Sum of `t` over the ranks: one all-gather, then additions in rank order, so every rank holds the same bits and
+    repeated runs do too (a float all-reduce leaves the order to the collective).  `t` itself on one rank."""
+    if not dist.is_initialized() or dist.get_world_size(group) == 1:
+        return t
+    gathered = [torch.empty_like(t) for _ in range(dist.get_world_size(group))]
+    dist.all_gather(gathered, t.contiguous(), group=group)
+    total = gathered[0]
+    for part in gathered[1:]:
+        total += part
+    return total
+
+
+def allreduce_exact_sum(t: torch.Tensor, group=None) -> torch.Tensor:
+    """In-place SUM all-reduce of an integer tensor (exact, so the order does not matter); nothing on one rank."""
+    if dist.is_initialized() and dist.get_world_size(group) > 1:
+        dist.all_reduce(t, op=dist.ReduceOp.SUM, group=group)
+    return t
 
 
 # ---- host placement: the end-to-end (host buffer) path is bound by PCIe and by the host's memory fabric --------------
