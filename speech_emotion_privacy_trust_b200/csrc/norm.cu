@@ -163,10 +163,15 @@ __global__ void __launch_bounds__(128 * kMergeSlices) speaker_merge_kernel(const
     }
 }
 
-__device__ __forceinline__ float normalize_one(float x, float mean, float sd, float mn, float mx, int mode) {
-    if (mode == 0) return (x - mean) / (sd + 1e-5f);
-    return (x - mn) / (mx - mn) * 2.0f - 1.0f;
+// z = fmaf(x - a, b, c): znorm a = mean, b = 1 / (std + 1e-5), c = 0; min_max a = min, b = 2 / (max - min), c = -1.
+// Both normalisation kernels (and the backward, norm_bwd.cu) evaluate this one expression, so the kernel a call takes
+// (F, pointer alignment) does not change a bit of its result.
+__device__ __forceinline__ void norm_coef(int mode, float mean, float sd, float mn, float mx, float& a, float& b) {
+    if (mode == 0) { a = mean; b = 1.0f / (sd + 1e-5f); }
+    else { a = mn; b = 2.0f / (mx - mn); }
 }
+
+__device__ __forceinline__ float norm_c(int mode) { return mode == 0 ? 0.f : -1.f; }
 
 __global__ void __launch_bounds__(256) normalize_kernel(const NormalizeParams p) {
     const int F = p.n_feat;
@@ -187,11 +192,14 @@ __global__ void __launch_bounds__(256) normalize_kernel(const NormalizeParams p)
     T = (int)(p.frame_off[u + 1] - f0);
     const float* st = p.stats + ((long long)p.spk_of_utt[u] * kStatRows) * F;
     const int total = rows * F;
+    const float c = norm_c(p.mode);
     for (int i = threadIdx.x; i < total; i += blockDim.x) {
         const int r = i / F, f = i - r * F;
         const int t = t_begin + r;
         const float x = t < T ? p.feat[(f0 + t) * F + f] : 0.f;
-        out[i] = normalize_one(x, st[F + f], st[2 * F + f], st[3 * F + f], st[4 * F + f], p.mode);
+        float a, b;
+        norm_coef(p.mode, st[F + f], st[2 * F + f], st[3 * F + f], st[4 * F + f], a, b);
+        out[i] = fmaf(x - a, b, c);
     }
 }
 
@@ -220,17 +228,13 @@ __global__ void __launch_bounds__(256) normalize4_kernel(const NormalizeParams p
     if (r0 >= rows_per_pass) return;
     const float4 mean = reinterpret_cast<const float4*>(st + p.n_feat)[q], sd = reinterpret_cast<const float4*>(st + 2 * p.n_feat)[q];
     const float4 mn = reinterpret_cast<const float4*>(st + 3 * p.n_feat)[q], mx = reinterpret_cast<const float4*>(st + 4 * p.n_feat)[q];
-    // z = (x - a) * b + c with the divisions done once per thread: znorm a = mean, b = 1 / (std + 1e-5), c = 0;
-    // min_max a = min, b = 2 / (max - min), c = -1.  Four rows are in flight per thread.
+    // the divisions of norm_coef are done once per thread; four rows are in flight per thread
     float4 a, b;
-    float c;
-    if (p.mode == 0) {
-        a = mean; c = 0.f;
-        b = make_float4(1.0f / (sd.x + 1e-5f), 1.0f / (sd.y + 1e-5f), 1.0f / (sd.z + 1e-5f), 1.0f / (sd.w + 1e-5f));
-    } else {
-        a = mn; c = -1.f;
-        b = make_float4(2.0f / (mx.x - mn.x), 2.0f / (mx.y - mn.y), 2.0f / (mx.z - mn.z), 2.0f / (mx.w - mn.w));
-    }
+    const float c = norm_c(p.mode);
+    norm_coef(p.mode, mean.x, sd.x, mn.x, mx.x, a.x, b.x);
+    norm_coef(p.mode, mean.y, sd.y, mn.y, mx.y, a.y, b.y);
+    norm_coef(p.mode, mean.z, sd.z, mn.z, mx.z, a.z, b.z);
+    norm_coef(p.mode, mean.w, sd.w, mn.w, mx.w, a.w, b.w);
     for (int r = r0; r < rows; r += 4 * rows_per_pass) {
         float4 x[4];
 #pragma unroll
@@ -250,9 +254,12 @@ __global__ void __launch_bounds__(256) normalize4_kernel(const NormalizeParams p
     }
 }
 
+static bool aligned16(const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; }
+
 cudaError_t launch_speaker_stats(const SpeakerStatsParams& p, cudaStream_t stream) {
     if (p.n_utts > 0) {
-        if (p.n_feat == 128) utt_partial128_kernel<<<p.n_utts, 256, 0, stream>>>(p);
+        // float4 rows: feat + f0 * 128 is 16-byte aligned for every utterance exactly when feat is
+        if (p.n_feat == 128 && aligned16(p.feat)) utt_partial128_kernel<<<p.n_utts, 256, 0, stream>>>(p);
         else utt_partial_kernel<<<p.n_utts, 128, 0, stream>>>(p);
     }
     if (p.n_spk > 0) speaker_merge_kernel<<<p.n_spk, 128 * kMergeSlices, 0, stream>>>(p);
@@ -262,8 +269,8 @@ cudaError_t launch_speaker_stats(const SpeakerStatsParams& p, cudaStream_t strea
 cudaError_t launch_normalize(const NormalizeParams& p, cudaStream_t stream) {
     const int blocks = p.win_utt ? p.n_windows : p.n_utts;
     if (blocks > 0) {
-        const bool vec = p.n_feat % 4 == 0 && p.n_feat / 4 <= 256 && (reinterpret_cast<uintptr_t>(p.feat) & 15) == 0 &&
-                         (reinterpret_cast<uintptr_t>(p.out) & 15) == 0 && (reinterpret_cast<uintptr_t>(p.stats) & 15) == 0;
+        const bool vec = p.n_feat % 4 == 0 && p.n_feat / 4 <= 256 && aligned16(p.feat) && aligned16(p.out) &&
+                         aligned16(p.stats);
         if (vec) normalize4_kernel<<<blocks, 256, 0, stream>>>(p);
         else normalize_kernel<<<blocks, 256, 0, stream>>>(p);
     }

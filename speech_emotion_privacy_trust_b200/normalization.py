@@ -38,13 +38,38 @@ def n_windows(n_frames: int, win_len: int = WIN_LEN, shift_len: int = SHIFT_LEN)
     return 1 if n_frames < win_len else (n_frames - win_len) // shift_len + 1
 
 
+def _check_feat(feat: torch.Tensor, st: SpeakerStats | None = None) -> None:
+    """feat is what the kernels read: a contiguous (total_frames, F) float32 CUDA tensor, with the F of `st`'s statistics
+    when they are given."""
+    _lib.require_cuda(feat)
+    if feat.dtype != torch.float32 or feat.dim() != 2 or not feat.is_contiguous():
+        raise ValueError("feat must be a contiguous (total_frames, F) float32 tensor")
+    if st is not None and feat.shape[1] != st.stats.shape[2]:
+        raise ValueError(f"feat has {feat.shape[1]} features, the statistics {st.stats.shape[2]}")
+
+
+def _check_window_table(win_utt, win_t0, n_utts: int, win_len: int):
+    """(win_utt, win_t0) as int32 arrays.  ValueError for an utterance outside [0, n_utts), or a start below 0 or so large
+    that a window's last row (t0 + win_len - 1, int32 in the kernels) would overflow.  Checked before the int32 cast."""
+    if win_len <= 0:
+        raise ValueError("win_len must be > 0")
+    wu = np.asarray(win_utt, dtype=np.int64).reshape(-1)
+    wt = np.asarray(win_t0, dtype=np.int64).reshape(-1)
+    if len(wu) != len(wt):
+        raise ValueError("win_utt and win_t0 must have the same length")
+    t_max = np.iinfo(np.int32).max - win_len
+    if len(wt) and (wt.min() < 0 or wt.max() > t_max):
+        raise ValueError(f"win_t0 must lie in [0, {t_max}]")
+    if len(wu) and (wu.min() < 0 or wu.max() >= n_utts):
+        raise ValueError(f"win_utt must lie in [0, {n_utts})")
+    return wu.astype(np.int32), wt.astype(np.int32)
+
+
 def speaker_stats(feat: torch.Tensor, lay: Layout, speaker_of_utt: Sequence, whole_utterance: Sequence[bool] | None = None,
                   win_len: int = WIN_LEN, shift_len: int = SHIFT_LEN) -> SpeakerStats:
     """Weighted per-speaker mean/std/min/max: a frame inside k training windows counts k times (:26-27), utterances
     flagged whole (test split, :56-60) count each frame once."""
-    _lib.require_cuda(feat)
-    if feat.dtype != torch.float32 or feat.dim() != 2 or not feat.is_contiguous():
-        raise ValueError("feat must be a contiguous (total_frames, F) float32 tensor")
+    _check_feat(feat)
     n_utts = len(lay.frame_off_host) - 1
     if len(speaker_of_utt) != n_utts:
         raise ValueError("one speaker label per utterance is required")
@@ -80,7 +105,7 @@ def _launch_speaker_stats(feat, lay, d_whole, win_len, shift_len, d_ptr, d_order
 
 def normalize(feat: torch.Tensor, lay: Layout, st: SpeakerStats, mode: str = "znorm") -> torch.Tensor:
     """Frame-wise normalisation with each utterance's speaker statistics (:377-381); same shape as feat."""
-    _lib.require_cuda(feat)
+    _check_feat(feat, st)
     out = torch.empty_like(feat)
     dev = feat.device
     with torch.cuda.device(dev):
@@ -107,14 +132,16 @@ def window_table(lay: Layout, utts: Sequence[int] | None = None, win_len: int = 
 def normalized_windows(feat: torch.Tensor, lay: Layout, st: SpeakerStats, win_utt: np.ndarray, win_t0: np.ndarray,
                        mode: str = "znorm", win_len: int = WIN_LEN) -> torch.Tensor:
     """(n_windows, 1, win_len, F) float32 batches for the cloak layer: normalised windows, short utterances zero-padded
-    BEFORE normalisation like :29-35."""
-    _lib.require_cuda(feat)
+    BEFORE normalisation like :29-35.  win_t0 outside [0, 2^31 - 1 - win_len] or win_utt outside [0, n_utts) raises
+    ValueError."""
+    _check_feat(feat, st)
+    wu, wt = _check_window_table(win_utt, win_t0, len(lay.frame_off_host) - 1, win_len)
     dev = feat.device
-    n = len(win_utt)
+    n = len(wu)
     F = feat.shape[1]
     out = torch.empty((n, 1, win_len, F), dtype=torch.float32, device=dev)
-    d_wu = torch.from_numpy(np.ascontiguousarray(win_utt, dtype=np.int32)).to(dev)
-    d_wt = torch.from_numpy(np.ascontiguousarray(win_t0, dtype=np.int32)).to(dev)
+    d_wu = torch.from_numpy(wu).to(dev)
+    d_wt = torch.from_numpy(wt).to(dev)
     with torch.cuda.device(dev):
         _lib.check(_lib.lib().sept_normalize_windows_f32(
             feat.data_ptr(), lay.frame_off.data_ptr(), st.spk_of_utt.data_ptr(), st.stats.data_ptr(), d_wu.data_ptr(),
@@ -198,9 +225,7 @@ def speaker_stats_grad(feat: torch.Tensor, lay: Layout, speaker_of_utt: Sequence
     mean and ddof-0 std of the weighted frames, min / max split over tied frames in proportion to their multiplicity.
     The count row gets none; where the std is exactly 0 (a constant feature column) none flows through the std.
     Deterministic (no atomics)."""
-    _lib.require_cuda(feat)
-    if feat.dtype != torch.float32 or feat.dim() != 2 or not feat.is_contiguous():
-        raise ValueError("feat must be a contiguous (total_frames, F) float32 tensor")
+    _check_feat(feat)
     n_utts = len(lay.frame_off_host) - 1
     if len(speaker_of_utt) != n_utts:
         raise ValueError("one speaker label per utterance is required")
@@ -264,9 +289,7 @@ def speaker_stats_distributed_grad(feat: torch.Tensor, lay: Layout, speaker_of_u
     and the upstream dstats are all global.  The backward is collective (one all-gather of dstats, one int32 all-reduce),
     so every rank of `group` must run it, as with any data-parallel backward.  Without an initialised process group, or
     with one rank, no collective runs.  Deterministic: every rank adds dstats in rank order."""
-    _lib.require_cuda(feat)
-    if feat.dtype != torch.float32 or feat.dim() != 2 or not feat.is_contiguous():
-        raise ValueError("feat must be a contiguous (total_frames, F) float32 tensor")
+    _check_feat(feat)
     n_utts = len(lay.frame_off_host) - 1
     if len(speaker_of_utt) != n_utts:
         raise ValueError("one speaker label per utterance is required")
@@ -354,18 +377,10 @@ def normalized_windows_grad(feat: torch.Tensor, lay: Layout, st: SpeakerStats, w
                             mode: str = "znorm", win_len: int = WIN_LEN) -> torch.Tensor:
     """normalized_windows() with a gradient: bit-identical (n_windows, 1, win_len, F) windows with a grad_fn to feat and,
     when st.stats requires grad (from speaker_stats_grad), to the statistics, padded rows included (they depend on the
-    statistics).  Any window table works (subsets, any order, repeated windows); win_t0 < 0 or win_utt outside
-    [0, n_utts) raises ValueError.  Deterministic (no atomics)."""
+    statistics).  Any window table works (subsets, any order, repeated windows); win_t0 outside
+    [0, 2^31 - 1 - win_len] or win_utt outside [0, n_utts) raises ValueError.  Deterministic (no atomics)."""
     _lib.require_cuda(feat)
     if mode not in MODES:
         raise ValueError(f"mode must be one of {sorted(MODES)}")
-    wu = np.ascontiguousarray(win_utt, dtype=np.int32).reshape(-1)
-    wt = np.ascontiguousarray(win_t0, dtype=np.int32).reshape(-1)
-    n_utts = len(lay.frame_off_host) - 1
-    if len(wu) != len(wt):
-        raise ValueError("win_utt and win_t0 must have the same length")
-    if len(wt) and wt.min() < 0:
-        raise ValueError("win_t0 must be >= 0")
-    if len(wu) and (wu.min() < 0 or wu.max() >= n_utts):
-        raise ValueError(f"win_utt must lie in [0, {n_utts})")
+    wu, wt = _check_window_table(win_utt, win_t0, len(lay.frame_off_host) - 1, win_len)
     return NormalizeFunction.apply(feat, st.stats, lay, st, (wu, wt, win_len), mode)
