@@ -163,27 +163,19 @@ int sept_normalize_bwd_f32(const float* feat_dev, const int64_t* frame_off_dev, 
                            void* workspace_dev, float* dfeat_dev, float* dstats_dev, sept_stream_t stream);
 
 /* Backward of sept_speaker_stats_f32 (what torch autograd gives through the reference's stacked-rows mean, ddof-0 std,
- * min and max): dfeat = d(sum dstats * stats) / d feat for every frame (written, 0 for frames in no training window).
- * Row 0 (count) of dstats_dev is ignored.  The min / max gradient goes to the frames equal to it in proportion to their
- * window multiplicity.  Where the forward's std is exactly 0 (every weighted value of that speaker and feature equal, e.g.
- * digital silence) no gradient flows through the std (sqrt's derivative there is 0 * inf in torch).  stats_dev is the
- * forward's result; spk_of_utt_dev [n_utts] the speaker row of each utterance.  workspace_dev holds
- * sept_speaker_stats_bwd_workspace_bytes(n_utts, n_spk, n_feat) bytes, 16-byte aligned.  Deterministic, no allocation,
- * capturable. */
-size_t sept_speaker_stats_bwd_workspace_bytes(int n_utts, int n_spk, int n_feat);
-int sept_speaker_stats_bwd_f32(const float* feat_dev, const int64_t* frame_off_dev, const uint8_t* whole_dev, int n_utts,
-                               int n_feat, int win_len, int shift_len, const int32_t* spk_of_utt_dev,
-                               const int32_t* spk_ptr_dev, const int32_t* spk_utts_dev, int n_spk, const float* stats_dev,
-                               const float* dstats_dev, void* workspace_dev, float* dfeat_dev, sept_stream_t stream);
-
-/* sept_speaker_stats_bwd_f32 in its two halves, for statistics merged over several ranks (each rank holds some of a
- * speaker's utterances).  Every rank passes the merged (global) stats_dev with the same n_spk speaker rows and the CSR
- * of its own utterances over those rows (a speaker the rank does not hold is an empty range and gets tie weight 0).
+ * min and max), in two calls, on one rank or on several (each rank holding some of a speaker's utterances).  Every rank
+ * passes the same stats_dev (the forward's result; merged over the ranks when there are several) with the same n_spk
+ * speaker rows, the CSR of its own utterances over those rows (a speaker the rank does not hold is an empty range and gets
+ * tie weight 0) and spk_of_utt_dev [n_utts], the speaker row of each of its utterances.
  * _ties_i32 writes ties_dev (n_spk, 2, n_feat) int32: the summed window multiplicity of the rank's frames equal to each
  * speaker's min (row 0) and max (row 1).  workspace_dev holds sept_speaker_stats_bwd_ties_workspace_bytes(n_utts, n_feat)
- * bytes, 16-byte aligned.  Sum ties_dev over the ranks (exact in int32) and dstats_dev over the ranks, then
- * _frames_f32 writes dfeat_dev (total_frames, n_feat) like sept_speaker_stats_bwd_f32.  On one rank the two calls give
- * what sept_speaker_stats_bwd_f32 gives, bit for bit.  Deterministic, no allocation, capturable. */
+ * bytes, 16-byte aligned.  With several ranks, sum ties_dev over the ranks (exact in int32) and dstats_dev over the ranks
+ * before the second call.
+ * _frames_f32 writes dfeat_dev (total_frames, n_feat) = d(sum dstats * stats) / d feat for every frame (0 for frames in
+ * no training window).  Row 0 (count) of dstats_dev is ignored.  The min / max gradient goes to the frames equal to it in
+ * proportion to their window multiplicity (ties_dev).  Where the forward's std is exactly 0 (every weighted value of that
+ * speaker and feature equal, e.g. digital silence) no gradient flows through the std (sqrt's derivative there is 0 * inf
+ * in torch).  Deterministic, no allocation, capturable. */
 size_t sept_speaker_stats_bwd_ties_workspace_bytes(int n_utts, int n_feat);
 int sept_speaker_stats_bwd_ties_i32(const float* feat_dev, const int64_t* frame_off_dev, const uint8_t* whole_dev,
                                     int n_utts, int n_feat, int win_len, int shift_len, const int32_t* spk_of_utt_dev,

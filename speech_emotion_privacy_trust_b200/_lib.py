@@ -35,9 +35,6 @@ _SIGNATURES = {
     "sept_normalize_bwd_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
     "sept_normalize_bwd_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                          c_ptr, c_ptr, c_ptr, C.c_int, c_ptr, c_ptr, c_ptr, c_ptr]),
-    "sept_speaker_stats_bwd_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int]),
-    "sept_speaker_stats_bwd_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr, C.c_int,
-                                             c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
     "sept_speaker_stats_bwd_ties_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
     "sept_speaker_stats_bwd_ties_i32": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr,
                                                   C.c_int, c_ptr, c_ptr, c_ptr, c_ptr]),

@@ -463,32 +463,8 @@ int sept_normalize_bwd_f32(const float* feat, const int64_t* frame_off, const in
     return SEPT_OK;
 }
 
-size_t sept_speaker_stats_bwd_workspace_bytes(int n_utts, int n_spk, int n_feat) {
-    return n_utts >= 0 && n_spk >= 0 && n_feat > 0 ? sept::speaker_stats_bwd_workspace_bytes(n_utts, n_spk, n_feat) : 0;
-}
-
-int sept_speaker_stats_bwd_f32(const float* feat, const int64_t* frame_off, const uint8_t* whole, int n_utts, int n_feat,
-                               int win_len, int shift_len, const int32_t* spk_of_utt, const int32_t* spk_ptr,
-                               const int32_t* spk_utts, int n_spk, const float* stats, const float* dstats,
-                               void* workspace, float* dfeat, sept_stream_t stream) {
-    if (!feat || !frame_off || !spk_of_utt || !spk_ptr || !spk_utts || !stats || !dstats || !workspace || !dfeat ||
-        n_utts < 0 || n_spk < 0 || n_feat <= 0 || win_len <= 0 || shift_len <= 0)
-        return fail(SEPT_E_BADARG, "sept_speaker_stats_bwd_f32: bad argument");
-    if (!aligned16(workspace)) return fail(SEPT_E_BADARG, "sept_speaker_stats_bwd_f32: workspace must be 16-byte aligned");
-    sept::SpeakerStatsBwdParams p{};
-    p.f.feat = feat; p.f.frame_off = frame_off; p.f.whole = whole; p.f.n_utts = n_utts; p.f.n_feat = n_feat;
-    p.f.win_len = win_len; p.f.shift_len = shift_len; p.f.spk_ptr = spk_ptr; p.f.spk_utts = spk_utts; p.f.n_spk = n_spk;
-    p.f.stats = const_cast<float*>(stats);
-    p.spk_of_utt = spk_of_utt; p.dstats = dstats; p.dfeat = dfeat;
-    unsigned char* ws = static_cast<unsigned char*>(workspace);
-    p.utt_ties = reinterpret_cast<int32_t*>(ws);
-    p.spk_ties = reinterpret_cast<int32_t*>(ws + sept::speaker_stats_bwd_ties_offset(n_utts, n_feat));
-    SEPT_CUDA(sept::launch_speaker_stats_bwd(p, static_cast<cudaStream_t>(stream)));
-    return SEPT_OK;
-}
-
 size_t sept_speaker_stats_bwd_ties_workspace_bytes(int n_utts, int n_feat) {
-    return n_utts >= 0 && n_feat > 0 ? sept::speaker_stats_bwd_ties_offset(n_utts, n_feat) : 0;
+    return n_utts >= 0 && n_feat > 0 ? sept::speaker_stats_bwd_ties_workspace_bytes(n_utts, n_feat) : 0;
 }
 
 int sept_speaker_stats_bwd_ties_i32(const float* feat, const int64_t* frame_off, const uint8_t* whole, int n_utts,

@@ -382,9 +382,4 @@ cudaError_t launch_speaker_stats_bwd_frames(const SpeakerStatsBwdParams& p, cuda
     return cudaGetLastError();
 }
 
-cudaError_t launch_speaker_stats_bwd(const SpeakerStatsBwdParams& p, cudaStream_t stream) {
-    const cudaError_t e = launch_speaker_stats_bwd_ties(p, stream);
-    return e != cudaSuccess ? e : launch_speaker_stats_bwd_frames(p, stream);
-}
-
 }  // namespace sept

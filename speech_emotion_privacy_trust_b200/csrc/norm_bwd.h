@@ -29,19 +29,16 @@ struct SpeakerStatsBwdParams {
     const int32_t* spk_of_utt;   // [n_utts]
     const float* dstats;         // (n_spk, 5, F); row 0 (count) is ignored
     int32_t* utt_ties;           // workspace (n_utts, 2, F): tie weight of the speaker's min / max in the utterance
-    int32_t* spk_ties;           // workspace (n_spk, 2, F), or the caller's buffer when the two halves run apart
+    int32_t* spk_ties;           // (n_spk, 2, F), the caller's: written by the ties half, read by the frames half
     float* dfeat;                // (total_frames, F)
 };
 
 // workspace of the normalisation backward: the per-utterance (S1, S2) partials
 inline size_t normalize_bwd_workspace_bytes(int n_utts, int n_feat) { return (size_t)n_utts * 2 * n_feat * sizeof(float); }
 
-// workspace of the statistics backward: utterance tie weights, then (16-byte aligned) speaker tie weights
-inline size_t speaker_stats_bwd_ties_offset(int n_utts, int n_feat) {
+// workspace of the statistics backward's ties half: the utterance tie weights, rounded up to 16 bytes
+inline size_t speaker_stats_bwd_ties_workspace_bytes(int n_utts, int n_feat) {
     return ((size_t)n_utts * 2 * n_feat * sizeof(int32_t) + 15) & ~(size_t)15;
-}
-inline size_t speaker_stats_bwd_workspace_bytes(int n_utts, int n_spk, int n_feat) {
-    return speaker_stats_bwd_ties_offset(n_utts, n_feat) + (size_t)n_spk * 2 * n_feat * sizeof(int32_t);
 }
 
 cudaError_t launch_normalize_bwd(const NormalizeBwdParams& p, cudaStream_t stream);
@@ -49,6 +46,5 @@ cudaError_t launch_normalize_bwd(const NormalizeBwdParams& p, cudaStream_t strea
 // ties (passes 1 and 2: utt_ties -> spk_ties; dstats and dfeat unused) and frames (pass 3: spk_ties -> dfeat)
 cudaError_t launch_speaker_stats_bwd_ties(const SpeakerStatsBwdParams& p, cudaStream_t stream);
 cudaError_t launch_speaker_stats_bwd_frames(const SpeakerStatsBwdParams& p, cudaStream_t stream);
-cudaError_t launch_speaker_stats_bwd(const SpeakerStatsBwdParams& p, cudaStream_t stream);   // ties, then frames
 
 }  // namespace sept

@@ -26,7 +26,7 @@ class SpeakerStats:
     speakers: list                 # speaker labels, row order of `stats`
     stats: torch.Tensor            # device (n_spk, 5, F): count, mean, std (ddof 0), min, max
     spk_of_utt: torch.Tensor       # device int32 [n_utts] row index per utterance
-    spk_of_utt_host: np.ndarray | None = None   # host copy of spk_of_utt: a backward builds its speaker lists from it
+    spk_lists: tuple | None = None  # device CSR (spk_ptr, spk_utts) the statistics were built with; a backward reuses it
 
     def as_dict(self) -> dict:
         h = self.stats.detach().cpu().numpy()
@@ -69,18 +69,32 @@ def speaker_stats(feat: torch.Tensor, lay: Layout, speaker_of_utt: Sequence, who
                   win_len: int = WIN_LEN, shift_len: int = SHIFT_LEN) -> SpeakerStats:
     """Weighted per-speaker mean/std/min/max: a frame inside k training windows counts k times (:26-27), utterances
     flagged whole (test split, :56-60) count each frame once."""
+    speakers, d_spk, spk_lists, d_whole = _speaker_table(feat, lay, speaker_of_utt, whole_utterance)
+    stats = _launch_speaker_stats(feat, lay, d_whole, win_len, shift_len, spk_lists)
+    return SpeakerStats(speakers, stats, d_spk, spk_lists)
+
+
+def _speaker_table(feat: torch.Tensor, lay: Layout, speaker_of_utt: Sequence, whole_utterance: Sequence[bool] | None,
+                   speakers: Sequence | None = None):
+    """What every statistics entry sets up: checks feat and the labels, gives each speaker a row (in first-seen order, or
+    in the order of `speakers`, which must hold every label) and returns (speaker rows, device int32 row of each
+    utterance, its device CSR, device whole-utterance flags or None)."""
     _check_feat(feat)
     n_utts = len(lay.frame_off_host) - 1
     if len(speaker_of_utt) != n_utts:
         raise ValueError("one speaker label per utterance is required")
-    speakers = list(dict.fromkeys(speaker_of_utt))
+    if speakers is None:
+        speakers = list(dict.fromkeys(speaker_of_utt))
+    else:
+        speakers = list(speakers)
+        missing = set(speaker_of_utt) - set(speakers)
+        if missing:
+            raise ValueError(f"speakers missing from all_speakers: {sorted(map(str, missing))}")
     row = {s: i for i, s in enumerate(speakers)}
     spk_idx = np.fromiter((row[s] for s in speaker_of_utt), dtype=np.int32, count=n_utts)
     dev = feat.device
-    d_ptr, d_order = _speaker_lists(spk_idx, len(speakers), dev)
     d_whole = None if whole_utterance is None else torch.from_numpy(np.asarray(whole_utterance, dtype=np.uint8)).to(dev)
-    stats = _launch_speaker_stats(feat, lay, d_whole, win_len, shift_len, d_ptr, d_order, len(speakers))
-    return SpeakerStats(speakers, stats, torch.from_numpy(spk_idx).to(dev), spk_idx)
+    return speakers, torch.from_numpy(spk_idx).to(dev), _speaker_lists(spk_idx, len(speakers), dev), d_whole
 
 
 def _speaker_lists(spk_idx: np.ndarray, n_spk: int, dev):
@@ -91,9 +105,12 @@ def _speaker_lists(spk_idx: np.ndarray, n_spk: int, dev):
     return torch.from_numpy(ptr).to(dev), torch.from_numpy(order).to(dev)
 
 
-def _launch_speaker_stats(feat, lay, d_whole, win_len, shift_len, d_ptr, d_order, n_spk) -> torch.Tensor:
+def _launch_speaker_stats(feat, lay, d_whole, win_len, shift_len, spk_lists) -> torch.Tensor:
+    """(n_spk, 5, F) statistics of the rows of the CSR spk_lists; a row with no utterance gets count, mean and std 0,
+    min FLT_MAX and max -FLT_MAX."""
     dev = feat.device
-    n_utts, F = len(lay.frame_off_host) - 1, feat.shape[1]
+    d_ptr, d_order = spk_lists
+    n_utts, n_spk, F = len(lay.frame_off_host) - 1, d_ptr.numel() - 1, feat.shape[1]
     partial = torch.empty((n_utts, 5, F), dtype=torch.float32, device=dev)
     stats = torch.empty((n_spk, 5, F), dtype=torch.float32, device=dev)
     with torch.cuda.device(dev):
@@ -156,63 +173,66 @@ def speaker_stats_distributed(feat: torch.Tensor, lay: Layout, speaker_of_utt: S
     sharding, SURVEY 8e): every rank reduces its own utterances with the kernels, then ONE all-gather of the
     (count, mean, M2, min, max) partials and a Chan merge in rank order give every rank the global statistics.
     `all_speakers` fixes the row order on every rank (speakers a rank does not hold contribute empty partials)."""
-    local = speaker_stats(feat, lay, speaker_of_utt, whole_utterance, win_len, shift_len)
-    stats = _merge_ranks(local, all_speakers, group)
-    spk_idx = _rows_of(speaker_of_utt, all_speakers)
-    return SpeakerStats(list(all_speakers), stats, torch.from_numpy(spk_idx).to(feat.device), spk_idx)
+    speakers, d_spk, spk_lists, d_whole = _speaker_table(feat, lay, speaker_of_utt, whole_utterance, all_speakers)
+    stats = _merge_ranks(_launch_speaker_stats(feat, lay, d_whole, win_len, shift_len, spk_lists), spk_lists[0], group)
+    return SpeakerStats(speakers, stats, d_spk, spk_lists)
 
 
-def _rows_of(speaker_of_utt: Sequence, all_speakers: Sequence) -> np.ndarray:
-    row = {s: i for i, s in enumerate(all_speakers)}
-    return np.array([row[s] for s in speaker_of_utt], dtype=np.int32)
-
-
-def _merge_ranks(local: SpeakerStats, all_speakers: Sequence, group) -> torch.Tensor:
-    """The rank's own statistics -> the global (len(all_speakers), 5, F) ones: one all-gather and a Chan merge in rank
-    order (parallel.merge_speaker_partials)."""
+def _merge_ranks(stats: torch.Tensor, spk_ptr: torch.Tensor, group) -> torch.Tensor:
+    """The rank's (n_spk, 5, F) statistics over the shared speaker rows (CSR pointer spk_ptr) -> the global ones: one
+    all-gather and a Chan merge in rank order (parallel.merge_speaker_partials).  A speaker the rank does not hold enters
+    with min +inf and max -inf, so a speaker no rank holds ends as (0, 0, 0, +inf, -inf)."""
     from . import parallel
-    dev, F = local.stats.device, local.stats.shape[2]
-    row = {s: i for i, s in enumerate(all_speakers)}
-    n_spk = len(all_speakers)
-    cnt = torch.zeros((n_spk, F), dtype=torch.float32, device=dev)
-    mean, m2 = torch.zeros_like(cnt), torch.zeros_like(cnt)
-    mn, mx = torch.full_like(cnt, float("inf")), torch.full_like(cnt, float("-inf"))
-    if local.speakers:
-        idx = torch.tensor([row[s] for s in local.speakers], device=dev)
-        st = local.stats
-        cnt[idx], mean[idx], m2[idx] = st[:, 0], st[:, 1], st[:, 2] * st[:, 2] * st[:, 0]
-        mn[idx], mx[idx] = st[:, 3], st[:, 4]
-    n, mu, sd, lo, hi = parallel.merge_speaker_partials(cnt, mean, m2, mn, mx, group=group)
+    held = (spk_ptr[1:] > spk_ptr[:-1]).unsqueeze(1)
+    cnt, mean, sd = stats[:, 0], stats[:, 1], stats[:, 2]
+    mn, mx = torch.where(held, stats[:, 3], float("inf")), torch.where(held, stats[:, 4], float("-inf"))
+    n, mu, sd, lo, hi = parallel.merge_speaker_partials(cnt, mean, sd * sd * cnt, mn, mx, group=group)
     return torch.stack([n, mu, sd, lo, hi], dim=1).contiguous()
 
 
 # ---- gradients: the same forward launches, with a grad_fn to feat (and to the statistics) ------------------------
 class SpeakerStatsFunction(torch.autograd.Function):
-    """speaker_stats() with a gradient to feat: forward is the sept_speaker_stats_f32 launch of speaker_stats(), backward
-    one sept_speaker_stats_bwd_f32 call (the count row gets no gradient; no double backward)."""
+    """speaker_stats() or speaker_stats_distributed() with a gradient to (this rank's) feat.  Forward: the
+    sept_speaker_stats_f32 launch over the given speaker rows, then, when distributed, the all-gather and Chan merge.
+    Backward: when distributed, dstats summed over the ranks in rank order (one all-gather); the rank's min / max tie
+    weights against the statistics (sept_speaker_stats_bwd_ties_i32); when distributed, one exact int32 SUM all-reduce of
+    them; then sept_speaker_stats_bwd_frames_f32.  The count row gets no gradient; no double backward.  `distributed`,
+    not `group`, selects the collectives: group None is the default world group, and the local path must run none even
+    when a process group is initialised."""
 
     @staticmethod
-    def forward(ctx, feat, lay, d_whole, win_len, shift_len, spk_of_utt, d_ptr, d_order, n_spk):
-        stats = _launch_speaker_stats(feat, lay, d_whole, win_len, shift_len, d_ptr, d_order, n_spk)
+    def forward(ctx, feat, lay, d_whole, win_len, shift_len, d_spk, spk_lists, distributed, group):
+        stats = _launch_speaker_stats(feat, lay, d_whole, win_len, shift_len, spk_lists)
+        if distributed:
+            stats = _merge_ranks(stats, spk_lists[0], group)
         ctx.save_for_backward(feat, stats)
-        ctx.cfg = (lay, d_whole, win_len, shift_len, spk_of_utt, d_ptr, d_order, n_spk)
+        ctx.cfg = (lay, d_whole, win_len, shift_len, d_spk, spk_lists, distributed, group)
         return stats
 
     @staticmethod
     @once_differentiable
     def backward(ctx, dstats):
+        from . import parallel
         feat, stats = ctx.saved_tensors
-        lay, d_whole, win_len, shift_len, spk_of_utt, d_ptr, d_order, n_spk = ctx.cfg
+        lay, d_whole, win_len, shift_len, d_spk, (d_ptr, d_order), distributed, group = ctx.cfg
         lib = _lib.lib()
-        dev, n_utts, F = feat.device, len(lay.frame_off_host) - 1, feat.shape[1]
-        dfeat = torch.empty_like(feat)
-        ws = torch.empty(max(16, lib.sept_speaker_stats_bwd_workspace_bytes(n_utts, n_spk, F)), dtype=torch.uint8, device=dev)
+        dev, n_utts, n_spk, F = feat.device, len(lay.frame_off_host) - 1, stats.shape[0], feat.shape[1]
         dstats = dstats.contiguous()
+        if distributed:
+            dstats = parallel.sum_in_rank_order(dstats, group)
+        ties = torch.empty((n_spk, 2, F), dtype=torch.int32, device=dev)
+        ws = torch.empty(max(16, lib.sept_speaker_stats_bwd_ties_workspace_bytes(n_utts, F)), dtype=torch.uint8, device=dev)
+        dfeat = torch.empty_like(feat)
+        whole = 0 if d_whole is None else d_whole.data_ptr()
         with torch.cuda.device(dev):
-            _lib.check(lib.sept_speaker_stats_bwd_f32(
-                feat.data_ptr(), lay.frame_off.data_ptr(), 0 if d_whole is None else d_whole.data_ptr(), n_utts, F, win_len,
-                shift_len, spk_of_utt.data_ptr(), d_ptr.data_ptr(), d_order.data_ptr(), n_spk, stats.data_ptr(),
-                dstats.data_ptr(), ws.data_ptr(), dfeat.data_ptr(), _stream(dev)))
+            _lib.check(lib.sept_speaker_stats_bwd_ties_i32(
+                feat.data_ptr(), lay.frame_off.data_ptr(), whole, n_utts, F, win_len, shift_len, d_spk.data_ptr(),
+                d_ptr.data_ptr(), d_order.data_ptr(), n_spk, stats.data_ptr(), ws.data_ptr(), ties.data_ptr(), _stream(dev)))
+            if distributed:
+                parallel.allreduce_exact_sum(ties, group)
+            _lib.check(lib.sept_speaker_stats_bwd_frames_f32(
+                feat.data_ptr(), lay.frame_off.data_ptr(), whole, n_utts, F, win_len, shift_len, d_spk.data_ptr(),
+                stats.data_ptr(), dstats.data_ptr(), ties.data_ptr(), dfeat.data_ptr(), _stream(dev)))
         return dfeat, None, None, None, None, None, None, None, None
 
 
@@ -225,58 +245,9 @@ def speaker_stats_grad(feat: torch.Tensor, lay: Layout, speaker_of_utt: Sequence
     mean and ddof-0 std of the weighted frames, min / max split over tied frames in proportion to their multiplicity.
     The count row gets none; where the std is exactly 0 (a constant feature column) none flows through the std.
     Deterministic (no atomics)."""
-    _check_feat(feat)
-    n_utts = len(lay.frame_off_host) - 1
-    if len(speaker_of_utt) != n_utts:
-        raise ValueError("one speaker label per utterance is required")
-    speakers = list(dict.fromkeys(speaker_of_utt))
-    row = {s: i for i, s in enumerate(speakers)}
-    spk_idx = np.fromiter((row[s] for s in speaker_of_utt), dtype=np.int32, count=n_utts)
-    dev = feat.device
-    d_ptr, d_order = _speaker_lists(spk_idx, len(speakers), dev)
-    d_whole = None if whole_utterance is None else torch.from_numpy(np.asarray(whole_utterance, dtype=np.uint8)).to(dev)
-    d_spk = torch.from_numpy(spk_idx).to(dev)
-    stats = SpeakerStatsFunction.apply(feat, lay, d_whole, win_len, shift_len, d_spk, d_ptr, d_order, len(speakers))
-    return SpeakerStats(speakers, stats, d_spk, spk_idx)
-
-
-class SpeakerStatsDistributedFunction(torch.autograd.Function):
-    """speaker_stats_distributed() with a gradient to this rank's feat.  Forward: the local launch, all-gather and Chan
-    merge of speaker_stats_distributed().  Backward: dstats summed over the ranks in rank order (one all-gather), the
-    rank's min / max tie weights against the global statistics (sept_speaker_stats_bwd_ties_i32), one exact int32 SUM
-    all-reduce of them, then sept_speaker_stats_bwd_frames_f32 (no double backward)."""
-
-    @staticmethod
-    def forward(ctx, feat, lay, speaker_of_utt, all_speakers, whole_utterance, group, win_len, shift_len, d_whole, d_spk,
-                d_ptr, d_order):
-        local = speaker_stats(feat, lay, speaker_of_utt, whole_utterance, win_len, shift_len)
-        stats = _merge_ranks(local, all_speakers, group)
-        ctx.save_for_backward(feat, stats)
-        ctx.cfg = (lay, group, win_len, shift_len, d_whole, d_spk, d_ptr, d_order)
-        return stats
-
-    @staticmethod
-    @once_differentiable
-    def backward(ctx, dstats):
-        from . import parallel
-        feat, stats = ctx.saved_tensors
-        lay, group, win_len, shift_len, d_whole, d_spk, d_ptr, d_order = ctx.cfg
-        lib = _lib.lib()
-        dev, n_utts, n_spk, F = feat.device, len(lay.frame_off_host) - 1, stats.shape[0], feat.shape[1]
-        dstats = parallel.sum_in_rank_order(dstats.contiguous(), group)
-        ties = torch.empty((n_spk, 2, F), dtype=torch.int32, device=dev)
-        ws = torch.empty(max(16, lib.sept_speaker_stats_bwd_ties_workspace_bytes(n_utts, F)), dtype=torch.uint8, device=dev)
-        dfeat = torch.empty_like(feat)
-        whole = 0 if d_whole is None else d_whole.data_ptr()
-        with torch.cuda.device(dev):
-            _lib.check(lib.sept_speaker_stats_bwd_ties_i32(
-                feat.data_ptr(), lay.frame_off.data_ptr(), whole, n_utts, F, win_len, shift_len, d_spk.data_ptr(),
-                d_ptr.data_ptr(), d_order.data_ptr(), n_spk, stats.data_ptr(), ws.data_ptr(), ties.data_ptr(), _stream(dev)))
-            parallel.allreduce_exact_sum(ties, group)
-            _lib.check(lib.sept_speaker_stats_bwd_frames_f32(
-                feat.data_ptr(), lay.frame_off.data_ptr(), whole, n_utts, F, win_len, shift_len, d_spk.data_ptr(),
-                stats.data_ptr(), dstats.data_ptr(), ties.data_ptr(), dfeat.data_ptr(), _stream(dev)))
-        return dfeat, None, None, None, None, None, None, None, None, None, None, None
+    speakers, d_spk, spk_lists, d_whole = _speaker_table(feat, lay, speaker_of_utt, whole_utterance)
+    stats = SpeakerStatsFunction.apply(feat, lay, d_whole, win_len, shift_len, d_spk, spk_lists, False, None)
+    return SpeakerStats(speakers, stats, d_spk, spk_lists)
 
 
 def speaker_stats_distributed_grad(feat: torch.Tensor, lay: Layout, speaker_of_utt: Sequence, all_speakers: Sequence,
@@ -289,31 +260,20 @@ def speaker_stats_distributed_grad(feat: torch.Tensor, lay: Layout, speaker_of_u
     and the upstream dstats are all global.  The backward is collective (one all-gather of dstats, one int32 all-reduce),
     so every rank of `group` must run it, as with any data-parallel backward.  Without an initialised process group, or
     with one rank, no collective runs.  Deterministic: every rank adds dstats in rank order."""
-    _check_feat(feat)
-    n_utts = len(lay.frame_off_host) - 1
-    if len(speaker_of_utt) != n_utts:
-        raise ValueError("one speaker label per utterance is required")
-    missing = set(speaker_of_utt) - set(all_speakers)
-    if missing:
-        raise ValueError(f"speakers missing from all_speakers: {sorted(map(str, missing))}")
-    spk_idx = _rows_of(speaker_of_utt, all_speakers)
-    dev = feat.device
-    d_ptr, d_order = _speaker_lists(spk_idx, len(all_speakers), dev)
-    d_whole = None if whole_utterance is None else torch.from_numpy(np.asarray(whole_utterance, dtype=np.uint8)).to(dev)
-    d_spk = torch.from_numpy(spk_idx).to(dev)
-    stats = SpeakerStatsDistributedFunction.apply(feat, lay, speaker_of_utt, all_speakers, whole_utterance, group, win_len,
-                                                  shift_len, d_whole, d_spk, d_ptr, d_order)
-    return SpeakerStats(list(all_speakers), stats, d_spk, spk_idx)
+    speakers, d_spk, spk_lists, d_whole = _speaker_table(feat, lay, speaker_of_utt, whole_utterance, all_speakers)
+    stats = SpeakerStatsFunction.apply(feat, lay, d_whole, win_len, shift_len, d_spk, spk_lists, True, group)
+    return SpeakerStats(speakers, stats, d_spk, spk_lists)
 
 
 class NormalizeFunction(torch.autograd.Function):
     """normalize() (win is None) or normalized_windows() with gradients to feat and to the statistics: forward is the
-    existing launch, backward one sept_normalize_bwd_f32 call.  The host tables the backward needs (each utterance's
-    windows sorted by start, each speaker's utterances) are built here, so the backward launches kernels only."""
+    existing launch, backward one sept_normalize_bwd_f32 call.  The tables the backward needs (each utterance's windows
+    sorted by start, built here; each speaker's utterances, the statistics' CSR) are on the device before it, so the
+    backward launches kernels only."""
 
     @staticmethod
     def forward(ctx, feat, stats, lay, st, win, mode):
-        st_fwd = SpeakerStats(st.speakers, stats, st.spk_of_utt, st.spk_of_utt_host)
+        st_fwd = SpeakerStats(st.speakers, stats, st.spk_of_utt, st.spk_lists)
         n_utts = len(lay.frame_off_host) - 1
         dev = feat.device
         if win is None:
@@ -327,10 +287,9 @@ class NormalizeFunction(torch.autograd.Function):
             np.cumsum(np.bincount(wu, minlength=n_utts), out=ptr[1:])
             tables = (torch.from_numpy(wt).to(dev), torch.from_numpy(ptr).to(dev), torch.from_numpy(order).to(dev),
                       len(wu), win_len)
-        spk_lists = None
-        if ctx.needs_input_grad[1]:
-            spk_idx = st.spk_of_utt_host if st.spk_of_utt_host is not None else st.spk_of_utt.cpu().numpy()
-            spk_lists = _speaker_lists(np.asarray(spk_idx, dtype=np.int32), stats.shape[0], dev)
+        spk_lists = st.spk_lists
+        if ctx.needs_input_grad[1] and spk_lists is None:                     # a SpeakerStats built by hand
+            spk_lists = _speaker_lists(np.asarray(st.spk_of_utt.cpu().numpy(), dtype=np.int32), stats.shape[0], dev)
         ctx.save_for_backward(feat, stats)
         ctx.cfg = (lay, st.spk_of_utt, tables, spk_lists, MODES[mode])
         return out

@@ -211,7 +211,8 @@ def test_distributed_speaker_stats_single_rank_equals_local():
     for s in ("x", "y", "z"):
         for k in ("count", "mean", "std", "min", "max"):
             assert np.allclose(da[s][k], db[s][k], rtol=0, atol=2e-5), (s, k)
-    assert float(db["absent"]["count"][0]) == 0.0
+    for k, want in (("count", 0.0), ("mean", 0.0), ("std", 0.0), ("min", np.inf), ("max", -np.inf)):
+        assert np.all(db["absent"][k] == want), (k, db["absent"][k])       # in every feature of the row no rank holds
     za, zb = nz.normalize(feat, lay, a), nz.normalize(feat, lay, b)
     assert float((za - zb).abs().max()) < 1e-4
 

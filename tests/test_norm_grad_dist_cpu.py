@@ -52,8 +52,6 @@ def test_ties_workspace_bytes():
     assert lib.sept_speaker_stats_bwd_ties_workspace_bytes(0, 128) == 0
     assert lib.sept_speaker_stats_bwd_ties_workspace_bytes(-1, 128) == 0
     assert lib.sept_speaker_stats_bwd_ties_workspace_bytes(4, 0) == 0
-    # the split workspace is the head of the one-call workspace (its utterance tie weights)
-    assert lib.sept_speaker_stats_bwd_ties_workspace_bytes(7, 37) < lib.sept_speaker_stats_bwd_workspace_bytes(7, 2, 37)
 
 
 @pytest.mark.parametrize("bad", [dict(feat=None), dict(frame_off=None), dict(spk=None), dict(ptr=None), dict(utts=None),

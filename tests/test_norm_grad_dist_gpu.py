@@ -153,9 +153,10 @@ def test_one_device_matches_speaker_stats_grad(kind, mode, form):
         assert _rel(g[u], oracle[u]) < 1e-5, (u, _rel(g[u], oracle[u]))
 
 
-def test_split_entries_equal_the_one_call_backward():
-    """sept_speaker_stats_bwd_ties_i32 + sept_speaker_stats_bwd_frames_f32 give sept_speaker_stats_bwd_f32's dfeat bit for
-    bit (n_feat 128: the vector kernels; 37: the scalar ones)."""
+def test_backward_halves_write_every_element():
+    """sept_speaker_stats_bwd_ties_i32 + sept_speaker_stats_bwd_frames_f32 called directly (n_feat 128: the vector
+    kernels; 37: the scalar ones) write every element of ties and dfeat, count every speaker's min and max at least once
+    on the tie-heavy corpus, and give speaker_stats_grad's feature gradient bit for bit."""
     from speech_emotion_privacy_trust_b200 import _lib
     from speech_emotion_privacy_trust_b200 import normalization as nz
     from speech_emotion_privacy_trust_b200.extraction import _stream
@@ -165,32 +166,28 @@ def test_split_entries_equal_the_one_call_backward():
         feats, spk, whole = _corpus("ties")
         feats = [f[:, :n_feat].copy() for f in feats]
         lay = _layout(feats, "cuda")
-        feat = torch.from_numpy(np.concatenate(feats)).cuda()
-        st = nz.speaker_stats(feat, lay, spk, whole)
-        d_ptr, d_order = nz._speaker_lists(st.spk_of_utt_host, len(st.speakers), feat.device)
+        feat = torch.from_numpy(np.concatenate(feats)).cuda().requires_grad_(True)
+        st = nz.speaker_stats_grad(feat, lay, spk, whole)
+        d_ptr, d_order = st.spk_lists
         d_whole = torch.from_numpy(np.asarray(whole, dtype=np.uint8)).cuda()
-        dstats = torch.from_numpy(rng.standard_normal(st.stats.shape).astype(np.float32)).cuda()
+        stats = st.stats.detach()
+        dstats = torch.from_numpy(rng.standard_normal(stats.shape).astype(np.float32)).cuda()
         n_spk, s = len(st.speakers), _stream(feat.device)
-        one = torch.empty_like(feat)
-        ws = torch.empty(lib.sept_speaker_stats_bwd_workspace_bytes(N_UTTS, n_spk, n_feat), dtype=torch.uint8, device="cuda")
-        _lib.check(lib.sept_speaker_stats_bwd_f32(
-            feat.data_ptr(), lay.frame_off.data_ptr(), d_whole.data_ptr(), N_UTTS, n_feat, 200, 50, st.spk_of_utt.data_ptr(),
-            d_ptr.data_ptr(), d_order.data_ptr(), n_spk, st.stats.data_ptr(), dstats.data_ptr(), ws.data_ptr(),
-            one.data_ptr(), s))
         ties = torch.full((n_spk, 2, n_feat), -7, dtype=torch.int32, device="cuda")
-        ws2 = torch.empty(lib.sept_speaker_stats_bwd_ties_workspace_bytes(N_UTTS, n_feat), dtype=torch.uint8, device="cuda")
+        ws = torch.empty(lib.sept_speaker_stats_bwd_ties_workspace_bytes(N_UTTS, n_feat), dtype=torch.uint8,
+                         device="cuda")
         _lib.check(lib.sept_speaker_stats_bwd_ties_i32(
             feat.data_ptr(), lay.frame_off.data_ptr(), d_whole.data_ptr(), N_UTTS, n_feat, 200, 50,
-            st.spk_of_utt.data_ptr(), d_ptr.data_ptr(), d_order.data_ptr(), n_spk, st.stats.data_ptr(), ws2.data_ptr(),
+            st.spk_of_utt.data_ptr(), d_ptr.data_ptr(), d_order.data_ptr(), n_spk, stats.data_ptr(), ws.data_ptr(),
             ties.data_ptr(), s))
-        two = torch.empty_like(feat)
+        dfeat = torch.full(feat.shape, -7.0, device="cuda")
         _lib.check(lib.sept_speaker_stats_bwd_frames_f32(
             feat.data_ptr(), lay.frame_off.data_ptr(), d_whole.data_ptr(), N_UTTS, n_feat, 200, 50,
-            st.spk_of_utt.data_ptr(), st.stats.data_ptr(), dstats.data_ptr(), ties.data_ptr(), two.data_ptr(), s))
-        assert torch.equal(one, two), n_feat
-        assert torch.all(ties >= 1)                          # every speaker's min and max is attained by a weighted frame
-        spk_tail = ws[lib.sept_speaker_stats_bwd_ties_workspace_bytes(N_UTTS, n_feat):].view(torch.int32)
-        assert torch.equal(spk_tail[:n_spk * 2 * n_feat].view(n_spk, 2, n_feat), ties)
+            st.spk_of_utt.data_ptr(), stats.data_ptr(), dstats.data_ptr(), ties.data_ptr(), dfeat.data_ptr(), s))
+        assert torch.all(ties >= 1), n_feat                  # every speaker's min and max is attained by a weighted frame
+        assert not torch.any(dfeat == -7), n_feat
+        st.stats.backward(dstats)
+        assert torch.equal(feat.grad, dfeat), n_feat
 
 
 # ---- several devices -------------------------------------------------------------------------------------------------
@@ -228,8 +225,10 @@ def _features_worker(rank, world, init_file, out_dir, backend, sharding):
             key = f"{kind}|{mode}|{form}"
             res[f"{key}|fwd_equal"] = np.array(torch.equal(st.stats.detach(), ref.stats))
             res[f"{key}|bwd_twice_equal"] = np.array(all(np.array_equal(a, b) for a, b in zip(g, g2)))
+            gl, _, _ = _grads(kind, mine, mode, form, dev, _union_stats)     # the local entry, under the process group
             for i, u in enumerate(mine):
                 res[f"{key}|{u}"] = g[i]
+                res[f"{key}|local|{u}"] = gl[i]
             if kind == "const":                              # the std path alone: exactly nothing for the silent column
                 feat.requires_grad_(True)
                 st = nz.speaker_stats_distributed_grad(feat, lay, ss, ALL_SPEAKERS, sw)
@@ -265,11 +264,14 @@ def test_ranks_match_the_one_gpu_union(backend, world, sharding, tmp_path):
         for r in res:
             assert r[f"{key}|fwd_equal"], (key, "forward differs from speaker_stats_distributed")
             assert r[f"{key}|bwd_twice_equal"], (key, "two backwards differ")
-            for u in r["mine"]:
+            # speaker_stats_grad on a rank is that rank's own gradient: it runs no collective, even under a process group
+            local = _grads(kind, list(r["mine"]), mode, form, torch.device("cuda", 0), _union_stats)[0]
+            for i, u in enumerate(r["mine"]):
                 g = r[f"{key}|{u}"]
                 assert np.all(np.isfinite(g)), (key, u)
                 assert _rel(g, union[u]) < 1e-5, (key, u, _rel(g, union[u]))
                 assert _rel(g, oracle[u]) < 1e-5, (key, u, _rel(g, oracle[u]))
+                assert torch.equal(torch.from_numpy(r[f"{key}|local|{u}"]), torch.from_numpy(local[i])), (key, u)
     for r in res:
         assert r["const|std_is_zero"] and r["const|std_only|col5_zero"] and r["const|std_only|finite"]
 

@@ -1,7 +1,7 @@
 """Gradient through the per-speaker statistics and normalised training windows (normalization.speaker_stats_grad /
-normalized_windows_grad / normalize_grad, sept_speaker_stats_bwd_f32 / sept_normalize_bwd_f32) on the GPU, against the
-float64 torch autograd oracle (oracle/norm_autograd.py) on the same fp32 features.  Metric: rel = |g - g64| / |g64| per
-utterance, with a random normal upstream gradient."""
+normalized_windows_grad / normalize_grad; sept_speaker_stats_bwd_ties_i32 + _frames_f32, sept_normalize_bwd_f32) on the
+GPU, against the float64 torch autograd oracle (oracle/norm_autograd.py) on the same fp32 features.  Metric:
+rel = |g - g64| / |g64| per utterance, with a random normal upstream gradient."""
 import numpy as np
 import pytest
 import torch
