@@ -218,6 +218,33 @@ int sept_cloak_grl_bwd_f32(const float* g_a_dev, const float* g_b_dev, float lam
 /* Backward of GradientReversalFunction (model/reversal_gradient.py:19-23): dx = -lambda * g. */
 int sept_grl_bwd_f32(const float* g_dev, float lambda, int64_t n, float* dx_dev, sept_stream_t stream);
 
+/* ---- waveform-domain cloak ----------------------------------------------------------------------------------------
+ * The signal-domain counterpart of cloak_noise: a learned noise of `period` samples (noise = locs + sigma(rhos) * eps,
+ * drawn by sept_cloak_fwd_f32 with batch = 0, wf = period) is tiled over every utterance of a ragged batch from the
+ * utterance's first sample: y[s] = x[s] + noise[(s - utt_off[u]) mod period].  Tile k of utterance u is its period
+ * utt_off[u] + k*period .. + period, clipped to the utterance.  period must be a multiple of 4; every utterance must be
+ * shorter than 2^31 samples and 0 <= utt_off[0] <= ... <= utt_off[n_utts] <= n_samples (sept_wave_cloak_layout checks
+ * both on the host). */
+
+/* HOST helper: tile_off_host[n_utts+1], the tiles of utterance u being tile_off[u] .. tile_off[u+1]-1
+ * (ceil(length / period) each); validates the offsets as above. */
+int sept_wave_cloak_layout(const int64_t* utt_off_host, int n_utts, int period, int64_t* tile_off_host);
+
+/* y = x + noise tiled over every utterance; samples before utt_off[0] and from utt_off[n_utts] to n_samples are copied.
+ * x_dev, y_dev (n_samples) and noise_dev (period) 16-byte aligned. */
+int sept_wave_cloak_fwd_f32(const float* x_dev, const int64_t* utt_off_dev, int n_utts, int64_t n_samples,
+                            const float* noise_dev, int period, float* y_dev, sept_stream_t stream);
+
+/* Backward of sept_wave_cloak_fwd_f32 with respect to the noise: r[j] = the sum of g over every in-utterance sample of
+ * phase j, r_dev (period).  dx = g needs no call; dlocs = r and drhos = r * eps * dsigma/drho follow from
+ * sept_cloak_grl_bwd_f32(g_a = r, batch = 1, mask = NULL).  tile_off_dev is sept_wave_cloak_layout's table on the device,
+ * n_tiles = tile_off[n_utts].  workspace_dev holds sept_wave_cloak_bwd_workspace_bytes(period) bytes (592 partial rows
+ * of the period, 16-byte aligned); g_dev and r_dev 16-byte aligned.  Deterministic: no atomics, a fixed summation order
+ * that does not depend on the GPU (DESIGN 3.3b); no allocation, capturable. */
+size_t sept_wave_cloak_bwd_workspace_bytes(int period);
+int sept_wave_cloak_bwd_f32(const float* g_dev, const int64_t* utt_off_dev, const int64_t* tile_off_dev, int n_utts,
+                            int64_t n_tiles, int period, void* workspace_dev, float* r_dev, sept_stream_t stream);
+
 /* Class-balance noise augmentation (preprocess_data/preprocess_adversary_data.py:392-421): job j adds to row
  * job_row[j] of data_dev (n_rows, row_elems) the noise samples draw_id[job_ptr[j] .. job_ptr[j+1]) in that order -- the
  * reference writes the noisy copy through an alias of the source window, so a window drawn m times carries the sum of its

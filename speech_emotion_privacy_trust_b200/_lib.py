@@ -47,6 +47,10 @@ _SIGNATURES = {
     "sept_cloak_grl_bwd_f32": (C.c_int, [c_ptr, c_ptr, C.c_float, c_ptr, c_ptr, c_ptr, C.c_float, C.c_float, C.c_int, C.c_int,
                                          c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
     "sept_grl_bwd_f32": (C.c_int, [c_ptr, C.c_float, C.c_int64, c_ptr, c_ptr]),
+    "sept_wave_cloak_layout": (C.c_int, [c_ptr, C.c_int, C.c_int, c_ptr]),
+    "sept_wave_cloak_fwd_f32": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int64, c_ptr, C.c_int, c_ptr, c_ptr]),
+    "sept_wave_cloak_bwd_workspace_bytes": (C.c_size_t, [C.c_int]),
+    "sept_wave_cloak_bwd_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int64, C.c_int, c_ptr, c_ptr, c_ptr]),
     "sept_add_noise_rows_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_uint64, C.c_float, c_ptr, c_ptr]),
 }
 

@@ -22,6 +22,7 @@
 #include "norm_bwd.h"
 #include "resample.h"
 #include "tables.h"
+#include "wave_cloak.h"
 
 namespace {
 
@@ -559,7 +560,52 @@ int sept_grl_bwd_f32(const float* g, float lambda, int64_t n, float* dx, sept_st
     return SEPT_OK;
 }
 
-int sept_add_noise_rows_f32(float* data_dev, const int64_t* job_row_dev, const int32_t* job_ptr_dev, const int64_t* draw_id_dev,
+int sept_wave_cloak_layout(const int64_t* utt_off, int n_utts, int period, int64_t* tile_off) {
+    if (!utt_off || !tile_off || n_utts < 0 || period <= 0) return fail(SEPT_E_BADARG, "sept_wave_cloak_layout: bad argument");
+    if (period % 4) return fail(SEPT_E_BADARG, "sept_wave_cloak_layout: period=%d must be a multiple of 4", period);
+    if (utt_off[0] < 0) return fail(SEPT_E_BADARG, "sept_wave_cloak_layout: utt_off[0] is negative");
+    tile_off[0] = 0;
+    for (int u = 0; u < n_utts; ++u) {
+        const int64_t n = utt_off[u + 1] - utt_off[u];
+        if (n < 0) return fail(SEPT_E_BADARG, "sept_wave_cloak_layout: offsets must be non-decreasing (utterance %d)", u);
+        if (n >= (int64_t)1 << 31) return fail(SEPT_E_BADARG, "sept_wave_cloak_layout: utterance %d is longer than 2^31 samples", u);
+        tile_off[u + 1] = tile_off[u] + (n + period - 1) / period;
+    }
+    return SEPT_OK;
+}
+
+int sept_wave_cloak_fwd_f32(const float* x, const int64_t* utt_off, int n_utts, int64_t n_samples, const float* noise,
+                            int period, float* y, sept_stream_t stream) {
+    if (!x || !utt_off || !noise || !y || n_utts < 0 || n_samples < 0 || period <= 0)
+        return fail(SEPT_E_BADARG, "sept_wave_cloak_fwd_f32: bad argument");
+    if (period % 4) return fail(SEPT_E_BADARG, "sept_wave_cloak_fwd_f32: period=%d must be a multiple of 4", period);
+    if (!aligned16(x) || !aligned16(noise) || !aligned16(y))
+        return fail(SEPT_E_BADARG, "sept_wave_cloak_fwd_f32: pointers must be 16-byte aligned");
+    sept::WaveAddParams p{};
+    p.x = x; p.utt_off = utt_off; p.n_utts = n_utts; p.n = n_samples; p.noise = noise; p.period = period; p.y = y;
+    SEPT_CUDA(sept::launch_wave_add(p, static_cast<cudaStream_t>(stream)));
+    return SEPT_OK;
+}
+
+size_t sept_wave_cloak_bwd_workspace_bytes(int period) {
+    return period > 0 && period % 4 == 0 ? (size_t)sept::kWaveSlices * period * sizeof(float) : 0;
+}
+
+int sept_wave_cloak_bwd_f32(const float* g, const int64_t* utt_off, const int64_t* tile_off, int n_utts, int64_t n_tiles,
+                            int period, void* workspace, float* r, sept_stream_t stream) {
+    if (!g || !utt_off || !tile_off || !workspace || !r || n_utts < 0 || n_tiles < 0 || period <= 0)
+        return fail(SEPT_E_BADARG, "sept_wave_cloak_bwd_f32: bad argument");
+    if (period % 4) return fail(SEPT_E_BADARG, "sept_wave_cloak_bwd_f32: period=%d must be a multiple of 4", period);
+    if (!aligned16(g) || !aligned16(workspace) || !aligned16(r))
+        return fail(SEPT_E_BADARG, "sept_wave_cloak_bwd_f32: pointers must be 16-byte aligned");
+    sept::WaveReduceParams p{};
+    p.g = g; p.utt_off = utt_off; p.tile_off = tile_off; p.n_utts = n_utts; p.n_tiles = n_tiles; p.period = period;
+    p.partial = static_cast<float*>(workspace); p.r = r;
+    SEPT_CUDA(sept::launch_wave_reduce(p, static_cast<cudaStream_t>(stream)));
+    return SEPT_OK;
+}
+
+int sept_add_noise_rows_f32(float* data_dev,const int64_t* job_row_dev, const int32_t* job_ptr_dev, const int64_t* draw_id_dev,
                             int n_jobs, int row_elems, uint64_t seed, float std, const float* noise_dev, sept_stream_t stream) {
     if (n_jobs == 0) return SEPT_OK;
     if (!data_dev || !job_row_dev || !job_ptr_dev || !draw_id_dev || n_jobs < 0 || row_elems <= 0)

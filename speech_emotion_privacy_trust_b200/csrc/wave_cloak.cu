@@ -1,0 +1,209 @@
+// Waveform-domain cloak: a learned noise of period L tiled over every utterance of a ragged batch (sm_100a).
+//
+//   wave_add_kernel     y[s] = x[s] + noise[(s - utt_off[u]) mod L] for every sample s of utterance u; samples before
+//                       the first and after the last utterance are copied.  Each CTA owns one contiguous run of aligned
+//                       quads; a thread finds its utterance once (binary search) and walks forward from there.  x and y
+//                       move as float4 whatever the utterance alignment; the noise (L floats, L2-resident) is read as
+//                       float4 when the quad's phase is a multiple of 4, else as scalars.  Quads that straddle an
+//                       utterance boundary or the end of the buffer go sample by sample.
+//   wave_reduce_kernel  backward, pass 1: r_s[j] = sum of g over the samples of phase j in slice s.  A tile is one
+//                       period of one utterance (tile k of utterance u covers utt_off[u] + kL .. + L, clipped to the
+//                       utterance); slice s owns the global tiles [n_tiles * s / S, n_tiles * (s+1) / S), S =
+//                       kWaveSlices.  Tiles are staged 256 at a time (chunk); within a chunk, lane l of R sums the
+//                       chunk's tiles l, l+R, ... in order, the lane sums are added in lane order, and the chunk sums
+//                       are added to the slice's row in chunk order.  R = 1 when L/4 >= 256 quads, else 256 / (L/4).
+//   wave_merge_kernel   backward, pass 2: r[j] = the slices summed in order: lane l of 8 sums slices 74l .. 74l+73 in
+//                       order, the 8 lane sums are added in lane order.
+// No atomics: the order above is fixed, so the gradient is the same bits on every run (tests/wave_cloak_order.py
+// restates it on the host).  All three are HBM-bound with no reuse of x, y or g.
+#include <cuda_runtime.h>
+#include <cstdint>
+
+#include "wave_cloak.h"
+
+namespace sept {
+
+__device__ __forceinline__ float4 f4add(float4 a, float4 b) { return make_float4(a.x + b.x, a.y + b.y, a.z + b.z, a.w + b.w); }
+
+__device__ __forceinline__ float& f4at(float4& v, int e) { return e == 0 ? v.x : e == 1 ? v.y : e == 2 ? v.z : v.w; }
+
+// the last index u in [0, n - 1] with off[u] <= key (0 when n <= 1): the utterance (or tile run) holding key
+__device__ __forceinline__ int last_le(const int64_t* off, int n, int64_t key) {
+    int lo = 0, hi = n - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (off[mid] <= key) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+constexpr int kAddUnroll = 4;   // quads in flight per thread
+
+__global__ void __launch_bounds__(kWaveThreads) wave_add_kernel(const WaveAddParams p) {
+    const int64_t nq = (p.n + 3) / 4;
+    const int64_t per = (nq + gridDim.x - 1) / gridDim.x;
+    const int64_t q0 = (int64_t)blockIdx.x * per, q1 = q0 + per < nq ? q0 + per : nq;
+    if (q0 + threadIdx.x >= q1) return;
+    const int64_t lo = p.utt_off[0], hi = p.utt_off[p.n_utts];      // samples outside [lo, hi) are copied
+    const uint32_t L = (uint32_t)p.period;
+    int u = last_le(p.utt_off, p.n_utts, 4 * (q0 + threadIdx.x));
+    int64_t b = 0, e = 0;                                           // bounds of utterance u (read once u is in range)
+    bool have = false;
+    for (int64_t qb = q0 + threadIdx.x; qb < q1; qb += kAddUnroll * kWaveThreads) {
+        float4 v[kAddUnroll];
+#pragma unroll
+        for (int k = 0; k < kAddUnroll; ++k) {
+            const int64_t q = qb + (int64_t)k * kWaveThreads;
+            if (q < q1 && 4 * q + 4 <= p.n) v[k] = __ldcs(reinterpret_cast<const float4*>(p.x) + q);
+        }
+#pragma unroll
+        for (int k = 0; k < kAddUnroll; ++k) {
+            const int64_t q = qb + (int64_t)k * kWaveThreads;
+            if (q >= q1) break;
+            const int64_t s = 4 * q;
+            if (s + 4 <= p.n && (s + 4 <= lo || s >= hi)) {            // wholly outside every utterance
+                __stcs(reinterpret_cast<float4*>(p.y) + q, v[k]);
+                continue;
+            }
+            if (s >= lo) {
+                while (u + 1 < p.n_utts && p.utt_off[u + 1] <= s) { ++u; have = false; }
+            }
+            if (!have && p.n_utts > 0) { b = p.utt_off[u]; e = p.utt_off[u + 1]; have = true; }
+            if (s + 4 <= p.n && s >= b && s + 4 <= e && have) {    // wholly inside utterance u
+                const uint32_t ph = (uint32_t)(s - b) % L;
+                float4 nz;
+                if ((ph & 3u) == 0) {
+                    nz = *reinterpret_cast<const float4*>(p.noise + ph);
+                } else {
+#pragma unroll
+                    for (int c = 0; c < 4; ++c) {
+                        const uint32_t j = ph + c;
+                        f4at(nz, c) = __ldg(p.noise + (j >= L ? j - L : j));
+                    }
+                }
+                __stcs(reinterpret_cast<float4*>(p.y) + q, f4add(v[k], nz));
+                continue;
+            }
+            // an utterance boundary, the edge of [lo, hi) or the end of the buffer lies inside this quad
+            int w = u;
+            for (int c = 0; c < 4 && s + c < p.n; ++c) {
+                const int64_t t = s + c;
+                float val = p.x[t];
+                if (t >= lo && t < hi) {
+                    while (w + 1 < p.n_utts && p.utt_off[w + 1] <= t) ++w;
+                    val += __ldg(p.noise + (uint32_t)(t - p.utt_off[w]) % L);
+                }
+                p.y[t] = val;
+            }
+        }
+    }
+}
+
+__device__ __forceinline__ float4 tile_quad(const float* g, int64_t base, int len, int j) {
+    if (j + 4 <= len && (base & 3) == 0) return __ldcs(reinterpret_cast<const float4*>(g + base + j));
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+    for (int c = 0; c < 4; ++c)
+        if (j + c < len) f4at(v, c) = __ldcs(g + base + j + c);
+    return v;
+}
+
+__global__ void __launch_bounds__(kWaveThreads) wave_reduce_kernel(const WaveReduceParams p) {
+    __shared__ int64_t s_base[kWaveThreads];
+    __shared__ int s_len[kWaveThreads];
+    __shared__ float4 s_red[kWaveThreads];
+    const int L = p.period, Q = L / 4;
+    const int R = Q >= kWaveThreads ? 1 : kWaveThreads / Q;
+    const int lane = R == 1 ? 0 : threadIdx.x / Q;
+    const int qt = R == 1 ? threadIdx.x : threadIdx.x % Q;
+    const int64_t T0 = p.n_tiles * blockIdx.x / kWaveSlices, T1 = p.n_tiles * (blockIdx.x + 1) / kWaveSlices;
+    float* row = p.partial + (size_t)blockIdx.x * L;
+    const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (T0 == T1) {                                                 // an empty slice still writes its (zero) row
+        if (lane == 0)
+            for (int q = qt; q < Q; q += kWaveThreads) *reinterpret_cast<float4*>(row + 4 * q) = zero;
+        return;
+    }
+    float4 acc = zero;                                              // R > 1: the row element of quad qt
+    for (int64_t c0 = T0; c0 < T1; c0 += kWaveThreads) {
+        const int nt = T1 - c0 < kWaveThreads ? (int)(T1 - c0) : kWaveThreads;
+        __syncthreads();                                            // the previous chunk is no longer read
+        if ((int)threadIdx.x < nt) {
+            const int64_t i = c0 + threadIdx.x;
+            const int u = last_le(p.tile_off, p.n_utts, i);
+            const int64_t base = p.utt_off[u] + (i - p.tile_off[u]) * L, left = p.utt_off[u + 1] - base;
+            s_base[threadIdx.x] = base;
+            s_len[threadIdx.x] = left < L ? (int)left : L;
+        }
+        __syncthreads();
+        if (R == 1) {
+            for (int q = qt; q < Q; q += kWaveThreads) {
+                float4 l = zero;
+#pragma unroll 8
+                for (int t = 0; t < nt; ++t) l = f4add(l, tile_quad(p.g, s_base[t], s_len[t], 4 * q));
+                float4* dst = reinterpret_cast<float4*>(row + 4 * q);
+                *dst = f4add(c0 == T0 ? zero : *dst, l);
+            }
+        } else {
+            float4 l = zero;
+            if (lane < R)
+                for (int t = lane; t < nt; t += R) l = f4add(l, tile_quad(p.g, s_base[t], s_len[t], 4 * qt));
+            s_red[threadIdx.x] = l;
+            __syncthreads();
+            if (lane == 0) {
+                float4 c = s_red[qt];
+                for (int k = 1; k < R; ++k) c = f4add(c, s_red[k * Q + qt]);
+                acc = f4add(acc, c);
+            }
+        }
+    }
+    if (R > 1 && lane == 0) *reinterpret_cast<float4*>(row + 4 * qt) = acc;
+}
+
+constexpr int kMergeQuads = kWaveThreads / kWaveMergeLanes;        // 32 quads per CTA
+static_assert(kWaveSlices % kWaveMergeLanes == 0, "equal slice runs per merge lane");
+
+__global__ void __launch_bounds__(kWaveThreads) wave_merge_kernel(const float* __restrict__ partial, int L,
+                                                                  float* __restrict__ r) {
+    __shared__ float4 s_red[kWaveThreads];
+    const int Q = L / 4, lane = threadIdx.x / kMergeQuads, qi = threadIdx.x % kMergeQuads;
+    const int q = blockIdx.x * kMergeQuads + qi;
+    constexpr int per = kWaveSlices / kWaveMergeLanes;
+    float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (q < Q) {
+#pragma unroll 8
+        for (int s = lane * per; s < (lane + 1) * per; ++s)
+            a = f4add(a, __ldcg(reinterpret_cast<const float4*>(partial + (size_t)s * L) + q));
+    }
+    s_red[threadIdx.x] = a;
+    __syncthreads();
+    if (lane == 0 && q < Q) {
+        float4 c = s_red[qi];
+        for (int k = 1; k < kWaveMergeLanes; ++k) c = f4add(c, s_red[k * kMergeQuads + qi]);
+        reinterpret_cast<float4*>(r)[q] = c;
+    }
+}
+
+cudaError_t launch_wave_add(const WaveAddParams& p, cudaStream_t stream) {
+    if (p.n == 0) return cudaSuccess;
+    int dev = 0, sms = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (e != cudaSuccess) return e;
+    const int64_t nq = (p.n + 3) / 4, want = (nq + kAddUnroll * kWaveThreads - 1) / (kAddUnroll * kWaveThreads);
+    const int blocks = (int)(want < (int64_t)sms * 8 ? want : (int64_t)sms * 8);     // 8 CTAs (2048 threads) per SM
+    wave_add_kernel<<<blocks, kWaveThreads, 0, stream>>>(p);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_wave_reduce(const WaveReduceParams& p, cudaStream_t stream) {
+    wave_reduce_kernel<<<kWaveSlices, kWaveThreads, 0, stream>>>(p);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    const int quads = p.period / 4;
+    wave_merge_kernel<<<(quads + kMergeQuads - 1) / kMergeQuads, kWaveThreads, 0, stream>>>(p.partial, p.period, p.r);
+    return cudaGetLastError();
+}
+
+}  // namespace sept

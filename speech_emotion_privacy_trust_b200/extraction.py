@@ -35,6 +35,18 @@ class Layout:
         return int(self.frame_off_host[u + 1] - self.frame_off_host[u])
 
 
+@dataclass
+class Tiles:
+    """Period tiles of a ragged batch (sept_wave_cloak_layout): tile k of utterance u is its k-th run of `period`
+    samples, clipped to the utterance; utterance u holds tiles tile_off[u] .. tile_off[u+1]-1."""
+    tile_off_host: np.ndarray        # int64 [n+1]
+    tile_off: torch.Tensor           # device int64 [n+1]
+
+    @property
+    def n_tiles(self) -> int:
+        return int(self.tile_off_host[-1])
+
+
 class RaggedAudio:
     """Utterances back to back in one device buffer: wav[utt_off[u]:utt_off[u+1]] (16 kHz mono fp32)."""
 
@@ -48,6 +60,7 @@ class RaggedAudio:
             raise ValueError("utt_off must be a 1-D offset array within wav")
         self.utt_off = torch.from_numpy(self.utt_off_host).to(wav.device, non_blocking=True)
         self._layouts: dict[tuple[int, int], Layout] = {}
+        self._tiles: dict[int, Tiles] = {}
 
     @classmethod
     def from_list(cls, waves: Sequence, device="cuda") -> "RaggedAudio":
@@ -74,6 +87,25 @@ class RaggedAudio:
                                         int(item_off[-1]))
         return self._layouts[key]
 
+    def tiles(self, period: int) -> Tiles:
+        """The period tiles of the batch (cached, like the frame layouts, so a CUDA-graph capture finds them built)."""
+        if period not in self._tiles:
+            tile_off = np.zeros(self.n_utts + 1, dtype=np.int64)
+            _lib.check(_lib.lib().sept_wave_cloak_layout(self.utt_off_host.ctypes.data, self.n_utts, int(period),
+                                                         tile_off.ctypes.data))
+            self._tiles[period] = Tiles(tile_off, torch.from_numpy(tile_off).to(self.wav.device))
+        return self._tiles[period]
+
+    def with_wav(self, wav: torch.Tensor) -> "RaggedAudio":
+        """The same utterances over another buffer of the same length (e.g. a processed copy of `wav` that carries a
+        grad_fn): shares the offsets and the cached layouts and tiles, so nothing is rebuilt or copied."""
+        if wav.shape != self.wav.shape or wav.dtype != self.wav.dtype or wav.device != self.wav.device:
+            raise ValueError(f"with_wav: a {tuple(self.wav.shape)} {self.wav.dtype} buffer on {self.wav.device} is needed")
+        out = RaggedAudio.__new__(RaggedAudio)
+        out.wav, out.utt_off_host, out.utt_off, out._layouts, out._tiles = (wav, self.utt_off_host, self.utt_off,
+                                                                            self._layouts, self._tiles)
+        return out
+
 
 def resample(batch: "RaggedAudio", orig_freq: int, new_freq: int = SAMPLE_RATE) -> "RaggedAudio":
     """Band-limited sinc resampling of every utterance (torchaudio.transforms.Resample(orig_freq, new_freq) as the
@@ -91,7 +123,7 @@ def resample(batch: "RaggedAudio", orig_freq: int, new_freq: int = SAMPLE_RATE) 
                                                 int(out_off[-1]), orig_freq, new_freq, out.data_ptr(),
                                                 torch.cuda.current_stream(dev).cuda_stream))
     res = RaggedAudio.__new__(RaggedAudio)
-    res.wav, res.utt_off_host, res.utt_off, res._layouts = out, out_off, d_out_off, {}
+    res.wav, res.utt_off_host, res.utt_off, res._layouts, res._tiles = out, out_off, d_out_off, {}, {}
     return res
 
 

@@ -1,0 +1,148 @@
+"""Waveform-domain cloak: a learned noise of period L added to the raw audio of a ragged batch, trained through the
+differentiable extraction chain (wav -> wave cloak -> logmel_grad -> speaker_stats_grad -> normalized_windows_grad -> ...).
+
+The signal-domain counterpart of cloak_noise (model/cloak_models.py:24-58): the same mu / rho parameterisation,
+sigma = (1 + tanh rho)/2 * (max_scale - min_scale) + min_scale, the same device Philox eps (one (L,) sample per forward,
+identical on every rank, fresh on every CUDA-graph replay) and a deterministic backward.  Forward: sept_cloak_fwd_f32 draws
+noise = mu + sigma * eps, sept_wave_cloak_fwd_f32 tiles it over every utterance from the utterance's first sample.
+Backward: dx = g; sept_wave_cloak_bwd_f32 sums g per phase, sept_cloak_grl_bwd_f32 turns that sum into dlocs and drhos."""
+from __future__ import annotations
+
+import torch
+import torch.nn as nn
+from torch.autograd.function import once_differentiable
+
+from . import _lib, cloak_ops
+from .extraction import RaggedAudio
+
+DEFAULT_PERIOD = 32000     # one 200-frame training window at hop 160
+EPS_STD = 0.1              # cloak_noise's Normal(0, 0.1) (cloak_models.py:37)
+
+
+def _stream(device) -> int:
+    return torch.cuda.current_stream(device).cuda_stream
+
+
+def _aligned(t: torch.Tensor) -> torch.Tensor:
+    """t, or a copy of it at a 16-byte aligned address (the kernels move float4s; a view at an odd offset needs the copy)."""
+    return t if t.data_ptr() % 16 == 0 else t.clone()
+
+
+def new_workspace(device: torch.device, period: int) -> tuple[torch.Tensor, torch.Tensor]:
+    """(partial rows of the phase reduction, workspace of the mu / rho backward).  The owner decides their lifetime, as
+    with cloak_ops.new_workspace: a WaveCloak layer allocates them on its first forward, before any CUDA-graph capture;
+    callers of WaveCloakFunction without one get fresh ones per backward."""
+    nbytes = _lib.lib().sept_wave_cloak_bwd_workspace_bytes(period)
+    if nbytes == 0:
+        raise ValueError(f"period={period} must be a positive multiple of 4")
+    return (torch.empty(nbytes // 4, dtype=torch.float32, device=device), cloak_ops.new_workspace(device, period))
+
+
+class WaveCloakFunction(torch.autograd.Function):
+    """y = wav + noise[(s - utt_off[u]) mod L] over every utterance u of `batch` (samples outside every utterance
+    unchanged), noise = locs + sigma(rhos) * eps.  eps: a caller's (L,) sample, or None to draw it on the device from
+    Philox(seed, offset) at the draw counter `draw` (advanced by one).  No double backward."""
+
+    @staticmethod
+    def forward(ctx, wav, locs, rhos, batch, eps, seed, offset, eps_std, min_scale, max_scale, draw=None, workspace=None):
+        _lib.require_cuda(wav)
+        period = locs.numel()
+        if rhos.numel() != period:
+            raise ValueError(f"locs ({period}) and rhos ({rhos.numel()}) must have one element per phase")
+        if wav.shape != batch.wav.shape:
+            raise ValueError(f"wav of shape {tuple(wav.shape)} is not the batch's buffer {tuple(batch.wav.shape)}")
+        tiles = batch.tiles(period)                                  # ValueError unless period is a multiple of 4
+        locs_c, rhos_c = cloak_ops._f32c(locs.detach()), cloak_ops._f32c(rhos.detach())
+        eps_c = None
+        if eps is not None:
+            eps_c = cloak_ops._f32c(eps.detach().to(wav.device)).reshape(-1)
+            if eps_c.numel() != period:
+                raise ValueError(f"eps has {eps_c.numel()} elements; the period is {period}")
+        _, eps_used, noise = cloak_ops.cloak_forward_raw(None, locs_c, rhos_c, None, eps_c, seed, offset, eps_std,
+                                                         min_scale, max_scale, want_noise=True, draw=draw)
+        x = _aligned(wav.detach())
+        y = torch.empty_like(x)
+        dev = x.device
+        with torch.cuda.device(dev):
+            _lib.check(_lib.lib().sept_wave_cloak_fwd_f32(x.data_ptr(), batch.utt_off.data_ptr(), batch.n_utts, x.numel(),
+                                                          noise.data_ptr(), period, y.data_ptr(), _stream(dev)))
+        ctx.save_for_backward(eps_used, rhos_c)
+        ctx.batch, ctx.tiles, ctx.workspace = batch, tiles, workspace
+        ctx.cfg = (float(min_scale), float(max_scale), tuple(locs.shape), tuple(rhos.shape))
+        return y
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        eps_used, rhos_c = ctx.saved_tensors
+        min_scale, max_scale, lshape, rshape = ctx.cfg
+        batch, tiles = ctx.batch, ctx.tiles
+        period = rhos_c.numel()
+        need_wav, need_locs, need_rhos = ctx.needs_input_grad[:3]
+        dlocs = drhos = None
+        if need_locs or need_rhos:
+            gc = _aligned(cloak_ops._f32c(g))
+            dev = gc.device
+            ws_r, ws_c = ctx.workspace if ctx.workspace is not None else new_workspace(dev, period)
+            r = torch.empty(period, dtype=torch.float32, device=dev)
+            dlocs = torch.empty(period, dtype=torch.float32, device=dev)
+            drhos = torch.empty(period, dtype=torch.float32, device=dev) if need_rhos else None
+            lib = _lib.lib()
+            with torch.cuda.device(dev):
+                _lib.check(lib.sept_wave_cloak_bwd_f32(gc.data_ptr(), batch.utt_off.data_ptr(), tiles.tile_off.data_ptr(),
+                                                       batch.n_utts, tiles.n_tiles, period, ws_r.data_ptr(), r.data_ptr(),
+                                                       _stream(dev)))
+                _lib.check(lib.sept_cloak_grl_bwd_f32(r.data_ptr(), None, 0.0, eps_used.data_ptr(), rhos_c.data_ptr(), None,
+                                                      min_scale, max_scale, 1, period, ws_c.data_ptr(), dlocs.data_ptr(),
+                                                      cloak_ops._ptr(drhos), None, _stream(dev)))
+        return (g if need_wav else None, dlocs.view(lshape) if need_locs else None,
+                drhos.view(rshape) if need_rhos else None) + (None,) * 9
+
+
+class WaveCloak(nn.Module):
+    """Learned waveform noise: forward(batch) returns a RaggedAudio with the same utterances whose wav is
+    batch.wav + (locs + scales() * eps) tiled from each utterance's first sample, with a grad_fn to locs and rhos (and to
+    batch.wav when that requires grad).
+
+    locs, rhos: (period,) parameters, rhos starting at -2 like cloak_noise's (ones - 3).  eps is drawn on the device
+    (Philox seeded with torch.initial_seed(), a device draw counter: identical on data-parallel ranks that share the
+    seed, fresh on every replay of a captured CUDA graph); set `external_eps` to a (period,) tensor to supply it."""
+
+    def __init__(self, min_scale: float, max_scale: float, period: int = DEFAULT_PERIOD, locs: torch.Tensor | None = None,
+                 device=None):
+        super().__init__()
+        if period <= 0 or period % 4:
+            raise ValueError(f"period={period} must be a positive multiple of 4")
+        self.period = int(period)
+        self.min_scale, self.max_scale = float(min_scale), float(max_scale)
+        init = torch.zeros(period) if locs is None else torch.as_tensor(locs, dtype=torch.float32).reshape(-1).clone()
+        if init.numel() != period:
+            raise ValueError(f"locs has {init.numel()} elements; the period is {period}")
+        self.locs = nn.Parameter(init.to(device))
+        self.rhos = nn.Parameter(torch.full((period,), -2.0, device=device))
+        self.external_eps = None
+        self._draws = None            # device counter of samples drawn (the Philox offset lives on the GPU)
+        self._workspace = None        # backward workspaces, owned by the layer (allocated on the first forward)
+
+    def scales(self) -> torch.Tensor:
+        return (1.0 + torch.tanh(self.rhos)) / 2 * (self.max_scale - self.min_scale) + self.min_scale
+
+    def _eps_source(self):
+        if self.external_eps is not None:
+            if self.external_eps.numel() != self.period:
+                raise ValueError(f"external_eps has {self.external_eps.numel()} elements; the period is {self.period}")
+            return self.external_eps, 0, None
+        if self._draws is None or self._draws.device != self.rhos.device:
+            self._draws = torch.zeros(1, dtype=torch.int64, device=self.rhos.device)
+        return None, torch.initial_seed(), self._draws
+
+    def _ws(self):
+        if self._workspace is None or self._workspace[0].device != self.rhos.device:
+            self._workspace = new_workspace(self.rhos.device, self.period)
+        return self._workspace
+
+    def forward(self, batch: RaggedAudio) -> RaggedAudio:
+        eps, seed, draw = self._eps_source()
+        wav = WaveCloakFunction.apply(batch.wav, self.locs, self.rhos, batch, eps, seed, 0, EPS_STD, self.min_scale,
+                                      self.max_scale, draw, self._ws())
+        return batch.with_wav(wav)
