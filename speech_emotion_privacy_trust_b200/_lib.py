@@ -3,60 +3,45 @@ nvcc if the toolchain is present, otherwise importing the compute layer fails lo
 from __future__ import annotations
 
 import ctypes as C
+import re
 from pathlib import Path
+
+import torch
 
 from . import build as _build
 
 _LIB = None
 
-c_f32p = C.c_void_p      # device / host pointers travel as integers (tensor.data_ptr())
-c_ptr = C.c_void_p
-
-_SIGNATURES = {
-    "sept_version": (C.c_int, []),
-    "sept_last_error": (C.c_char_p, []),
-    "sept_source_hash": (C.c_char_p, []),
-    "sept_init": (C.c_int, [C.c_int]),
-    "sept_frames_per_item": (C.c_int, [C.c_int]),
-    "sept_extract_layout": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr]),
-    "sept_logmel_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr]),
-    "sept_logmel_bwd_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int64]),
-    "sept_logmel_bwd_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int64, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr,
-                                      c_ptr]),
-    "sept_mfcc_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int64, c_ptr, c_ptr, c_ptr, c_ptr]),
-    "sept_mfcc_bwd_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int64, C.c_int64]),
-    "sept_mfcc_bwd_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int64, C.c_int64, c_ptr, c_ptr, c_ptr, c_ptr]),
-    "sept_resample_layout": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, c_ptr]),
-    "sept_resample_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int64, C.c_int, C.c_int, c_ptr, c_ptr]),
-    "sept_pcm16_to_f32": (C.c_int, [c_ptr, C.c_int64, c_ptr, c_ptr]),
-    "sept_speaker_stats_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, C.c_int, c_ptr, c_ptr, c_ptr]),
-    "sept_normalize_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr]),
-    "sept_normalize_windows_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr]),
-    "sept_normalize_bwd_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
-    "sept_normalize_bwd_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
-                                         c_ptr, c_ptr, c_ptr, C.c_int, c_ptr, c_ptr, c_ptr, c_ptr]),
-    "sept_speaker_stats_bwd_ties_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
-    "sept_speaker_stats_bwd_ties_i32": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr,
-                                                  C.c_int, c_ptr, c_ptr, c_ptr, c_ptr]),
-    "sept_speaker_stats_bwd_frames_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr,
-                                                    c_ptr, c_ptr, c_ptr]),
-    "sept_counter_add_u64": (C.c_int, [c_ptr, C.c_uint64, c_ptr]),
-    "sept_cloak_fwd_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, C.c_uint64, C.c_uint64, c_ptr, C.c_int, C.c_float, C.c_float, C.c_float,
-                                     C.c_int, C.c_int, c_ptr, c_ptr, c_ptr, c_ptr]),
-    "sept_cloak_bwd_workspace_bytes": (C.c_size_t, [C.c_int]),
-    "sept_cloak_grl_bwd_f32": (C.c_int, [c_ptr, c_ptr, C.c_float, c_ptr, c_ptr, c_ptr, C.c_float, C.c_float, C.c_int, C.c_int,
-                                         c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
-    "sept_grl_bwd_f32": (C.c_int, [c_ptr, C.c_float, C.c_int64, c_ptr, c_ptr]),
-    "sept_wave_cloak_layout": (C.c_int, [c_ptr, C.c_int, C.c_int, c_ptr]),
-    "sept_wave_cloak_fwd_f32": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int64, c_ptr, C.c_int, c_ptr, c_ptr]),
-    "sept_wave_cloak_bwd_workspace_bytes": (C.c_size_t, [C.c_int]),
-    "sept_wave_cloak_bwd_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, C.c_int, C.c_int64, C.c_int, c_ptr, c_ptr, c_ptr]),
-    "sept_add_noise_rows_f32": (C.c_int, [c_ptr, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int, C.c_uint64, C.c_float, c_ptr, c_ptr]),
-}
-
-EXPORTS = tuple(_SIGNATURES)
-
 SEPT_E_BADARG, SEPT_E_UNSUPPORTED, SEPT_E_TOO_SHORT, SEPT_E_CUDA = -1, -2, -3, -4
+
+_RESTYPES = {"int": C.c_int, "size_t": C.c_size_t, "const char*": C.c_char_p}
+_ARGTYPES = {"int": C.c_int, "int64_t": C.c_int64, "uint64_t": C.c_uint64, "float": C.c_float, "size_t": C.c_size_t,
+             "sept_stream_t": C.c_void_p}
+_PROTO = re.compile(r"^[ \t]*(\w[\w \t]*?[ \t*]+)(sept_\w+)\s*\(([^)]*)\)\s*;", re.M)
+
+
+def _ctype(table: dict, decl: str, name: str):
+    try:
+        return table[decl]
+    except KeyError:
+        raise RuntimeError(f"{_build.HEADER.name}: {name} uses the type {decl!r}, which the binding does not map") from None
+
+
+def signatures(header: str) -> dict:
+    """{name: (restype, argtypes)} of every sept_* prototype of the header text.  Pointers (device and host memory alike
+    travel as integers, e.g. tensor.data_ptr()) and the stream are c_void_p; any other type must be one the tables above
+    map, or this raises."""
+    sigs = {}
+    for ret, name, params in _PROTO.findall(re.sub(r"/\*.*?\*/", " ", header, flags=re.S)):
+        args = []
+        for p in ([] if params.strip() == "void" else params.split(",")):
+            args.append(C.c_void_p if "*" in p else _ctype(_ARGTYPES, " ".join(p.split()[:-1]), name))
+        sigs[name] = (_ctype(_RESTYPES, " ".join(ret.split()).replace(" *", "*"), name), args)
+    return sigs
+
+
+_SIGS = signatures(_build.HEADER.read_text())     # parsed once, when the binding is imported
+EXPORTS = tuple(_SIGS)
 
 
 def library_path() -> Path:
@@ -67,7 +52,7 @@ def lib() -> C.CDLL:
     """Load libsept_b200.so.  The library carries the sha256 of the sources it was compiled from; if it is absent or
     that hash differs from the sources in the tree (a stale prebuilt .so), it is rebuilt first (under a file lock:
     several ranks may start together), and if it cannot be rebuilt the call raises -- a stale library is never used
-    silently and there is no CPU fallback."""
+    silently and there is no CPU fallback.  The ctypes signatures are those of include/sept.h."""
     global _LIB
     if _LIB is None:
         import os
@@ -84,7 +69,7 @@ def lib() -> C.CDLL:
                         state = "missing" if not path.exists() else "stale (built from other sources than the tree holds)"
                         raise RuntimeError(f"{path.name} is {state} and cannot be rebuilt: {exc}") from exc
         handle = C.CDLL(str(path))
-        for name, (res, args) in _SIGNATURES.items():
+        for name, (res, args) in _SIGS.items():
             try:
                 fn = getattr(handle, name)
             except AttributeError:
@@ -109,6 +94,24 @@ def check(rc: int) -> None:
     if rc in (SEPT_E_BADARG, SEPT_E_UNSUPPORTED):
         raise ValueError(msg)
     raise RuntimeError(msg)       # too-short utterance (torch.stft raises RuntimeError too) and CUDA errors
+
+
+def call(name: str, *args) -> None:
+    """Call the C entry `name` and check its status.  A tensor passes as its data_ptr(), None as NULL, anything else as
+    it is."""
+    check(getattr(lib(), name)(*[a.data_ptr() if isinstance(a, torch.Tensor) else a for a in args]))
+
+
+def launch(name: str, *args, device) -> None:
+    """call() with `device` current and its current stream appended as the last argument (the entry's sept_stream_t)."""
+    with torch.cuda.device(device):
+        call(name, *args, torch.cuda.current_stream(device).cuda_stream)
+
+
+def workspace(nbytes: int, device, zeroed: bool = False) -> torch.Tensor:
+    """A workspace of max(16, nbytes) bytes for an entry that sizes its own (never empty, so never a NULL pointer).
+    zeroed: for a kernel that needs it to start at zero."""
+    return (torch.zeros if zeroed else torch.empty)(max(16, nbytes), dtype=torch.uint8, device=device)
 
 
 def require_cuda(t) -> None:

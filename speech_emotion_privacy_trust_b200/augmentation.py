@@ -74,17 +74,14 @@ def apply_plan(windows: torch.Tensor, plan: BalancePlan, std: float = 0.05, seed
     job_row = torch.from_numpy(rows.astype(np.int64)).to(dev)
     job_ptr_t = torch.from_numpy(job_ptr).to(dev)
     draw_id = torch.from_numpy(order.astype(np.int64)).to(dev)
-    noise_ptr = None
     if noise is not None:
         _lib.require_cuda(noise)
         if noise.dtype != torch.float32 or not noise.is_contiguous() or noise.numel() != plan.n_aug * row_elems:
             raise ValueError("noise must be a contiguous float32 tensor of shape (n_aug, *window shape)")
-        noise_ptr = noise.data_ptr()
-    stream = torch.cuda.current_stream(dev).cuda_stream
     for j0 in range(0, rows.size, 65535):
         j1 = min(rows.size, j0 + 65535)
-        _lib.check(_lib.lib().sept_add_noise_rows_f32(out.data_ptr(), job_row[j0:].data_ptr(), job_ptr_t[j0:].data_ptr(),
-                                                      draw_id.data_ptr(), j1 - j0, row_elems, seed, std, noise_ptr, stream))
+        _lib.launch("sept_add_noise_rows_f32", out, job_row[j0:], job_ptr_t[j0:], draw_id, j1 - j0, row_elems, seed, std, noise,
+                    device=dev)
     return out
 
 

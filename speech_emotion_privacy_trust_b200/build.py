@@ -17,6 +17,7 @@ from pathlib import Path
 PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB = PKG / "libsept_b200.so"
+HEADER = PKG.parent / "include" / "sept.h"
 SOURCES = ["api.cu", "extract.cu", "extract_bwd.cu", "mfcc_bwd.cu", "mfcc_dct.cu", "cloak.cu", "norm.cu", "norm_bwd.cu", "resample.cu", "augment.cu",
            "wave_cloak.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "--expt-relaxed-constexpr",
@@ -34,7 +35,7 @@ def source_hash() -> str:
     """sha256 over every source the library is compiled from (+ the compiler flags).  Content, not mtime: the tree is
     copied to the GPU box, where timestamps mean nothing."""
     h = hashlib.sha256()
-    deps = sorted(list(CSRC.glob("*.cu")) + list(CSRC.glob("*.cuh")) + list(CSRC.glob("*.h")) + [PKG.parent / "include" / "sept.h"])
+    deps = sorted(list(CSRC.glob("*.cu")) + list(CSRC.glob("*.cuh")) + list(CSRC.glob("*.h")) + [HEADER])
     for d in deps:
         h.update(d.name.encode() + b"\0" + d.read_bytes() + b"\0")
     h.update(" ".join(NVCC_FLAGS).encode())
@@ -62,7 +63,7 @@ def build(force: bool = False, verbose: bool = False) -> Path:
     extra = os.environ.get("SEPT_NVCC_EXTRA", "").split()        # experiments only (compiler flag A/B)
     objdir = PKG / "build"
     objdir.mkdir(exist_ok=True)
-    headers = sorted(list(CSRC.glob("*.cuh")) + list(CSRC.glob("*.h")) + [PKG.parent / "include" / "sept.h"])
+    headers = sorted(list(CSRC.glob("*.cuh")) + list(CSRC.glob("*.h")) + [HEADER])
     common = hashlib.sha256(b"".join(h.read_bytes() for h in headers) + " ".join(NVCC_FLAGS + extra).encode()).hexdigest()
     procs = []
     for src in SOURCES:

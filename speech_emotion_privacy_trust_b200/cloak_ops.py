@@ -5,21 +5,13 @@ import torch
 
 from . import _lib
 
-def _stream(device) -> int:
-    return torch.cuda.current_stream(device).cuda_stream
-
 
 def new_workspace(device: torch.device, wf: int) -> torch.Tensor:
     """Partial-sum buffer + column counters of the backward kernel (counters start at zero; the kernel leaves them at
     zero again).  The OWNER decides its lifetime: a cloak_noise layer keeps one for as long as it lives -- allocated on
     its first forward, i.e. before any CUDA-graph capture of the step, never inside one -- and callers of the functional
     API get a fresh one per call.  Backward launches that may overlap (different streams) need different workspaces."""
-    nbytes = _lib.lib().sept_cloak_bwd_workspace_bytes(wf)
-    return torch.zeros((nbytes + 3) // 4, dtype=torch.int32, device=device)
-
-
-def _ptr(t):
-    return 0 if t is None else t.data_ptr()
+    return _lib.workspace(_lib.lib().sept_cloak_bwd_workspace_bytes(wf), device, zeroed=True)
 
 
 def _f32c(t: torch.Tensor) -> torch.Tensor:
@@ -48,15 +40,12 @@ def cloak_forward_raw(x, locs, rhos, mask, eps, seed, offset, eps_std, min_scale
     out = torch.empty_like(x) if x is not None else None
     eps_used = torch.empty(batch * wf if per_sample else wf, dtype=torch.float32, device=dev) if eps is None else eps
     noise = torch.empty_like(locs) if want_noise else None
-    with torch.cuda.device(dev):
-        _lib.check(_lib.lib().sept_cloak_fwd_f32(
-            _ptr(x) if x is not None else locs.data_ptr(), locs.data_ptr(), rhos.data_ptr(), _ptr(mask), _ptr(eps),
-            int(seed) & 0xFFFFFFFFFFFFFFFF, int(offset) & 0xFFFFFFFFFFFFFFFF, _ptr(draw) if eps is None else 0, int(per_sample), float(eps_std),
-            float(min_scale), float(max_scale),
-            batch, wf, _ptr(out) if out is not None else locs.data_ptr(), eps_used.data_ptr() if eps is None else 0,
-            _ptr(noise), _stream(dev)))
-        if draw is not None and eps is None:
-            _lib.check(_lib.lib().sept_counter_add_u64(draw.data_ptr(), batch if per_sample else 1, _stream(dev)))
+    _lib.launch("sept_cloak_fwd_f32", locs if x is None else x, locs, rhos, mask, eps, int(seed) & 0xFFFFFFFFFFFFFFFF,
+                int(offset) & 0xFFFFFFFFFFFFFFFF, draw if eps is None else None, int(per_sample), float(eps_std),
+                float(min_scale), float(max_scale), batch, wf, locs if out is None else out,
+                eps_used if eps is None else None, noise, device=dev)
+    if draw is not None and eps is None:
+        _lib.launch("sept_counter_add_u64", draw, batch if per_sample else 1, device=dev)
     return out, eps_used, noise
 
 
@@ -102,10 +91,8 @@ class CloakNoiseFunction(torch.autograd.Function):
         drhos = torch.empty(wf, dtype=torch.float32, device=dev) if need_rhos else None
         dx = torch.empty_like(g_a) if need_x else None
         ws = ctx.workspace if ctx.workspace is not None else new_workspace(dev, wf)
-        with torch.cuda.device(dev):
-            _lib.check(_lib.lib().sept_cloak_grl_bwd_f32(
-                g_a.data_ptr(), _ptr(g_b), lam, eps_used.data_ptr(), rhos_c.data_ptr(), _ptr(mask_c), min_scale, max_scale,
-                batch, wf, ws.data_ptr(), dlocs.data_ptr(), _ptr(drhos), _ptr(dx), _stream(dev)))
+        _lib.launch("sept_cloak_grl_bwd_f32", g_a, g_b, lam, eps_used, rhos_c, mask_c, min_scale, max_scale, batch, wf, ws,
+                    dlocs, drhos, dx, device=dev)
         return (dx, dlocs.view(pshape) if need_locs else None, drhos.view(pshape) if need_rhos else None,
                 None, None, None, None, None, None, None, None, None, None, None)
 
@@ -124,6 +111,5 @@ class GradientReversalFunction(torch.autograd.Function):
         _lib.require_cuda(grads)
         g = _f32c(grads)
         dx = torch.empty_like(g)
-        with torch.cuda.device(g.device):
-            _lib.check(_lib.lib().sept_grl_bwd_f32(g.data_ptr(), ctx.lambda_, g.numel(), dx.data_ptr(), _stream(g.device)))
+        _lib.launch("sept_grl_bwd_f32", g, ctx.lambda_, g.numel(), dx, device=g.device)
         return dx, None

@@ -80,8 +80,8 @@ class RaggedAudio:
             n = self.n_utts
             frame_off = np.zeros(n + 1, dtype=np.int64)
             item_off = np.zeros(n + 1, dtype=np.int32)
-            _lib.check(_lib.lib().sept_extract_layout(self.utt_off_host.ctypes.data, n, n_fft, hop,
-                                                      frame_off.ctypes.data, item_off.ctypes.data))
+            _lib.call("sept_extract_layout", self.utt_off_host.ctypes.data, n, n_fft, hop, frame_off.ctypes.data,
+                      item_off.ctypes.data)
             dev = self.wav.device
             self._layouts[key] = Layout(frame_off, torch.from_numpy(frame_off).to(dev), torch.from_numpy(item_off).to(dev),
                                         int(item_off[-1]))
@@ -91,8 +91,7 @@ class RaggedAudio:
         """The period tiles of the batch (cached, like the frame layouts, so a CUDA-graph capture finds them built)."""
         if period not in self._tiles:
             tile_off = np.zeros(self.n_utts + 1, dtype=np.int64)
-            _lib.check(_lib.lib().sept_wave_cloak_layout(self.utt_off_host.ctypes.data, self.n_utts, int(period),
-                                                         tile_off.ctypes.data))
+            _lib.call("sept_wave_cloak_layout", self.utt_off_host.ctypes.data, self.n_utts, int(period), tile_off.ctypes.data)
             self._tiles[period] = Tiles(tile_off, torch.from_numpy(tile_off).to(self.wav.device))
         return self._tiles[period]
 
@@ -114,21 +113,15 @@ def resample(batch: "RaggedAudio", orig_freq: int, new_freq: int = SAMPLE_RATE) 
         return batch
     n = batch.n_utts
     out_off = np.zeros(n + 1, dtype=np.int64)
-    _lib.check(_lib.lib().sept_resample_layout(batch.utt_off_host.ctypes.data, n, orig_freq, new_freq, out_off.ctypes.data))
+    _lib.call("sept_resample_layout", batch.utt_off_host.ctypes.data, n, orig_freq, new_freq, out_off.ctypes.data)
     dev = batch.wav.device
     out = torch.empty(int(out_off[-1]), dtype=torch.float32, device=dev)
     d_out_off = torch.from_numpy(out_off).to(dev)
-    with torch.cuda.device(dev):
-        _lib.check(_lib.lib().sept_resample_f32(batch.wav.data_ptr(), batch.utt_off.data_ptr(), d_out_off.data_ptr(), n,
-                                                int(out_off[-1]), orig_freq, new_freq, out.data_ptr(),
-                                                torch.cuda.current_stream(dev).cuda_stream))
+    _lib.launch("sept_resample_f32", batch.wav, batch.utt_off, d_out_off, n, int(out_off[-1]), orig_freq, new_freq, out,
+                device=dev)
     res = RaggedAudio.__new__(RaggedAudio)
     res.wav, res.utt_off_host, res.utt_off, res._layouts, res._tiles = out, out_off, d_out_off, {}, {}
     return res
-
-
-def _stream(device) -> int:
-    return torch.cuda.current_stream(device).cuda_stream
 
 
 def logmel(batch: RaggedAudio, n_fft: int = 800, n_mels: int = 128, hop: int = HOP_MEL, band_major: bool = False,
@@ -144,10 +137,8 @@ def logmel(batch: RaggedAudio, n_fft: int = 800, n_mels: int = 128, hop: int = H
     if out is None:
         shape = (lay.total_frames * n_mels,) if band_major else (lay.total_frames, n_mels)
         out = torch.empty(shape, dtype=torch.float32, device=dev)
-    with torch.cuda.device(dev):
-        _lib.check(_lib.lib().sept_logmel_f32(batch.wav.data_ptr(), batch.utt_off.data_ptr(), lay.frame_off.data_ptr(),
-                                              lay.item_off.data_ptr(), batch.n_utts, n_fft, hop, n_mels, int(deriv),
-                                              1 if band_major else 0, out.data_ptr(), _stream(dev)))
+    _lib.launch("sept_logmel_f32", batch.wav, batch.utt_off, lay.frame_off, lay.item_off, batch.n_utts, n_fft, hop, n_mels,
+                int(deriv), 1 if band_major else 0, out, device=dev)
     return out, lay
 
 
@@ -168,15 +159,10 @@ class LogMelFunction(torch.autograd.Function):
         (wav,) = ctx.saved_tensors
         batch, lay = ctx.batch, ctx.lay
         n_fft, n_mels, hop = ctx.shape
-        lib = _lib.lib()
         dwav = torch.zeros_like(wav)                              # samples outside every utterance get no gradient
-        ws = torch.empty(max(1, lib.sept_logmel_bwd_workspace_bytes(n_fft, hop, lay.n_items)), dtype=torch.uint8,
-                         device=wav.device)
-        grad = grad.contiguous()
-        with torch.cuda.device(wav.device):
-            _lib.check(lib.sept_logmel_bwd_f32(wav.data_ptr(), batch.utt_off.data_ptr(), lay.frame_off.data_ptr(),
-                                               lay.item_off.data_ptr(), batch.n_utts, lay.n_items, n_fft, hop, n_mels,
-                                               grad.data_ptr(), ws.data_ptr(), dwav.data_ptr(), _stream(wav.device)))
+        ws = _lib.workspace(_lib.lib().sept_logmel_bwd_workspace_bytes(n_fft, hop, lay.n_items), wav.device)
+        _lib.launch("sept_logmel_bwd_f32", wav, batch.utt_off, lay.frame_off, lay.item_off, batch.n_utts, lay.n_items, n_fft,
+                    hop, n_mels, grad.contiguous(), ws, dwav, device=wav.device)
         return dwav, None, None, None, None
 
 
@@ -206,10 +192,8 @@ def mfcc(batch: RaggedAudio, out: torch.Tensor | None = None) -> tuple[torch.Ten
         out = torch.empty(tf * 3 * N_MFCC, dtype=torch.float32, device=dev)
     scratch = torch.empty(tf * 257, dtype=torch.float32, device=dev)
     utt_max = torch.empty(2 * batch.n_utts, dtype=torch.int32, device=dev)
-    with torch.cuda.device(dev):
-        _lib.check(_lib.lib().sept_mfcc_f32(batch.wav.data_ptr(), batch.utt_off.data_ptr(), lay.frame_off.data_ptr(),
-                                            lay.item_off.data_ptr(), batch.n_utts, tf, scratch.data_ptr(),
-                                            utt_max.data_ptr(), out.data_ptr(), _stream(dev)))
+    _lib.launch("sept_mfcc_f32", batch.wav, batch.utt_off, lay.frame_off, lay.item_off, batch.n_utts, tf, scratch, utt_max,
+                out, device=dev)
     return out, lay
 
 
@@ -229,15 +213,10 @@ class MfccFunction(torch.autograd.Function):
     def backward(ctx, grad):
         (wav,) = ctx.saved_tensors
         batch, lay = ctx.batch, ctx.lay
-        lib = _lib.lib()
         dwav = torch.zeros_like(wav)                              # samples outside every utterance get no gradient
-        ws = torch.empty(max(1, lib.sept_mfcc_bwd_workspace_bytes(batch.n_utts, lay.total_frames, lay.n_items)),
-                         dtype=torch.uint8, device=wav.device)
-        grad = grad.contiguous()
-        with torch.cuda.device(wav.device):
-            _lib.check(lib.sept_mfcc_bwd_f32(wav.data_ptr(), batch.utt_off.data_ptr(), lay.frame_off.data_ptr(),
-                                             lay.item_off.data_ptr(), batch.n_utts, lay.total_frames, lay.n_items,
-                                             grad.data_ptr(), ws.data_ptr(), dwav.data_ptr(), _stream(wav.device)))
+        ws = _lib.workspace(_lib.lib().sept_mfcc_bwd_workspace_bytes(batch.n_utts, lay.total_frames, lay.n_items), wav.device)
+        _lib.launch("sept_mfcc_bwd_f32", wav, batch.utt_off, lay.frame_off, lay.item_off, batch.n_utts, lay.total_frames,
+                    lay.n_items, grad.contiguous(), ws, dwav, device=wav.device)
         return dwav, None
 
 
@@ -275,12 +254,11 @@ def logmel_host(wav_host: torch.Tensor, utt_off_host: np.ndarray, n_fft: int = 8
     if wav_host.is_cuda or wav_host.dtype not in (torch.float32, torch.int16) or wav_host.dim() != 1:
         raise ValueError("wav_host must be a 1-D float32 (or 16-bit PCM int16) host tensor")
     pcm16 = wav_host.dtype == torch.int16
-    lib = _lib.lib()
     off = np.ascontiguousarray(utt_off_host, dtype=np.int64)
     n = len(off) - 1
     frame_off = np.zeros(n + 1, dtype=np.int64)
     item_off = np.zeros(n + 1, dtype=np.int32)
-    _lib.check(lib.sept_extract_layout(off.ctypes.data, n, n_fft, hop, frame_off.ctypes.data, item_off.ctypes.data))
+    _lib.call("sept_extract_layout", off.ctypes.data, n, n_fft, hop, frame_off.ctypes.data, item_off.ctypes.data)
     total_frames = int(frame_off[-1])
     if out_host is None:
         out_host = torch.empty((total_frames, n_mels), dtype=torch.float32, pin_memory=True)
@@ -326,12 +304,12 @@ def logmel_host(wav_host: torch.Tensor, utt_off_host: np.ndarray, n_fft: int = 8
                 if pcm16:
                     pbuf = pcm_bufs[c % len(streams)]
                     pbuf[:ns].copy_(wav_host[int(off[a]):int(off[b])], non_blocking=True)
-                    _lib.check(lib.sept_pcm16_to_f32(pbuf.data_ptr(), ns, wbuf.data_ptr(), s.cuda_stream))
+                    _lib.call("sept_pcm16_to_f32", pbuf, ns, wbuf, s.cuda_stream)
                 else:
                     wbuf[:ns].copy_(wav_host[int(off[a]):int(off[b])], non_blocking=True)
                 base = tab_dev.data_ptr() + 8 * p
-                _lib.check(lib.sept_logmel_f32(wbuf.data_ptr(), base, base + 8 * k, base + 16 * k, b - a, n_fft, hop, n_mels,
-                                               0, 0, obuf.data_ptr(), s.cuda_stream))
+                _lib.call("sept_logmel_f32", wbuf, base, base + 8 * k, base + 16 * k, b - a, n_fft, hop, n_mels, 0, 0, obuf,
+                          s.cuda_stream)
                 out_host[frame_off[a]:frame_off[b]].copy_(obuf[:nf], non_blocking=True)
         for s in streams:
             main.wait_stream(s)

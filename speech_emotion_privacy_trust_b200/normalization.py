@@ -15,7 +15,7 @@ import torch
 from torch.autograd.function import once_differentiable
 
 from . import _lib
-from .extraction import Layout, _stream
+from .extraction import Layout
 
 WIN_LEN, SHIFT_LEN = 200, 50      # training_data_preprocess.sh:6-8 ; preprocess_adversary_data.py:131
 MODES = {"znorm": 0, "min_max": 1}
@@ -113,10 +113,8 @@ def _launch_speaker_stats(feat, lay, d_whole, win_len, shift_len, spk_lists) -> 
     n_utts, n_spk, F = len(lay.frame_off_host) - 1, d_ptr.numel() - 1, feat.shape[1]
     partial = torch.empty((n_utts, 5, F), dtype=torch.float32, device=dev)
     stats = torch.empty((n_spk, 5, F), dtype=torch.float32, device=dev)
-    with torch.cuda.device(dev):
-        _lib.check(_lib.lib().sept_speaker_stats_f32(
-            feat.data_ptr(), lay.frame_off.data_ptr(), 0 if d_whole is None else d_whole.data_ptr(), n_utts, F, win_len,
-            shift_len, d_ptr.data_ptr(), d_order.data_ptr(), n_spk, partial.data_ptr(), stats.data_ptr(), _stream(dev)))
+    _lib.launch("sept_speaker_stats_f32", feat, lay.frame_off, d_whole, n_utts, F, win_len, shift_len, d_ptr, d_order, n_spk,
+                partial, stats, device=dev)
     return stats
 
 
@@ -124,11 +122,8 @@ def normalize(feat: torch.Tensor, lay: Layout, st: SpeakerStats, mode: str = "zn
     """Frame-wise normalisation with each utterance's speaker statistics (:377-381); same shape as feat."""
     _check_feat(feat, st)
     out = torch.empty_like(feat)
-    dev = feat.device
-    with torch.cuda.device(dev):
-        _lib.check(_lib.lib().sept_normalize_f32(feat.data_ptr(), lay.frame_off.data_ptr(), st.spk_of_utt.data_ptr(),
-                                                 st.stats.data_ptr(), len(lay.frame_off_host) - 1, feat.shape[1], MODES[mode],
-                                                 out.data_ptr(), _stream(dev)))
+    _lib.launch("sept_normalize_f32", feat, lay.frame_off, st.spk_of_utt, st.stats, len(lay.frame_off_host) - 1, feat.shape[1],
+                MODES[mode], out, device=feat.device)
     return out
 
 
@@ -159,10 +154,8 @@ def normalized_windows(feat: torch.Tensor, lay: Layout, st: SpeakerStats, win_ut
     out = torch.empty((n, 1, win_len, F), dtype=torch.float32, device=dev)
     d_wu = torch.from_numpy(wu).to(dev)
     d_wt = torch.from_numpy(wt).to(dev)
-    with torch.cuda.device(dev):
-        _lib.check(_lib.lib().sept_normalize_windows_f32(
-            feat.data_ptr(), lay.frame_off.data_ptr(), st.spk_of_utt.data_ptr(), st.stats.data_ptr(), d_wu.data_ptr(),
-            d_wt.data_ptr(), n, win_len, F, MODES[mode], out.data_ptr(), _stream(dev)))
+    _lib.launch("sept_normalize_windows_f32", feat, lay.frame_off, st.spk_of_utt, st.stats, d_wu, d_wt, n, win_len, F,
+                MODES[mode], out, device=dev)
     return out
 
 
@@ -215,24 +208,19 @@ class SpeakerStatsFunction(torch.autograd.Function):
         from . import parallel
         feat, stats = ctx.saved_tensors
         lay, d_whole, win_len, shift_len, d_spk, (d_ptr, d_order), distributed, group = ctx.cfg
-        lib = _lib.lib()
         dev, n_utts, n_spk, F = feat.device, len(lay.frame_off_host) - 1, stats.shape[0], feat.shape[1]
         dstats = dstats.contiguous()
         if distributed:
             dstats = parallel.sum_in_rank_order(dstats, group)
         ties = torch.empty((n_spk, 2, F), dtype=torch.int32, device=dev)
-        ws = torch.empty(max(16, lib.sept_speaker_stats_bwd_ties_workspace_bytes(n_utts, F)), dtype=torch.uint8, device=dev)
+        ws = _lib.workspace(_lib.lib().sept_speaker_stats_bwd_ties_workspace_bytes(n_utts, F), dev)
         dfeat = torch.empty_like(feat)
-        whole = 0 if d_whole is None else d_whole.data_ptr()
-        with torch.cuda.device(dev):
-            _lib.check(lib.sept_speaker_stats_bwd_ties_i32(
-                feat.data_ptr(), lay.frame_off.data_ptr(), whole, n_utts, F, win_len, shift_len, d_spk.data_ptr(),
-                d_ptr.data_ptr(), d_order.data_ptr(), n_spk, stats.data_ptr(), ws.data_ptr(), ties.data_ptr(), _stream(dev)))
-            if distributed:
-                parallel.allreduce_exact_sum(ties, group)
-            _lib.check(lib.sept_speaker_stats_bwd_frames_f32(
-                feat.data_ptr(), lay.frame_off.data_ptr(), whole, n_utts, F, win_len, shift_len, d_spk.data_ptr(),
-                stats.data_ptr(), dstats.data_ptr(), ties.data_ptr(), dfeat.data_ptr(), _stream(dev)))
+        _lib.launch("sept_speaker_stats_bwd_ties_i32", feat, lay.frame_off, d_whole, n_utts, F, win_len, shift_len, d_spk,
+                    d_ptr, d_order, n_spk, stats, ws, ties, device=dev)
+        if distributed:
+            parallel.allreduce_exact_sum(ties, group)
+        _lib.launch("sept_speaker_stats_bwd_frames_f32", feat, lay.frame_off, d_whole, n_utts, F, win_len, shift_len, d_spk,
+                    stats, dstats, ties, dfeat, device=dev)
         return dfeat, None, None, None, None, None, None, None, None
 
 
@@ -302,24 +290,14 @@ class NormalizeFunction(torch.autograd.Function):
         need_feat, need_stats = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
         if not (need_feat or need_stats):
             return None, None, None, None, None, None
-        lib = _lib.lib()
         dev, n_utts, F = feat.device, len(lay.frame_off_host) - 1, feat.shape[1]
         dfeat = torch.empty_like(feat) if need_feat else None
         dstats = torch.empty_like(stats) if need_stats else None
-        ws = (torch.empty(max(16, lib.sept_normalize_bwd_workspace_bytes(n_utts, F)), dtype=torch.uint8, device=dev)
-              if need_stats else None)
+        ws = _lib.workspace(_lib.lib().sept_normalize_bwd_workspace_bytes(n_utts, F), dev) if need_stats else None
         d_wt, d_ptr, d_list, n_win, win_len = tables if tables is not None else (None, None, None, 0, 0)
         s_ptr, s_list = spk_lists if need_stats else (None, None)
-        grad = grad.contiguous()
-
-        def ptr(t):
-            return 0 if t is None else t.data_ptr()
-
-        with torch.cuda.device(dev):
-            _lib.check(lib.sept_normalize_bwd_f32(
-                feat.data_ptr(), lay.frame_off.data_ptr(), spk_of_utt.data_ptr(), stats.data_ptr(), ptr(d_wt), ptr(d_ptr),
-                ptr(d_list), n_win, win_len, n_utts, F, mode, grad.data_ptr(), ptr(s_ptr), ptr(s_list), stats.shape[0],
-                ptr(ws), ptr(dfeat), ptr(dstats), _stream(dev)))
+        _lib.launch("sept_normalize_bwd_f32", feat, lay.frame_off, spk_of_utt, stats, d_wt, d_ptr, d_list, n_win, win_len,
+                    n_utts, F, mode, grad.contiguous(), s_ptr, s_list, stats.shape[0], ws, dfeat, dstats, device=dev)
         return dfeat, dstats, None, None, None, None
 
 

@@ -19,10 +19,6 @@ DEFAULT_PERIOD = 32000     # one 200-frame training window at hop 160
 EPS_STD = 0.1              # cloak_noise's Normal(0, 0.1) (cloak_models.py:37)
 
 
-def _stream(device) -> int:
-    return torch.cuda.current_stream(device).cuda_stream
-
-
 def _aligned(t: torch.Tensor) -> torch.Tensor:
     """t, or a copy of it at a 16-byte aligned address (the kernels move float4s; a view at an odd offset needs the copy)."""
     return t if t.data_ptr() % 16 == 0 else t.clone()
@@ -35,7 +31,7 @@ def new_workspace(device: torch.device, period: int) -> tuple[torch.Tensor, torc
     nbytes = _lib.lib().sept_wave_cloak_bwd_workspace_bytes(period)
     if nbytes == 0:
         raise ValueError(f"period={period} must be a positive multiple of 4")
-    return (torch.empty(nbytes // 4, dtype=torch.float32, device=device), cloak_ops.new_workspace(device, period))
+    return _lib.workspace(nbytes, device), cloak_ops.new_workspace(device, period)
 
 
 class WaveCloakFunction(torch.autograd.Function):
@@ -62,10 +58,7 @@ class WaveCloakFunction(torch.autograd.Function):
                                                          min_scale, max_scale, want_noise=True, draw=draw)
         x = _aligned(wav.detach())
         y = torch.empty_like(x)
-        dev = x.device
-        with torch.cuda.device(dev):
-            _lib.check(_lib.lib().sept_wave_cloak_fwd_f32(x.data_ptr(), batch.utt_off.data_ptr(), batch.n_utts, x.numel(),
-                                                          noise.data_ptr(), period, y.data_ptr(), _stream(dev)))
+        _lib.launch("sept_wave_cloak_fwd_f32", x, batch.utt_off, batch.n_utts, x.numel(), noise, period, y, device=x.device)
         ctx.save_for_backward(eps_used, rhos_c)
         ctx.batch, ctx.tiles, ctx.workspace = batch, tiles, workspace
         ctx.cfg = (float(min_scale), float(max_scale), tuple(locs.shape), tuple(rhos.shape))
@@ -87,14 +80,10 @@ class WaveCloakFunction(torch.autograd.Function):
             r = torch.empty(period, dtype=torch.float32, device=dev)
             dlocs = torch.empty(period, dtype=torch.float32, device=dev)
             drhos = torch.empty(period, dtype=torch.float32, device=dev) if need_rhos else None
-            lib = _lib.lib()
-            with torch.cuda.device(dev):
-                _lib.check(lib.sept_wave_cloak_bwd_f32(gc.data_ptr(), batch.utt_off.data_ptr(), tiles.tile_off.data_ptr(),
-                                                       batch.n_utts, tiles.n_tiles, period, ws_r.data_ptr(), r.data_ptr(),
-                                                       _stream(dev)))
-                _lib.check(lib.sept_cloak_grl_bwd_f32(r.data_ptr(), None, 0.0, eps_used.data_ptr(), rhos_c.data_ptr(), None,
-                                                      min_scale, max_scale, 1, period, ws_c.data_ptr(), dlocs.data_ptr(),
-                                                      cloak_ops._ptr(drhos), None, _stream(dev)))
+            _lib.launch("sept_wave_cloak_bwd_f32", gc, batch.utt_off, tiles.tile_off, batch.n_utts, tiles.n_tiles, period, ws_r,
+                        r, device=dev)
+            _lib.launch("sept_cloak_grl_bwd_f32", r, None, 0.0, eps_used, rhos_c, None, min_scale, max_scale, 1, period, ws_c,
+                        dlocs, drhos, None, device=dev)
         return (g if need_wav else None, dlocs.view(lshape) if need_locs else None,
                 drhos.view(rshape) if need_rhos else None) + (None,) * 9
 

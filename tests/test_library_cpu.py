@@ -27,6 +27,31 @@ def test_library_exports_every_declared_symbol():
     assert [handle.sept_frames_per_item(n) for n in (400, 800, 1600, 1024)] == [8, 4, 2, 0]
 
 
+def test_signatures_are_read_from_the_header():
+    """The ctypes signatures come from include/sept.h: pointers and the stream as c_void_p, every scalar at its width (a
+    c_int where the header says int64_t would truncate without an error)."""
+    from speech_emotion_privacy_trust_b200 import _lib
+    handle = _lib.lib()
+    p, i, u64, f = ctypes.c_void_p, ctypes.c_int, ctypes.c_uint64, ctypes.c_float
+    fn = handle.sept_cloak_fwd_f32
+    assert fn.restype is i
+    assert fn.argtypes == [p, p, p, p, p, u64, u64, p, i, f, f, f, i, i, p, p, p, p]
+    fn = handle.sept_logmel_bwd_workspace_bytes
+    assert fn.restype is ctypes.c_size_t and fn.argtypes == [i, i, ctypes.c_int64]
+    fn = handle.sept_last_error
+    assert fn.restype is ctypes.c_char_p and fn.argtypes == []
+
+
+def test_signature_parser_rejects_an_unknown_type():
+    from speech_emotion_privacy_trust_b200 import _lib
+    good = "int sept_a(const double* x, /* int64_t in a comment */ int64_t n,\n           sept_stream_t s);"
+    assert _lib.signatures(good) == {"sept_a": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int64, ctypes.c_void_p])}
+    with pytest.raises(RuntimeError, match="'double'"):
+        _lib.signatures("int sept_b(double x);")
+    with pytest.raises(RuntimeError, match="'uint64_t'"):
+        _lib.signatures("uint64_t sept_c(void);")
+
+
 def test_loader_refuses_a_stale_library(tmp_path, monkeypatch):
     """VERDICT r1: a prebuilt .so compiled from other sources than the tree holds must never be tested silently.  The
     library carries the sha256 of its sources; the loader compares it with the tree and rebuilds or raises."""

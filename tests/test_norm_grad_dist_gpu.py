@@ -159,7 +159,6 @@ def test_backward_halves_write_every_element():
     on the tie-heavy corpus, and give speaker_stats_grad's feature gradient bit for bit."""
     from speech_emotion_privacy_trust_b200 import _lib
     from speech_emotion_privacy_trust_b200 import normalization as nz
-    from speech_emotion_privacy_trust_b200.extraction import _stream
     lib = _lib.lib()
     for n_feat in (128, 37):
         rng = np.random.default_rng(n_feat)
@@ -172,7 +171,7 @@ def test_backward_halves_write_every_element():
         d_whole = torch.from_numpy(np.asarray(whole, dtype=np.uint8)).cuda()
         stats = st.stats.detach()
         dstats = torch.from_numpy(rng.standard_normal(stats.shape).astype(np.float32)).cuda()
-        n_spk, s = len(st.speakers), _stream(feat.device)
+        n_spk, s = len(st.speakers), torch.cuda.current_stream(feat.device).cuda_stream
         ties = torch.full((n_spk, 2, n_feat), -7, dtype=torch.int32, device="cuda")
         ws = torch.empty(lib.sept_speaker_stats_bwd_ties_workspace_bytes(N_UTTS, n_feat), dtype=torch.uint8,
                          device="cuda")
