@@ -16,6 +16,7 @@
 
 #include "extract.h"
 #include "extract_core.cuh"
+#include "launch_shape.h"
 #include "tmem.cuh"
 
 namespace sept {
@@ -224,7 +225,7 @@ __device__ __forceinline__ void mel_fast(int lane, const pk2* P, uint32_t taddr,
     float* o;
     if (MODE == kModeDbBandMajor) o = prm.out + job.f0 * 128 + (long long)lane * job.T + job.t0;
     else o = prm.out + ((MODE == kModeMfccPower ? (long long)job.stream * prm.total_frames : 0) + job.f0 + job.t0) * 128 + lane;
-    const int band_stride = 32 * job.T;
+    const long long band_stride = 32LL * job.T;                   // 96 T overflows int from T = 22,369,622 frames
     float vmax = 0.f;
 #pragma unroll
     for (int r = 0; r < 4; ++r) {
@@ -480,21 +481,12 @@ __global__ void __launch_bounds__(ExtractWarps<R>::value * 32, 1) extract_kernel
 }
 
 
-// ---- host launchers ----------------------------------------------------------------------------------------
-constexpr size_t kMaxSmem = kMaxDynSmem - 64;  // minus the static shared memory (tmem_base, cta_next)
-
-template <int R>
-static int extract_warps(int hop, int n_mel_entries) {
-    using G = Geo<R>;
-    return warps_that_fit(extract_const_bytes(R, n_mel_entries), G::stage_floats(hop) * 4 + G::Y_PK4 * 16,
-                          ExtractWarps<R>::value, kMaxSmem);
-}
-
+// ---- host launchers (warps per CTA: launch_shape.h) ---------------------------------------------------------
 template <int R>
 static size_t extract_smem_bytes(int hop, int n_mel_entries) {
     using G = Geo<R>;
     const int w = extract_warps<R>(hop, n_mel_entries);
-    if (w == 0) return kMaxSmem + 1;
+    if (w == 0) return kExtractMaxSmem + 1;
     return (size_t)extract_const_bytes(R, n_mel_entries) + (size_t)w * (G::stage_floats(hop) * 4 + G::Y_PK4 * 16);
 }
 

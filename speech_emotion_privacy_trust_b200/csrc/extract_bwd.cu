@@ -13,6 +13,7 @@
 
 #include "extract_bwd.cuh"
 #include "extract_bwd.h"
+#include "launch_shape.h"
 
 namespace sept {
 
@@ -101,7 +102,7 @@ template <int R, int DERIV>
 static cudaError_t launch_frames(const LogmelBwdParams& prm, int sms, cudaStream_t stream) {
     const auto kernel = logmel_bwd_frames_kernel<R, DERIV>;
     const size_t cb = extract_const_bytes(R, prm.f.n_mel_entries), wb = Bwd<Geo<R>>::warp_floats(prm.f.hop, prm.f.n_mels) * 4;
-    const int warps = warps_that_fit(cb, wb, kBwdWarps, kMaxDynSmem);
+    const int warps = logmel_bwd_warps<R>(prm.f.hop, prm.f.n_mels, prm.f.n_mel_entries);
     if (warps == 0) return cudaErrorInvalidConfiguration;
     const size_t smem = cb + warps * wb;
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
