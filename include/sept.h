@@ -235,6 +235,27 @@ int sept_wave_cloak_layout(const int64_t* utt_off_host, int n_utts, int period, 
 int sept_wave_cloak_fwd_f32(const float* x_dev, const int64_t* utt_off_dev, int n_utts, int64_t n_samples,
                             const float* noise_dev, int period, float* y_dev, sept_stream_t stream);
 
+/* Evaluation with fresh noise per utterance: y[s] = x[s] + (locs[j] + sigma(rhos[j]) * eps_u[j]) for every sample s of
+ * utterance u, j = (s - utt_off[u]) mod period; samples before utt_off[0] and from utt_off[n_utts] to n_samples are
+ * copied.  The sum and the product are rounded separately, as in sept_cloak_fwd_f32.  eps_u is generated inside the kernel;
+ * no (n_utts, period) buffer is written.
+ * Draw rule (L = period): utterance u uses draw index d_u = (*draw_dev or 0) + utt_draw[u], or + u when utt_draw_dev
+ * is NULL. eps_u is bit for bit row d_u of what sept_cloak_fwd_f32(per_sample = 1, wf = L) draws: component j % 4 of
+ * normal4(seed, offset + d_u * ceil(L/4), j / 4, eps_std). It is the same Philox stream and the same (seed, offset, draw)
+ * rules as every other draw in the library.
+ * With global utterance ids in utt_draw_dev (int64, n_utts; the caller keeps them distinct and non-negative), an
+ * utterance's noisy audio depends neither on its batch, nor on its position in the batch, nor on the rank that holds it.
+ * The call does not advance *draw_dev (sept_counter_add_u64 does).  eps_dev (n_utts, period), indexed by batch position
+ * u, replaces the draw; it may be NULL.  workspace_dev holds sept_wave_cloak_eval_workspace_bytes(period) bytes (sigma of
+ * every phase, written by the call).  x_dev, y_dev, locs_dev, rhos_dev, eps_dev and workspace_dev 16-byte aligned; period
+ * and the offsets as above.  No atomics, no allocation, capturable. */
+size_t sept_wave_cloak_eval_workspace_bytes(int period);
+int sept_wave_cloak_eval_f32(const float* x_dev, const int64_t* utt_off_dev, int n_utts, int64_t n_samples,
+                             const float* locs_dev, const float* rhos_dev, const float* eps_dev,
+                             uint64_t seed, uint64_t offset, const uint64_t* draw_dev, const int64_t* utt_draw_dev,
+                             float eps_std, float min_scale, float max_scale, int period,
+                             void* workspace_dev, float* y_dev, sept_stream_t stream);
+
 /* Backward of sept_wave_cloak_fwd_f32 with respect to the noise: r[j] = the sum of g over every in-utterance sample of
  * phase j, r_dev (period).  dx = g needs no call; dlocs = r and drhos = r * eps * dsigma/drho follow from
  * sept_cloak_grl_bwd_f32(g_a = r, batch = 1, mask = NULL).  tile_off_dev is sept_wave_cloak_layout's table on the device,

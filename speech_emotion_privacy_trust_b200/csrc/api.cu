@@ -587,6 +587,27 @@ int sept_wave_cloak_fwd_f32(const float* x, const int64_t* utt_off, int n_utts, 
     return SEPT_OK;
 }
 
+size_t sept_wave_cloak_eval_workspace_bytes(int period) {
+    return period > 0 && period % 4 == 0 ? (size_t)period * sizeof(float) : 0;
+}
+
+int sept_wave_cloak_eval_f32(const float* x, const int64_t* utt_off, int n_utts, int64_t n_samples, const float* locs,
+                             const float* rhos, const float* eps, uint64_t seed, uint64_t offset, const uint64_t* draw_dev,
+                             const int64_t* utt_draw_dev, float eps_std, float min_scale, float max_scale, int period,
+                             void* workspace, float* y, sept_stream_t stream) {
+    if (!x || !utt_off || !locs || !rhos || !workspace || !y || n_utts < 0 || n_samples < 0 || period <= 0)
+        return fail(SEPT_E_BADARG, "sept_wave_cloak_eval_f32: bad argument");
+    if (period % 4) return fail(SEPT_E_BADARG, "sept_wave_cloak_eval_f32: period=%d must be a multiple of 4", period);
+    if (!aligned16(x) || !aligned16(locs) || !aligned16(rhos) || !aligned16(eps) || !aligned16(workspace) || !aligned16(y))
+        return fail(SEPT_E_BADARG, "sept_wave_cloak_eval_f32: pointers must be 16-byte aligned");
+    sept::WaveEvalParams p{};
+    p.x = x; p.utt_off = utt_off; p.n_utts = n_utts; p.n = n_samples; p.locs = locs; p.rhos = rhos; p.eps = eps;
+    p.seed = seed; p.offset = offset; p.draw = draw_dev; p.utt_draw = utt_draw_dev; p.eps_std = eps_std;
+    p.min_scale = min_scale; p.max_scale = max_scale; p.period = period; p.sigma = static_cast<float*>(workspace); p.y = y;
+    SEPT_CUDA(sept::launch_wave_eval(p, static_cast<cudaStream_t>(stream)));
+    return SEPT_OK;
+}
+
 size_t sept_wave_cloak_bwd_workspace_bytes(int period) {
     return period > 0 && period % 4 == 0 ? (size_t)sept::kWaveSlices * period * sizeof(float) : 0;
 }

@@ -16,6 +16,7 @@
 #include <cstdint>
 
 #include "cloak.h"
+#include "cloak_noise.cuh"
 #include "philox.cuh"
 
 namespace sept {
@@ -23,20 +24,15 @@ namespace sept {
 __device__ __forceinline__ float4 ld4(const float* p) { return *reinterpret_cast<const float4*>(p); }
 __device__ __forceinline__ void st4(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
 
-__device__ __forceinline__ float sigma_of(float rho, float mn, float mx) {
-    return __fadd_rn(__fmul_rn((1.0f + tanhf(rho)) / 2.0f, mx - mn), mn);   // operation order of cloak_models.py:43
-}
-
 constexpr int kCloakThreads = 128;
 
 __device__ __forceinline__ float4 cloak_noise4(const CloakFwdParams& p, float4 mu, float4 rho, float4 e, float4 m) {
     if (p.mask) { e.x *= m.x; e.y *= m.y; e.z *= m.z; e.w *= m.w; }
     float4 nz;
-    // product and sum rounded separately, like the reference's two ATen ops (no FMA contraction)
-    nz.x = __fadd_rn(mu.x, __fmul_rn(sigma_of(rho.x, p.min_scale, p.max_scale), e.x));
-    nz.y = __fadd_rn(mu.y, __fmul_rn(sigma_of(rho.y, p.min_scale, p.max_scale), e.y));
-    nz.z = __fadd_rn(mu.z, __fmul_rn(sigma_of(rho.z, p.min_scale, p.max_scale), e.z));
-    nz.w = __fadd_rn(mu.w, __fmul_rn(sigma_of(rho.w, p.min_scale, p.max_scale), e.w));
+    nz.x = noise_of(mu.x, sigma_of(rho.x, p.min_scale, p.max_scale), e.x);
+    nz.y = noise_of(mu.y, sigma_of(rho.y, p.min_scale, p.max_scale), e.y);
+    nz.z = noise_of(mu.z, sigma_of(rho.z, p.min_scale, p.max_scale), e.z);
+    nz.w = noise_of(mu.w, sigma_of(rho.w, p.min_scale, p.max_scale), e.w);
     return nz;
 }
 

@@ -1,0 +1,15 @@
+// The cloak's per-element noise, shared by the feature cloak (cloak.cu) and the waveform cloak's evaluation kernel
+// (wave_cloak.cu), so both evaluate one definition of sigma and of mu + sigma * eps.
+#pragma once
+#include <cuda_runtime.h>
+
+namespace sept {
+
+__device__ __forceinline__ float sigma_of(float rho, float mn, float mx) {
+    return __fadd_rn(__fmul_rn((1.0f + tanhf(rho)) / 2.0f, mx - mn), mn);   // operation order of cloak_models.py:43
+}
+
+// product and sum rounded separately, like the reference's two ATen ops (no FMA contraction)
+__device__ __forceinline__ float noise_of(float mu, float sigma, float eps) { return __fadd_rn(mu, __fmul_rn(sigma, eps)); }
+
+}  // namespace sept

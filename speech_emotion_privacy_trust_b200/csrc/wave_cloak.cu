@@ -14,11 +14,17 @@
 //                       are added to the slice's row in chunk order.  R = 1 when L/4 >= 256 quads, else 256 / (L/4).
 //   wave_merge_kernel   backward, pass 2: r[j] = the slices summed in order: lane l of 8 sums slices 74l .. 74l+73 in
 //                       order, the 8 lane sums are added in lane order.
+//   wave_sigma_kernel   evaluation, pre-pass: sigma(rhos[j]) of the period into the caller's workspace, once per call.
+//   wave_eval_add_kernel evaluation: y[s] = x[s] + (mu[j] + sigma[j] * eps_u[j]), j = (s - utt_off[u]) mod L, a fresh
+//                       eps_u per utterance drawn inside the kernel (row d_u of sept_cloak_fwd_f32's per-sample draw);
+//                       a thread walks the phase quads that start in its aligned quad, one normal4 per phase quad.
 // No atomics: the order above is fixed, so the gradient is the same bits on every run (tests/wave_cloak_order.py
-// restates it on the host).  All three are HBM-bound with no reuse of x, y or g.
+// restates it on the host).  The add and the backward are HBM-bound with no reuse of x, y or g.
 #include <cuda_runtime.h>
 #include <cstdint>
 
+#include "cloak_noise.cuh"
+#include "philox.cuh"
 #include "wave_cloak.h"
 
 namespace sept {
@@ -94,6 +100,115 @@ __global__ void __launch_bounds__(kWaveThreads) wave_add_kernel(const WaveAddPar
                     val += __ldg(p.noise + (uint32_t)(t - p.utt_off[w]) % L);
                 }
                 p.y[t] = val;
+            }
+        }
+    }
+}
+
+__global__ void __launch_bounds__(kWaveThreads) wave_sigma_kernel(const float* __restrict__ rhos, int L, float mn, float mx,
+                                                                  float* __restrict__ sigma) {
+    for (int j = blockIdx.x * kWaveThreads + threadIdx.x; j < L; j += gridDim.x * kWaveThreads) sigma[j] = sigma_of(rhos[j], mn, mx);
+}
+
+struct EvalUtt {
+    int64_t b;               // first sample
+    uint64_t ctr;            // Philox counter of phase quad 0: offset + draw index * L/4
+    const float* eps;        // the caller's row, or null
+};
+
+__device__ __forceinline__ EvalUtt eval_utt(const WaveEvalParams& p, int u, uint64_t draw0) {
+    const uint64_t d = draw0 + (p.utt_draw ? (uint64_t)p.utt_draw[u] : (uint64_t)u);
+    return {p.utt_off[u], p.offset + d * (uint64_t)(p.period / 4), p.eps ? p.eps + (size_t)u * p.period : nullptr};
+}
+
+// mu + sigma * eps of the phases j .. j+3 (j a multiple of 4): one normal4, the same one sept_cloak_fwd_f32 draws for
+// row d, elements j .. j+3
+__device__ __forceinline__ float4 eval_noise4(const WaveEvalParams& p, const EvalUtt& t, uint32_t j) {
+    const float4 e = t.eps ? __ldg(reinterpret_cast<const float4*>(t.eps + j)) : normal4(p.seed, t.ctr, j / 4, p.eps_std);
+    const float4 mu = __ldg(reinterpret_cast<const float4*>(p.locs + j));
+    const float4 sg = __ldg(reinterpret_cast<const float4*>(p.sigma + j));
+    return make_float4(noise_of(mu.x, sg.x, e.x), noise_of(mu.y, sg.y, e.y), noise_of(mu.z, sg.z, e.z), noise_of(mu.w, sg.w, e.w));
+}
+
+// four consecutive samples at x + s, where s = a (mod 4) and x is 16-byte aligned
+__device__ __forceinline__ float4 ld_quad(const float* x, int64_t s, int a) {
+    if (a == 0) return __ldcs(reinterpret_cast<const float4*>(x + s));
+    if (a == 2) {
+        const float2 l = __ldcs(reinterpret_cast<const float2*>(x + s)), h = __ldcs(reinterpret_cast<const float2*>(x + s + 2));
+        return make_float4(l.x, l.y, h.x, h.y);
+    }
+    return make_float4(__ldcs(x + s), __ldcs(x + s + 1), __ldcs(x + s + 2), __ldcs(x + s + 3));
+}
+
+__device__ __forceinline__ void st_quad(float* y, int64_t s, int a, float4 v) {
+    if (a == 0) { __stcs(reinterpret_cast<float4*>(y + s), v); return; }
+    if (a == 2) {
+        __stcs(reinterpret_cast<float2*>(y + s), make_float2(v.x, v.y));
+        __stcs(reinterpret_cast<float2*>(y + s + 2), make_float2(v.z, v.w));
+        return;
+    }
+    __stcs(y + s, v.x); __stcs(y + s + 1, v.y); __stcs(y + s + 2, v.z); __stcs(y + s + 3, v.w);
+}
+
+constexpr int kEvalUnroll = 4;   // quads whose x is loaded before the first draw
+
+// Thread q owns the phase quads that start in the aligned quad [4q, 4q + 4): utterance u's phase quad k covers samples
+// b_u + 4k .. + 3 (clipped to the utterance), and exactly one of its samples 4q + (b_u & 3) lies in each aligned quad.
+// So every in-utterance sample is written once, one normal4 per phase quad, and x / y are moved at the utterance's
+// alignment (float4, two float2 or four floats).  The common case is a phase quad wholly inside the utterance that also
+// covers the whole aligned quad; anything else (an utterance start, end or gap in the quad) goes to the general path.
+__global__ void __launch_bounds__(kWaveThreads) wave_eval_add_kernel(const WaveEvalParams p) {
+    const int64_t nq = (p.n + 3) / 4;
+    const int64_t per = (nq + gridDim.x - 1) / gridDim.x;
+    const int64_t q0 = (int64_t)blockIdx.x * per, q1 = q0 + per < nq ? q0 + per : nq;
+    if (q0 + threadIdx.x >= q1) return;
+    const int64_t lo = p.utt_off[0], hi = p.utt_off[p.n_utts];      // samples outside [lo, hi) are copied
+    const uint32_t L = (uint32_t)p.period;
+    const uint64_t draw0 = p.draw ? *p.draw : 0;
+    int u = last_le(p.utt_off, p.n_utts, 4 * (q0 + threadIdx.x));
+    int64_t b = 0, e = 0;                                           // bounds of utterance u (read once u is in range)
+    bool have = false;
+    int tu = -1;                                                    // the utterance t describes
+    EvalUtt t{};
+    for (int64_t qb = q0 + threadIdx.x; qb < q1; qb += kEvalUnroll * kWaveThreads) {
+        float4 v[kEvalUnroll];
+        int uk[kEvalUnroll];
+        bool fast[kEvalUnroll];
+#pragma unroll
+        for (int k = 0; k < kEvalUnroll; ++k) {
+            const int64_t q = qb + (int64_t)k * kWaveThreads, s0 = 4 * q;
+            fast[k] = false;
+            if (q >= q1) continue;
+            if (s0 >= lo) {
+                while (u + 1 < p.n_utts && p.utt_off[u + 1] <= s0) { ++u; have = false; }
+            }
+            if (!have && p.n_utts > 0) { b = p.utt_off[u]; e = p.utt_off[u + 1]; have = true; }
+            uk[k] = u;
+            const int a = (int)(b & 3);
+            fast[k] = have && b <= s0 && s0 + a + 4 <= e;
+            if (fast[k]) v[k] = ld_quad(p.x, s0 + a, a);
+        }
+#pragma unroll
+        for (int k = 0; k < kEvalUnroll; ++k) {
+            const int64_t q = qb + (int64_t)k * kWaveThreads, s0 = 4 * q;
+            if (q >= q1) break;
+            if (fast[k]) {
+                if (uk[k] != tu) { t = eval_utt(p, uk[k], draw0); tu = uk[k]; }
+                const int a = (int)(t.b & 3);
+                const int64_t s = s0 + a;
+                const float4 nz = eval_noise4(p, t, (uint32_t)(s - t.b) % L), x = v[k];
+                st_quad(p.y, s, a, make_float4(__fadd_rn(x.x, nz.x), __fadd_rn(x.y, nz.y), __fadd_rn(x.z, nz.z), __fadd_rn(x.w, nz.w)));
+                continue;
+            }
+            const int64_t s1 = s0 + 4 < p.n ? s0 + 4 : p.n;
+            for (int64_t s = s0; s < s1; ++s)                       // samples outside every utterance
+                if (s < lo || s >= hi) p.y[s] = p.x[s];
+            for (int w = uk[k]; w < p.n_utts && p.utt_off[w] < s0 + 4; ++w) {   // phase quads starting in this quad
+                const EvalUtt tw = eval_utt(p, w, draw0);
+                const int64_t s = s0 + (tw.b & 3), ew = p.utt_off[w + 1];
+                if (s < tw.b || s >= ew) continue;
+                float4 nz = eval_noise4(p, tw, (uint32_t)(s - tw.b) % L);
+                for (int c = 0; c < 4 && s + c < ew; ++c) p.y[s + c] = __fadd_rn(p.x[s + c], f4at(nz, c));
             }
         }
     }
@@ -194,6 +309,23 @@ cudaError_t launch_wave_add(const WaveAddParams& p, cudaStream_t stream) {
     const int64_t nq = (p.n + 3) / 4, want = (nq + kAddUnroll * kWaveThreads - 1) / (kAddUnroll * kWaveThreads);
     const int blocks = (int)(want < (int64_t)sms * 8 ? want : (int64_t)sms * 8);     // 8 CTAs (2048 threads) per SM
     wave_add_kernel<<<blocks, kWaveThreads, 0, stream>>>(p);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_wave_eval(const WaveEvalParams& p, cudaStream_t stream) {
+    if (p.n == 0) return cudaSuccess;
+    int dev = 0, sms = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    if (e != cudaSuccess) return e;
+    const int sb = (p.period + kWaveThreads - 1) / kWaveThreads;
+    wave_sigma_kernel<<<sb < sms ? sb : sms, kWaveThreads, 0, stream>>>(p.rhos, p.period, p.min_scale, p.max_scale, p.sigma);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    const int64_t nq = (p.n + 3) / 4, want = (nq + kEvalUnroll * kWaveThreads - 1) / (kEvalUnroll * kWaveThreads);
+    const int blocks = (int)(want < (int64_t)sms * 8 ? want : (int64_t)sms * 8);
+    wave_eval_add_kernel<<<blocks, kWaveThreads, 0, stream>>>(p);
     return cudaGetLastError();
 }
 

@@ -32,7 +32,25 @@ struct WaveReduceParams {
     float* r;                // (period)
 };
 
+struct WaveEvalParams {
+    const float* x;          // (n) 16-byte aligned
+    const int64_t* utt_off;  // (n_utts + 1) device
+    int n_utts;
+    int64_t n;
+    const float* locs;       // (period) 16-byte aligned
+    const float* rhos;       // (period) 16-byte aligned
+    const float* eps;        // (n_utts, period) 16-byte aligned, or null -> Philox(seed, offset)
+    uint64_t seed, offset;
+    const uint64_t* draw;    // device counter or null (0)
+    const int64_t* utt_draw; // (n_utts) device draw index of each utterance, or null (u)
+    float eps_std, min_scale, max_scale;
+    int period;              // multiple of 4
+    float* sigma;            // workspace (period): sigma(rhos), written by the pre-pass
+    float* y;                // (n) 16-byte aligned
+};
+
 cudaError_t launch_wave_add(const WaveAddParams& p, cudaStream_t stream);
+cudaError_t launch_wave_eval(const WaveEvalParams& p, cudaStream_t stream);
 cudaError_t launch_wave_reduce(const WaveReduceParams& p, cudaStream_t stream);
 
 }  // namespace sept

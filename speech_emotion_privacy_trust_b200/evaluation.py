@@ -6,6 +6,9 @@ copies two softmax rows to the host per window, and finally averages them and ta
 (training/adversary_cloak_evaluation.py:60-93).  Here all windows of many utterances go through one forward: windows are
 gathered and normalised by sept_normalize_windows_f32, the cloak kernel gives every window its own eps (per_sample), the
 softmax rows are averaged per utterance with one index_add, and only the predictions travel to the host.
+
+A waveform cloak (wave_cloak.WaveCloak) is evaluated by wave_cloak_evaluate: the noise goes on the test audio, one fresh
+sample per utterance, before extraction; the window loop is the same.
 """
 from __future__ import annotations
 
@@ -14,8 +17,8 @@ from typing import Sequence
 import numpy as np
 import torch
 
-from . import cloak_ops, normalization
-from .extraction import Layout
+from . import cloak_ops, extraction, normalization
+from .extraction import Layout, RaggedAudio
 
 EPS_STD = 0.1
 
@@ -50,15 +53,7 @@ def cloak_evaluate(noise_layer, baseline_model, adversary_model, feat: torch.Ten
     once per window, in window order, exactly like the reference's loop; `layer.external_eps` -- ONE (1, W, F) sample --
     would give every window the same noise, which the reference never does, so it is rejected; otherwise eps comes from
     the device Philox stream (one draw per window, counter advanced by the number of windows)."""
-    baseline_model.eval()
-    adversary_model.eval()
     dev = feat.device
-    utts = list(range(len(lay.frame_off_host) - 1)) if utts is None else list(utts)
-    win_utt, win_t0 = eval_window_table(lay, utts)
-    n_win, n_utt = len(win_utt), len(utts)
-    slot = {u: i for i, u in enumerate(utts)}
-    seg_host = np.fromiter((slot[int(u)] for u in win_utt), dtype=np.int64, count=n_win)      # non-decreasing
-    counts = torch.from_numpy(np.maximum(np.bincount(seg_host, minlength=n_utt), 1)).to(dev).unsqueeze(1).float()
     locs, rhos = noise_layer.locs.detach().float().contiguous(), noise_layer.rhos.detach().float().contiguous()
     mask_c = None if mask is None else mask.detach().to(dev).float().contiguous()
     lo, hi = noise_layer._bounds() if hasattr(noise_layer, "_bounds") else (float(noise_layer.min_scale), float(noise_layer.max_scale))
@@ -66,10 +61,9 @@ def cloak_evaluate(noise_layer, baseline_model, adversary_model, feat: torch.Ten
         raise ValueError("cloak_evaluate draws one eps per window; layer.external_eps holds a single sample -- pass "
                          "external_eps=(n_windows, W, F) instead")
     sampler = vars(noise_layer.normal).get("sample") if external_eps is None and hasattr(noise_layer, "normal") else None
-    emo_sum = gen_sum = None
-    for a in range(0, n_win, max_windows):
-        b = min(n_win, a + max_windows)
-        x = normalization.normalized_windows(feat, lay, stats, win_utt[a:b], win_t0[a:b], mode=norm_mode)
+
+    def noisy_windows(a, b, wu, wt):
+        x = normalization.normalized_windows(feat, lay, stats, wu, wt, mode=norm_mode)
         eps = None
         seed, draw = 0, None
         if external_eps is not None:
@@ -79,8 +73,30 @@ def cloak_evaluate(noise_layer, baseline_model, adversary_model, feat: torch.Ten
         else:
             _, seed, draw = noise_layer._eps_source()
         noisy, _, _ = cloak_ops.cloak_forward_raw(x, locs, rhos, mask_c, eps, seed, 0, EPS_STD, lo, hi, draw=draw, per_sample=True)
-        p_emo = torch.softmax(baseline_model(noisy), dim=1)
-        p_gen = torch.softmax(adversary_model(noisy), dim=1)
+        return noisy
+
+    return _classify_windows(baseline_model, adversary_model, lay, utts, noisy_windows, max_windows, dev)
+
+
+@torch.no_grad()
+def _classify_windows(baseline_model, adversary_model, lay: Layout, utts, windows, max_windows: int, dev):
+    """The evaluation loop both evaluators share: the windows of eval_window_table(lay, utts) in chunks of max_windows,
+    windows(a, b, win_utt[a:b], win_t0[a:b]) -> the classifiers' (b - a, 1, W, F) input, softmax of both models, the
+    per-utterance mean and argmax.  Returns (emotion_pred, gender_pred, emotion_prob, gender_prob) on the host."""
+    baseline_model.eval()
+    adversary_model.eval()
+    utts = list(range(len(lay.frame_off_host) - 1)) if utts is None else list(utts)
+    win_utt, win_t0 = eval_window_table(lay, utts)
+    n_win, n_utt = len(win_utt), len(utts)
+    slot = {u: i for i, u in enumerate(utts)}
+    seg_host = np.fromiter((slot[int(u)] for u in win_utt), dtype=np.int64, count=n_win)      # non-decreasing
+    counts = torch.from_numpy(np.maximum(np.bincount(seg_host, minlength=n_utt), 1)).to(dev).unsqueeze(1).float()
+    emo_sum = gen_sum = None
+    for a in range(0, n_win, max_windows):
+        b = min(n_win, a + max_windows)
+        x = windows(a, b, win_utt[a:b], win_t0[a:b])
+        p_emo = torch.softmax(baseline_model(x), dim=1)
+        p_gen = torch.softmax(adversary_model(x), dim=1)
         if emo_sum is None:
             emo_sum = torch.zeros((n_utt, p_emo.shape[1]), device=dev)
             gen_sum = torch.zeros((n_utt, p_gen.shape[1]), device=dev)
@@ -93,3 +109,34 @@ def cloak_evaluate(noise_layer, baseline_model, adversary_model, feat: torch.Ten
     out = torch.cat([emo_prob.argmax(1, keepdim=True).float(), gen_prob.argmax(1, keepdim=True).float(), emo_prob, gen_prob], 1).cpu()
     ne = emo_prob.shape[1]
     return out[:, 0].long().numpy(), out[:, 1].long().numpy(), out[:, 2:2 + ne].numpy(), out[:, 2 + ne:].numpy()
+
+
+def _check_stats_source(speaker_of_utt, stats) -> None:
+    if (speaker_of_utt is None) == (stats is None):
+        raise ValueError("give exactly one of speaker_of_utt (statistics of the noisy test features) and stats")
+
+
+@torch.no_grad()
+def wave_cloak_evaluate(layer, baseline_model, adversary_model, batch: RaggedAudio, speaker_of_utt: Sequence | None = None,
+                        stats: normalization.SpeakerStats | None = None, utts: Sequence[int] | None = None, utt_ids=None,
+                        n_draws: int | None = None, external_eps: torch.Tensor | None = None, n_fft: int = 800,
+                        n_mels: int = 128, norm_mode: str = "znorm", max_windows: int = 512):
+    """Evaluation of a waveform cloak (wave_cloak.WaveCloak) on test audio: configs 2 and 5 of BASELINE.json with the
+    noise on the signal.  Returns what cloak_evaluate returns, (emotion_pred, gender_pred, emotion_prob, gender_prob) per
+    utterance of `utts` (default all), on the host.
+
+    Every utterance gets its own noise sample (layer.noisy_per_utterance: utt_ids, n_draws and external_eps as there), tiled
+    from its first sample -- the signal-domain counterpart of the reference's fresh eps per window, whose 200-frame
+    windows overlap by 150 frames of audio.  Then log-mel (extraction.logmel, n_fft / n_mels), per-speaker statistics,
+    the test windows (eval_window_table) normalised in chunks of max_windows, both classifiers, the per-utterance softmax
+    mean and argmax.  Statistics: `stats`, or those of the noisy features of the batch by speaker_of_utt with every
+    utterance counted whole (the test split's rule, preprocess_adversary_data.py:56-60); exactly one must be given.  Under
+    data parallelism pass speaker_stats_distributed statistics of the noisy features and global utt_ids."""
+    _check_stats_source(speaker_of_utt, stats)
+    noisy = layer.noisy_per_utterance(batch, utt_ids=utt_ids, n_draws=n_draws, external_eps=external_eps)
+    feat, lay = extraction.logmel(noisy, n_fft=n_fft, n_mels=n_mels)
+    if stats is None:
+        stats = normalization.speaker_stats(feat, lay, speaker_of_utt, whole_utterance=[True] * batch.n_utts)
+    return _classify_windows(baseline_model, adversary_model, lay, utts,
+                             lambda a, b, wu, wt: normalization.normalized_windows(feat, lay, stats, wu, wt, mode=norm_mode),
+                             max_windows, feat.device)

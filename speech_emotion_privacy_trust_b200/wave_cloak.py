@@ -5,9 +5,12 @@ The signal-domain counterpart of cloak_noise (model/cloak_models.py:24-58): the 
 sigma = (1 + tanh rho)/2 * (max_scale - min_scale) + min_scale, the same device Philox eps (one (L,) sample per forward,
 identical on every rank, fresh on every CUDA-graph replay) and a deterministic backward.  Forward: sept_cloak_fwd_f32 draws
 noise = mu + sigma * eps, sept_wave_cloak_fwd_f32 tiles it over every utterance from the utterance's first sample.
-Backward: dx = g; sept_wave_cloak_bwd_f32 sums g per phase, sept_cloak_grl_bwd_f32 turns that sum into dlocs and drhos."""
+Backward: dx = g; sept_wave_cloak_bwd_f32 sums g per phase, sept_cloak_grl_bwd_f32 turns that sum into dlocs and drhos.
+Evaluation (WaveCloak.noisy_per_utterance): sept_wave_cloak_eval_f32 gives every utterance its own eps, drawn inside the
+add kernel."""
 from __future__ import annotations
 
+import numpy as np
 import torch
 import torch.nn as nn
 from torch.autograd.function import once_differentiable
@@ -135,3 +138,57 @@ class WaveCloak(nn.Module):
         wav = WaveCloakFunction.apply(batch.wav, self.locs, self.rhos, batch, eps, seed, 0, EPS_STD, self.min_scale,
                                       self.max_scale, draw, self._ws())
         return batch.with_wav(wav)
+
+    @torch.no_grad()
+    def noisy_per_utterance(self, batch: RaggedAudio, utt_ids=None, n_draws: int | None = None,
+                            external_eps: torch.Tensor | None = None) -> RaggedAudio:
+        """The batch under the cloak with a fresh eps per utterance, as evaluation needs it (the reference never
+        evaluates with one noise sample shared by many utterances): utterance u gets locs + scales() * eps_u tiled from
+        its first sample, eps_u drawn on the device from draw index (layer counter) + utt_ids[u].  Returns a RaggedAudio
+        with the same offsets and cached layouts.
+
+        utt_ids: the utterances' global draw ids (default 0 .. n_utts - 1), non-negative, distinct and below n_draws
+        (default n_utts).  With global ids an utterance's noise depends neither on its batch, nor on its position, nor on
+        the rank holding it; the layer's draw counter then advances by n_draws, so the ranks of a sharded evaluation stay
+        in step.  external_eps: (n_utts, period) samples, one per utterance in batch order (parity tests); the counter does
+        not move.  layer.external_eps holds a single sample and is rejected, as cloak_evaluate rejects it."""
+        n = batch.n_utts
+        L = self.period
+        n_draws = n if n_draws is None else int(n_draws)
+        ids = None
+        if utt_ids is not None:
+            ids = np.asarray(utt_ids).reshape(-1)
+            if ids.size and not np.issubdtype(ids.dtype, np.integer):
+                raise ValueError(f"utt_ids must be integers, got {ids.dtype}")
+            ids = ids.astype(np.int64)
+            if len(ids) != n:
+                raise ValueError(f"utt_ids has {len(ids)} entries; the batch has {n} utterances")
+            if len(ids) and (ids.min() < 0 or ids.max() >= n_draws):
+                raise ValueError(f"utt_ids must lie in [0, n_draws = {n_draws})")
+            if len(np.unique(ids)) != len(ids):
+                raise ValueError("utt_ids must be distinct: two utterances would share one noise sample")
+        elif n > n_draws:
+            raise ValueError(f"n_draws = {n_draws} is smaller than the batch's {n} utterances")
+        if external_eps is not None:
+            if tuple(external_eps.shape) != (n, L):
+                raise ValueError(f"external_eps must be (n_utts, period) = ({n}, {L}), got {tuple(external_eps.shape)}")
+        elif self.external_eps is not None:
+            raise ValueError("noisy_per_utterance draws one eps per utterance; layer.external_eps holds a single sample -- "
+                             "pass external_eps=(n_utts, period) instead")
+        _lib.require_cuda(batch.wav)
+        dev = batch.wav.device
+        x = _aligned(batch.wav.detach())
+        locs_c, rhos_c = cloak_ops._f32c(self.locs.detach()), cloak_ops._f32c(self.rhos.detach())
+        if external_eps is not None:
+            eps, seed, draw = _aligned(cloak_ops._f32c(external_eps.detach().to(dev))), 0, None
+        else:
+            eps, seed, draw = self._eps_source()
+        d_ids = None if ids is None else torch.from_numpy(ids).to(dev)
+        ws = _lib.workspace(_lib.lib().sept_wave_cloak_eval_workspace_bytes(L), dev)
+        y = torch.empty_like(x)
+        _lib.launch("sept_wave_cloak_eval_f32", x, batch.utt_off, n, x.numel(), locs_c, rhos_c, eps,
+                    int(seed) & 0xFFFFFFFFFFFFFFFF, 0, draw, d_ids, EPS_STD, self.min_scale, self.max_scale, L, ws, y,
+                    device=dev)
+        if draw is not None:
+            _lib.launch("sept_counter_add_u64", draw, n_draws, device=dev)
+        return batch.with_wav(y)
