@@ -266,6 +266,24 @@ size_t sept_wave_cloak_bwd_workspace_bytes(int period);
 int sept_wave_cloak_bwd_f32(const float* g_dev, const int64_t* utt_off_dev, const int64_t* tile_off_dev, int n_utts,
                             int64_t n_tiles, int period, void* workspace_dev, float* r_dev, sept_stream_t stream);
 
+/* Backward of sept_wave_cloak_eval_f32 with respect to locs and rhos, for training with fresh noise per utterance:
+ * dlocs[j] = the sum of g over every in-utterance sample of phase j (the bits of sept_wave_cloak_bwd_f32's r), and
+ * drhos[j] = q[j] * dsigma/drho(rhos[j]), q[j] = the sum of g * eps_u[j] over the same samples, each product rounded on
+ * its own and summed in the order of r (DESIGN 3.3d); dsigma/drho = (1 - tanh^2 rho) / 2 * (max_scale - min_scale), as
+ * in sept_cloak_grl_bwd_f32.  dx = g needs no call.  eps_u follows sept_wave_cloak_eval_f32's draw rule with the same
+ * (eps_dev, seed, offset, draw_dev, utt_draw_dev, eps_std) and is generated again inside the kernel, not stored.  The call
+ * must receive the draw base its forward read: that forward's *draw_dev before sept_counter_add_u64 moved it (copy it
+ * to a buffer of its own before the counter moves).  tile_off_dev and n_tiles as for sept_wave_cloak_bwd_f32.
+ * workspace_dev holds sept_wave_cloak_bwd_per_utt_workspace_bytes(period) bytes (2 x 592 partial rows of the period);
+ * g_dev, rhos_dev, eps_dev, workspace_dev, dlocs_dev and drhos_dev 16-byte aligned.  Deterministic: no atomics, and the
+ * bits depend only on the layout and the draw inputs, not on the GPU; no allocation, capturable. */
+size_t sept_wave_cloak_bwd_per_utt_workspace_bytes(int period);
+int sept_wave_cloak_bwd_per_utt_f32(const float* g_dev, const int64_t* utt_off_dev, const int64_t* tile_off_dev,
+                                    int n_utts, int64_t n_tiles, int period, const float* rhos_dev,
+                                    const float* eps_dev, uint64_t seed, uint64_t offset, const uint64_t* draw_dev,
+                                    const int64_t* utt_draw_dev, float eps_std, float min_scale, float max_scale,
+                                    void* workspace_dev, float* dlocs_dev, float* drhos_dev, sept_stream_t stream);
+
 /* Class-balance noise augmentation (preprocess_data/preprocess_adversary_data.py:392-421): job j adds to row
  * job_row[j] of data_dev (n_rows, row_elems) the noise samples draw_id[job_ptr[j] .. job_ptr[j+1]) in that order -- the
  * reference writes the noisy copy through an alias of the source window, so a window drawn m times carries the sum of its

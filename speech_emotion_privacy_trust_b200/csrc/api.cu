@@ -626,6 +626,29 @@ int sept_wave_cloak_bwd_f32(const float* g, const int64_t* utt_off, const int64_
     return SEPT_OK;
 }
 
+size_t sept_wave_cloak_bwd_per_utt_workspace_bytes(int period) {
+    return period > 0 && period % 4 == 0 ? 2 * (size_t)sept::kWaveSlices * period * sizeof(float) : 0;
+}
+
+int sept_wave_cloak_bwd_per_utt_f32(const float* g, const int64_t* utt_off, const int64_t* tile_off, int n_utts,
+                                    int64_t n_tiles, int period, const float* rhos, const float* eps, uint64_t seed,
+                                    uint64_t offset, const uint64_t* draw_dev, const int64_t* utt_draw_dev, float eps_std,
+                                    float min_scale, float max_scale, void* workspace, float* dlocs, float* drhos,
+                                    sept_stream_t stream) {
+    if (!g || !utt_off || !tile_off || !rhos || !workspace || !dlocs || !drhos || n_utts < 0 || n_tiles < 0 || period <= 0)
+        return fail(SEPT_E_BADARG, "sept_wave_cloak_bwd_per_utt_f32: bad argument");
+    if (period % 4) return fail(SEPT_E_BADARG, "sept_wave_cloak_bwd_per_utt_f32: period=%d must be a multiple of 4", period);
+    if (!aligned16(g) || !aligned16(rhos) || !aligned16(eps) || !aligned16(workspace) || !aligned16(dlocs) || !aligned16(drhos))
+        return fail(SEPT_E_BADARG, "sept_wave_cloak_bwd_per_utt_f32: pointers must be 16-byte aligned");
+    sept::WaveReducePerUttParams p{};
+    p.r.g = g; p.r.utt_off = utt_off; p.r.tile_off = tile_off; p.r.n_utts = n_utts; p.r.n_tiles = n_tiles;
+    p.r.period = period; p.r.partial = static_cast<float*>(workspace); p.r.r = dlocs;
+    p.rhos = rhos; p.eps = eps; p.seed = seed; p.offset = offset; p.draw = draw_dev; p.utt_draw = utt_draw_dev;
+    p.eps_std = eps_std; p.min_scale = min_scale; p.max_scale = max_scale; p.drhos = drhos;
+    SEPT_CUDA(sept::launch_wave_reduce_per_utt(p, static_cast<cudaStream_t>(stream)));
+    return SEPT_OK;
+}
+
 int sept_add_noise_rows_f32(float* data_dev,const int64_t* job_row_dev, const int32_t* job_ptr_dev, const int64_t* draw_id_dev,
                             int n_jobs, int row_elems, uint64_t seed, float std, const float* noise_dev, sept_stream_t stream) {
     if (n_jobs == 0) return SEPT_OK;

@@ -133,16 +133,15 @@ __global__ void __launch_bounds__(kCloakThreads) cloak_bwd_kernel(const CloakBwd
     st4(p.dlocs + i, t);
     if (p.drhos) {
         const float4 rho = ld4(p.rhos + i), e = ld4(p.eps + i);
-        const float range = p.max_scale - p.min_scale;
-        const float th[4] = {tanhf(rho.x), tanhf(rho.y), tanhf(rho.z), tanhf(rho.w)};
+        const float ds[4] = {dsigma_of(rho.x, p.min_scale, p.max_scale), dsigma_of(rho.y, p.min_scale, p.max_scale),
+                             dsigma_of(rho.z, p.min_scale, p.max_scale), dsigma_of(rho.w, p.min_scale, p.max_scale)};
         const float em[4] = {e.x * m.x, e.y * m.y, e.z * m.z, e.w * m.w};
         const float tt[4] = {t.x, t.y, t.z, t.w};
         float r[4];
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
-            const float dsig = (1.0f - th[c] * th[c]) * 0.5f * range;
             // reg_coef = -scale_lambda / (wf * mean sigma): gradient of -scale_lambda * log(mean(sigma)) wrt sigma_i
-            r[c] = (tt[c] * em[c] + p.reg_coef) * dsig;
+            r[c] = (tt[c] * em[c] + p.reg_coef) * ds[c];
         }
         st4(p.drhos + i, make_float4(r[0], r[1], r[2], r[3]));
     }

@@ -18,6 +18,10 @@
 //   wave_eval_add_kernel evaluation: y[s] = x[s] + (mu[j] + sigma[j] * eps_u[j]), j = (s - utt_off[u]) mod L, a fresh
 //                       eps_u per utterance drawn inside the kernel (row d_u of sept_cloak_fwd_f32's per-sample draw);
 //                       a thread walks the phase quads that start in its aligned quad, one normal4 per phase quad.
+//   wave_reduce_per_utt_kernel  backward of the evaluation forward, pass 1: wave_reduce_kernel's rows of g and, in the
+//                       same order, rows of g * eps_u (each eps_u drawn again inside the kernel, one normal4 per tile and
+//                       phase quad, each product rounded on its own).
+//   wave_merge_per_utt_kernel   pass 2: both row sets merged in wave_merge_kernel's order; dlocs, drhos = q * sigma'.
 // No atomics: the order above is fixed, so the gradient is the same bits on every run (tests/wave_cloak_order.py
 // restates it on the host).  The add and the backward are HBM-bound with no reuse of x, y or g.
 #include <cuda_runtime.h>
@@ -223,7 +227,31 @@ __device__ __forceinline__ float4 tile_quad(const float* g, int64_t base, int le
     return v;
 }
 
-__global__ void __launch_bounds__(kWaveThreads) wave_reduce_kernel(const WaveReduceParams p) {
+__device__ __forceinline__ float4 f4mul(float4 a, float4 b) {                 // rounded on its own: no FMA into a sum
+    return make_float4(__fmul_rn(a.x, b.x), __fmul_rn(a.y, b.y), __fmul_rn(a.z, b.z), __fmul_rn(a.w, b.w));
+}
+
+// The per-utterance backward's staged tile data beyond base and length: the tile's Philox counter of phase quad 0
+// (offset + d_u * L/4, the draw rule of eval_utt), or, with the caller's eps, the offset of its utterance's row.
+__device__ __forceinline__ uint64_t* s_tile_ctr() { __shared__ uint64_t s[kWaveThreads]; return s; }
+__device__ __forceinline__ float4* s_red_eps() { __shared__ float4 s[kWaveThreads]; return s; }
+
+__device__ __forceinline__ uint64_t tile_ctr(const WaveReducePerUttParams& e, int u) {
+    const int L = e.r.period;
+    if (e.eps) return (uint64_t)u * L;
+    const uint64_t d = (e.draw ? *e.draw : 0) + (e.utt_draw ? (uint64_t)e.utt_draw[u] : (uint64_t)u);
+    return e.offset + d * (uint64_t)(L / 4);
+}
+
+// eps_u of the phases j .. j+3 (j a multiple of 4) of a tile: one normal4, the one wave_eval_add_kernel draws there
+__device__ __forceinline__ float4 tile_eps(const WaveReducePerUttParams& e, uint64_t ctr, int j) {
+    return e.eps ? __ldg(reinterpret_cast<const float4*>(e.eps + ctr + j)) : normal4(e.seed, ctr, (uint32_t)j / 4, e.eps_std);
+}
+
+// Backward pass 1 of slice blockIdx.x: the row of g (and, kEps, the row of g * eps_u, in the same order; a quad past
+// the tile's end adds nothing to it, as +0 would not).
+template <bool kEps>
+__device__ __forceinline__ void reduce_slice(const WaveReduceParams& p, const WaveReducePerUttParams* e) {
     __shared__ int64_t s_base[kWaveThreads];
     __shared__ int s_len[kWaveThreads];
     __shared__ float4 s_red[kWaveThreads];
@@ -233,13 +261,17 @@ __global__ void __launch_bounds__(kWaveThreads) wave_reduce_kernel(const WaveRed
     const int qt = R == 1 ? threadIdx.x : threadIdx.x % Q;
     const int64_t T0 = p.n_tiles * blockIdx.x / kWaveSlices, T1 = p.n_tiles * (blockIdx.x + 1) / kWaveSlices;
     float* row = p.partial + (size_t)blockIdx.x * L;
+    float* row_e = kEps ? p.partial + (size_t)(kWaveSlices + blockIdx.x) * L : nullptr;
     const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
     if (T0 == T1) {                                                 // an empty slice still writes its (zero) row
         if (lane == 0)
-            for (int q = qt; q < Q; q += kWaveThreads) *reinterpret_cast<float4*>(row + 4 * q) = zero;
+            for (int q = qt; q < Q; q += kWaveThreads) {
+                *reinterpret_cast<float4*>(row + 4 * q) = zero;
+                if constexpr (kEps) *reinterpret_cast<float4*>(row_e + 4 * q) = zero;
+            }
         return;
     }
-    float4 acc = zero;                                              // R > 1: the row element of quad qt
+    float4 acc = zero, acc_e = zero;                                // R > 1: the row elements of quad qt
     for (int64_t c0 = T0; c0 < T1; c0 += kWaveThreads) {
         const int nt = T1 - c0 < kWaveThreads ? (int)(T1 - c0) : kWaveThreads;
         __syncthreads();                                            // the previous chunk is no longer read
@@ -249,40 +281,72 @@ __global__ void __launch_bounds__(kWaveThreads) wave_reduce_kernel(const WaveRed
             const int64_t base = p.utt_off[u] + (i - p.tile_off[u]) * L, left = p.utt_off[u + 1] - base;
             s_base[threadIdx.x] = base;
             s_len[threadIdx.x] = left < L ? (int)left : L;
+            if constexpr (kEps) s_tile_ctr()[threadIdx.x] = tile_ctr(*e, u);
         }
         __syncthreads();
         if (R == 1) {
             for (int q = qt; q < Q; q += kWaveThreads) {
-                float4 l = zero;
+                float4 l = zero, le = zero;
 #pragma unroll 8
-                for (int t = 0; t < nt; ++t) l = f4add(l, tile_quad(p.g, s_base[t], s_len[t], 4 * q));
+                for (int t = 0; t < nt; ++t) {
+                    const float4 gq = tile_quad(p.g, s_base[t], s_len[t], 4 * q);
+                    l = f4add(l, gq);
+                    if constexpr (kEps)
+                        if (4 * q < s_len[t]) le = f4add(le, f4mul(gq, tile_eps(*e, s_tile_ctr()[t], 4 * q)));
+                }
                 float4* dst = reinterpret_cast<float4*>(row + 4 * q);
                 *dst = f4add(c0 == T0 ? zero : *dst, l);
+                if constexpr (kEps) {
+                    float4* dst_e = reinterpret_cast<float4*>(row_e + 4 * q);
+                    *dst_e = f4add(c0 == T0 ? zero : *dst_e, le);
+                }
             }
         } else {
-            float4 l = zero;
+            float4 l = zero, le = zero;
             if (lane < R)
-                for (int t = lane; t < nt; t += R) l = f4add(l, tile_quad(p.g, s_base[t], s_len[t], 4 * qt));
+                for (int t = lane; t < nt; t += R) {
+                    const float4 gq = tile_quad(p.g, s_base[t], s_len[t], 4 * qt);
+                    l = f4add(l, gq);
+                    if constexpr (kEps)
+                        if (4 * qt < s_len[t]) le = f4add(le, f4mul(gq, tile_eps(*e, s_tile_ctr()[t], 4 * qt)));
+                }
             s_red[threadIdx.x] = l;
+            if constexpr (kEps) s_red_eps()[threadIdx.x] = le;
             __syncthreads();
             if (lane == 0) {
                 float4 c = s_red[qt];
                 for (int k = 1; k < R; ++k) c = f4add(c, s_red[k * Q + qt]);
                 acc = f4add(acc, c);
+                if constexpr (kEps) {
+                    const float4* se = s_red_eps();
+                    float4 ce = se[qt];
+                    for (int k = 1; k < R; ++k) ce = f4add(ce, se[k * Q + qt]);
+                    acc_e = f4add(acc_e, ce);
+                }
             }
         }
     }
-    if (R > 1 && lane == 0) *reinterpret_cast<float4*>(row + 4 * qt) = acc;
+    if (R > 1 && lane == 0) {
+        *reinterpret_cast<float4*>(row + 4 * qt) = acc;
+        if constexpr (kEps) *reinterpret_cast<float4*>(row_e + 4 * qt) = acc_e;
+    }
+}
+
+__global__ void __launch_bounds__(kWaveThreads) wave_reduce_kernel(const WaveReduceParams p) {
+    reduce_slice<false>(p, nullptr);
+}
+
+__global__ void __launch_bounds__(kWaveThreads) wave_reduce_per_utt_kernel(const __grid_constant__ WaveReducePerUttParams p) {
+    reduce_slice<true>(p.r, &p);
 }
 
 constexpr int kMergeQuads = kWaveThreads / kWaveMergeLanes;        // 32 quads per CTA
 static_assert(kWaveSlices % kWaveMergeLanes == 0, "equal slice runs per merge lane");
 
-__global__ void __launch_bounds__(kWaveThreads) wave_merge_kernel(const float* __restrict__ partial, int L,
-                                                                  float* __restrict__ r) {
-    __shared__ float4 s_red[kWaveThreads];
+// Backward pass 2 at quad q of the period: the kWaveSlices rows at `partial` summed in order, valid in lane 0.  Every
+// thread of the CTA calls it (it synchronises); s_red is the caller's shared scratch of kWaveThreads quads.
+__device__ __forceinline__ float4 merge_quad(const float* __restrict__ partial, int L, int q, float4* s_red) {
     const int Q = L / 4, lane = threadIdx.x / kMergeQuads, qi = threadIdx.x % kMergeQuads;
-    const int q = blockIdx.x * kMergeQuads + qi;
     constexpr int per = kWaveSlices / kWaveMergeLanes;
     float4 a = make_float4(0.f, 0.f, 0.f, 0.f);
     if (q < Q) {
@@ -292,10 +356,36 @@ __global__ void __launch_bounds__(kWaveThreads) wave_merge_kernel(const float* _
     }
     s_red[threadIdx.x] = a;
     __syncthreads();
+    float4 c = a;
     if (lane == 0 && q < Q) {
-        float4 c = s_red[qi];
+        c = s_red[qi];
         for (int k = 1; k < kWaveMergeLanes; ++k) c = f4add(c, s_red[k * kMergeQuads + qi]);
-        reinterpret_cast<float4*>(r)[q] = c;
+    }
+    return c;
+}
+
+__global__ void __launch_bounds__(kWaveThreads) wave_merge_kernel(const float* __restrict__ partial, int L,
+                                                                  float* __restrict__ r) {
+    __shared__ float4 s_red[kWaveThreads];
+    const int q = blockIdx.x * kMergeQuads + threadIdx.x % kMergeQuads;
+    const float4 c = merge_quad(partial, L, q, s_red);
+    if (threadIdx.x < kMergeQuads && q < L / 4) reinterpret_cast<float4*>(r)[q] = c;
+}
+
+// dlocs = the merged rows of g; drhos = the merged rows of g * eps_u times sigma'(rho), rounded on its own
+__global__ void __launch_bounds__(kWaveThreads) wave_merge_per_utt_kernel(const float* __restrict__ partial, int L,
+                                                                          const float* __restrict__ rhos, float mn,
+                                                                          float mx, float* __restrict__ dlocs,
+                                                                          float* __restrict__ drhos) {
+    __shared__ float4 s_red[kWaveThreads], s_red_e[kWaveThreads];
+    const int q = blockIdx.x * kMergeQuads + threadIdx.x % kMergeQuads;
+    const float4 c = merge_quad(partial, L, q, s_red);
+    const float4 w = merge_quad(partial + (size_t)kWaveSlices * L, L, q, s_red_e);
+    if (threadIdx.x < kMergeQuads && q < L / 4) {
+        reinterpret_cast<float4*>(dlocs)[q] = c;
+        const float4 rho = __ldg(reinterpret_cast<const float4*>(rhos) + q);
+        reinterpret_cast<float4*>(drhos)[q] = f4mul(w, make_float4(dsigma_of(rho.x, mn, mx), dsigma_of(rho.y, mn, mx),
+                                                                   dsigma_of(rho.z, mn, mx), dsigma_of(rho.w, mn, mx)));
     }
 }
 
@@ -335,6 +425,16 @@ cudaError_t launch_wave_reduce(const WaveReduceParams& p, cudaStream_t stream) {
     if (e != cudaSuccess) return e;
     const int quads = p.period / 4;
     wave_merge_kernel<<<(quads + kMergeQuads - 1) / kMergeQuads, kWaveThreads, 0, stream>>>(p.partial, p.period, p.r);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_wave_reduce_per_utt(const WaveReducePerUttParams& p, cudaStream_t stream) {
+    wave_reduce_per_utt_kernel<<<kWaveSlices, kWaveThreads, 0, stream>>>(p);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    const int quads = p.r.period / 4;
+    wave_merge_per_utt_kernel<<<(quads + kMergeQuads - 1) / kMergeQuads, kWaveThreads, 0, stream>>>(
+        p.r.partial, p.r.period, p.rhos, p.min_scale, p.max_scale, p.r.r, p.drhos);
     return cudaGetLastError();
 }
 

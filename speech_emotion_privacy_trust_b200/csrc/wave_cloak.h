@@ -6,7 +6,7 @@
 
 namespace sept {
 
-constexpr int kWaveThreads = 256;     // threads per CTA of all three kernels; also the tiles staged per chunk
+constexpr int kWaveThreads = 256;     // threads per CTA of every kernel; also the tiles staged per chunk
 constexpr int kWaveSlices = 592;      // backward: partial rows (4 per B200 SM).  A constant, not the SM count: the
                                       // summation order, and so the bits of the gradient, are the same on every GPU
 constexpr int kWaveMergeLanes = 8;    // backward: lanes of the ordered slice sum (kWaveSlices / 8 = 74 slices each)
@@ -49,8 +49,20 @@ struct WaveEvalParams {
     float* y;                // (n) 16-byte aligned
 };
 
+struct WaveReducePerUttParams {
+    WaveReduceParams r;      // partial: workspace (2, kWaveSlices, period), the rows of g then those of g * eps_u; r: dlocs
+    const float* rhos;       // (period) 16-byte aligned
+    const float* eps;        // (n_utts, period) 16-byte aligned, or null -> Philox(seed, offset), as in WaveEvalParams
+    uint64_t seed, offset;
+    const uint64_t* draw;    // device draw base or null (0)
+    const int64_t* utt_draw; // (n_utts) device draw index of each utterance, or null (u)
+    float eps_std, min_scale, max_scale;
+    float* drhos;            // (period) 16-byte aligned
+};
+
 cudaError_t launch_wave_add(const WaveAddParams& p, cudaStream_t stream);
 cudaError_t launch_wave_eval(const WaveEvalParams& p, cudaStream_t stream);
 cudaError_t launch_wave_reduce(const WaveReduceParams& p, cudaStream_t stream);
+cudaError_t launch_wave_reduce_per_utt(const WaveReducePerUttParams& p, cudaStream_t stream);
 
 }  // namespace sept

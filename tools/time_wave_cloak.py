@@ -2,8 +2,10 @@
 """Time the waveform-domain cloak (wave_cloak.WaveCloak, period 32 000) on the bench corpus (5531 utterances, ~9.2
 audio-hours, ~532 M samples: x, y and the gradient each exceed L2), with CUDA events after a warm-up: the forward (noise
 draw + wave_add_kernel) and the backward (wave_reduce_kernel + wave_merge_kernel + the mu / rho kernel), per-kernel times
-from torch.profiler, and the bytes each must move, computed from shapes, against the HBM data-sheet bandwidth.  The card's
-name and power limit are read in the same run.  Prints one JSON line; with --out also writes it there."""
+from torch.profiler, and the bytes each must move, computed from shapes, against the HBM data-sheet bandwidth.  In the
+same run, the same for per-utterance noise (WaveCloak(per_utterance=True): wave_sigma_kernel + wave_eval_add_kernel
+forward, wave_reduce_per_utt_kernel + wave_merge_per_utt_kernel backward), under "per_utterance".  The card's name and
+power limit are read in the same run.  Prints one JSON line; with --out also writes it there."""
 import argparse
 import json
 import subprocess
@@ -18,7 +20,8 @@ import bench
 from speech_emotion_privacy_trust_b200 import extraction, wave_cloak
 
 HBM_TBPS = 7.7            # NVIDIA HGX B200 data sheet, per GPU
-KERNELS = ("wave_add_kernel", "wave_reduce_kernel", "wave_merge_kernel", "cloak_fwd_kernel", "cloak_bwd_kernel")
+KERNELS = ("wave_add_kernel", "wave_reduce_kernel", "wave_merge_kernel", "cloak_fwd_kernel", "cloak_bwd_kernel",
+           "wave_sigma_kernel", "wave_eval_add_kernel", "wave_reduce_per_utt_kernel", "wave_merge_per_utt_kernel")
 
 
 def events_ms(fn, reps):
@@ -80,13 +83,36 @@ def main():
         "wave_reduce_kernel": 4 * n + 2 * table + ws_rows,                    # g read, offsets + tiles, partial rows written
         "wave_merge_kernel": ws_rows + 4 * L,
     }
-    kernels = {}
-    for name, ms in k.items():
-        row = {"ms": round(ms, 4)}
-        if name in need:
-            row.update(gb=round(need[name] / 1e9, 3), gb_per_s=round(need[name] / ms / 1e6, 1),
-                       share_of_hbm=round(need[name] / ms / 1e9 / HBM_TBPS, 3))
-        kernels[name] = row
+
+    pu = wave_cloak.WaveCloak(1e-4, 1e-2, period=L, per_utterance=True).to(dev)
+
+    def forward_pu():
+        return pu(batch).wav
+
+    y_pu = forward_pu()
+    y_pu.backward(G, retain_graph=True)                                       # warm-up
+    fwd_pu = events_ms(forward_pu, args.reps)
+    bwd_pu = events_ms(lambda: y_pu.backward(G, retain_graph=True), args.reps)
+    k_pu = kernel_ms(forward_pu, args.reps)
+    k_pu.update(kernel_ms(lambda: y_pu.backward(G, retain_graph=True), args.reps))
+    ws_pu = wave_cloak._lib.lib().sept_wave_cloak_bwd_per_utt_workspace_bytes(L)
+    need.update({
+        "wave_eval_add_kernel": 8 * n + table + 8 * L,                        # x read, y written, offsets, mu and sigma
+        "wave_reduce_per_utt_kernel": 4 * n + 2 * table + ws_pu,              # g read, offsets + tiles, both row sets written
+        "wave_merge_per_utt_kernel": ws_pu + 12 * L,                          # both row sets, rho read, dlocs / drhos written
+    })
+
+    def rows(ks):
+        out = {}
+        for name, ms in ks.items():
+            row = {"ms": round(ms, 4)}
+            if name in need:
+                row.update(gb=round(need[name] / 1e9, 3), gb_per_s=round(need[name] / ms / 1e6, 1),
+                           share_of_hbm=round(need[name] / ms / 1e9 / HBM_TBPS, 3))
+            out[name] = row
+        return out
+
+    kernels = rows(k)
     fwd_bytes, bwd_bytes = 8 * n + table, 4 * n
     line = json.dumps({
         "gpu": gpu, "period": L, "audio_hours": round(hours, 3), "utterances": int(batch.n_utts), "samples": int(n),
@@ -95,6 +121,8 @@ def main():
         "forward_gb": round(fwd_bytes / 1e9, 3), "backward_gb": round(bwd_bytes / 1e9, 3),
         "forward_gb_per_s": round(fwd_bytes / fwd / 1e6, 1), "backward_gb_per_s": round(bwd_bytes / bwd / 1e6, 1),
         "kernels": kernels, "hbm_bound_tb_per_s": HBM_TBPS,
+        "per_utterance": {"forward_ms": round(fwd_pu, 3), "backward_ms": round(bwd_pu, 3), "kernels": rows(k_pu),
+                          "backward_workspace_gb": round(ws_pu / 1e9, 4)},
     })
     print(line)
     if args.out:
