@@ -112,9 +112,14 @@ int sept_mfcc_bwd_f32(const float* wav_dev, const int64_t* utt_off_dev, const in
  * Band-limited sinc resampling of a ragged batch.  Replaces torchaudio.transforms.Resample(sample_rate, 16000) as the
  * reference applies it to the 44.1 kHz MSP-Improv corpus (feature_extraction/audio_feature_extraction.py:139-141 ->
  * torchaudio/functional/functional.py _get_sinc_resample_kernel/_apply_sinc_resample_kernel: sinc_interp_hann,
- * lowpass_filter_width 6, rolloff 0.99).  Output length per utterance: ceil(new_freq * n / orig_freq). */
+ * lowpass_filter_width 6, rolloff 0.99).  Rates are reduced by their gcd to orig/up; at most 4096 of each
+ * (SEPT_E_UNSUPPORTED beyond).  Output length per utterance of n samples is torchaudio's:
+ * min(ceil(float32(up * n / orig)), (n / orig + 1) * up), the quotient taken in double, as Python's int / int, and
+ * rounded to float32, the default dtype torch.as_tensor gives it, before the ceil.  So it can differ by one either way
+ * from the exact ceil(up * n / orig); the second term is the number of samples torchaudio's conv1d produces. */
 
-/* HOST helper: out_off_host[n_utts+1] from in_off_host[n_utts+1]. */
+/* HOST helper: out_off_host[n_utts+1] from in_off_host[n_utts+1].  SEPT_E_BADARG for decreasing offsets and for an
+ * utterance with up * n >= 2^53, where the double quotient would no longer be Python's. */
 int sept_resample_layout(const int64_t* in_off_host, int n_utts, int orig_freq, int new_freq, int64_t* out_off_host);
 
 int sept_resample_f32(const float* in_dev, const int64_t* in_off_dev, const int64_t* out_off_dev, int n_utts,

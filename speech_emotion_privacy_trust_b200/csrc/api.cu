@@ -2,7 +2,9 @@
 #include <cuda_runtime.h>
 #include <cstdlib>
 
+#include <cmath>
 #include <cstdarg>
+#include <cstdint>
 #include <cstdio>
 #include <cstring>
 #include <map>
@@ -352,11 +354,23 @@ int sept_resample_layout(const int64_t* in_off, int n_utts, int orig_freq, int n
     if (!in_off || !out_off || n_utts < 0 || orig_freq <= 0 || new_freq <= 0)
         return fail(SEPT_E_BADARG, "sept_resample_layout: bad argument");
     const long long g = gcd_ll(orig_freq, new_freq), orig = orig_freq / g, up = new_freq / g;
+    if (orig > 4096 || up > 4096)
+        return fail(SEPT_E_UNSUPPORTED, "sept_resample_layout: %d -> %d reduces to %lld/%lld, beyond the 4096-phase table limit",
+                    orig_freq, new_freq, up, orig);
     out_off[0] = 0;
     for (int u = 0; u < n_utts; ++u) {
         const long long n = in_off[u + 1] - in_off[u];
         if (n < 0) return fail(SEPT_E_BADARG, "sept_resample_layout: offsets must be non-decreasing");
-        out_off[u + 1] = out_off[u] + (up * n + orig - 1) / orig;     // ceil(new * length / orig), functional.py
+        // torchaudio's _apply_sinc_resample_kernel cuts at ceil(torch.as_tensor(new * length / orig)): Python's double
+        // quotient, rounded to the default dtype float32 before the ceil, and at most the (n / orig + 1) * up samples its
+        // conv1d produces.  The double quotient below is Python's while up * n < 2^53.
+        if (n > ((1LL << 53) - 1) / up)
+            return fail(SEPT_E_BADARG, "sept_resample_layout: utterance %d has %lld samples, too many for the length rule", u, n);
+        const long long cut = (long long)ceilf((float)((double)(up * n) / (double)orig));
+        const long long conv = (n / orig + 1) * up;
+        const long long len = cut < conv ? cut : conv;
+        if (out_off[u] > INT64_MAX - len) return fail(SEPT_E_BADARG, "sept_resample_layout: total output length overflows");
+        out_off[u + 1] = out_off[u] + len;
     }
     return SEPT_OK;
 }

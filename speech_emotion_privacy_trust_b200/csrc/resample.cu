@@ -14,6 +14,7 @@
 #include <cstdint>
 
 #include "resample.h"
+#include "resample_shape.h"
 #include "vec.cuh"
 
 namespace sept {
@@ -65,28 +66,9 @@ __global__ void __launch_bounds__(kResampleThreads) resample_kernel(const Resamp
 // torchaudio's padding) next to the grouped weight table, and a thread computes a 4 x 4 tile -- four consecutive phases
 // j of four consecutive rows m (output sample m * up + j) -- walking once over the group's TG-tap window: one 16-byte
 // weight load and four input loads feed sixteen FMAs.  Accumulation runs over ascending taps like the kernel above.
-constexpr int kTileThreads = 256;
-
-struct TileGeom { int rows_per_cta, stage_floats; };
-
-__host__ __device__ inline TileGeom resample_tile_geom(int orig, int n_groups, int tg, int base_min, int base_max) {
-    // rows (m) per CTA: a multiple of 4, about kTileThreads tiles, and a stage of at most ~9k floats
-    int mg = kTileThreads / n_groups;
-    const int mg_fit = (9000 / orig - 4) / 4;
-    if (mg > mg_fit) mg = mg_fit;
-    if (mg < 1) mg = 1;
-    TileGeom g;
-    g.rows_per_cta = 4 * mg;
-    // rows m_lo .. m_lo + 4 (mg + 1) - 1 can be touched (a CTA's sample range need not start on a row boundary)
-    g.stage_floats = ((4 * (mg + 1) - 1) * orig + (base_max - base_min) + tg + 3 + 4) & ~3;   // + 3: 16-byte aligned fill
-    return g;
-}
-
 // A CTA is two independent halves of kTileThreads threads that share the weight table and each walk their own chunk
 // range with their own stage and their own named barrier: a third more resident warps for the same shared memory.
 __device__ __forceinline__ void half_barrier(int half) { asm volatile("bar.sync %0, %1;" ::"r"(half + 1), "n"(kTileThreads) : "memory"); }
-
-constexpr int kTileTapsFast = 43;                      // taps of a 4-phase group at 44.1 -> 16 kHz (the reference's MSP-Improv case)
 
 template <int TG>                                      // TG > 0: p.tg == TG, the tap loop is unrolled; 0: any tap count
 __global__ void __launch_bounds__(2 * kTileThreads) resample_tiled_kernel(const ResampleParams p) {
@@ -211,11 +193,6 @@ __global__ void __launch_bounds__(2 * kTileThreads) resample_tiled_kernel(const 
     }
 }
 
-static size_t resample_tiled_smem(const ResampleParams& p) {
-    const TileGeom geo = resample_tile_geom(p.orig, p.n_groups, p.tg, p.base_min, p.base_max);
-    return (size_t)p.n_groups * p.tg * 16 + (size_t)((p.n_groups + 3) & ~3) * 4 + 2 * (size_t)geo.stage_floats * 4;
-}
-
 // 16-bit PCM -> float in [-1, 1): x / 32768, what torchaudio.load(normalize=True) does on the host before the reference's
 // callables see the audio (audio_feature_extraction.py:182).  Lets a bulk job ship half the bytes over PCIe.
 __global__ void __launch_bounds__(256) pcm16_to_f32_kernel(const short* __restrict__ in, long long n, float* __restrict__ out) {
@@ -233,20 +210,17 @@ cudaError_t launch_pcm16_to_f32(const short* in, long long n, float* out, cudaSt
 
 cudaError_t launch_resample(const ResampleParams& p, cudaStream_t stream) {
     if (p.total_out <= 0) return cudaSuccess;
-    if (p.tile_wt) {
-        const size_t smem = resample_tiled_smem(p);
-        if (smem <= 112 * 1024) {                                  // two CTAs per SM at least; larger tables take the simple kernel
-            const TileGeom geo = resample_tile_geom(p.orig, p.n_groups, p.tg, p.base_min, p.base_max);
-            const long long per_cta = (long long)geo.rows_per_cta * p.up;
-            long long blocks = (p.total_out + per_cta - 1) / per_cta;
-            const long long resident = 148LL * (smem <= 72 * 1024 ? 3 : 2);   // CTAs of two independent halves
-            if (blocks > resident) blocks = resident;              // persistent: the weight table is loaded once per CTA
-            auto kern = p.tg == kTileTapsFast ? resample_tiled_kernel<kTileTapsFast> : resample_tiled_kernel<0>;
-            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            if (e != cudaSuccess) return e;
-            kern<<<(unsigned)blocks, 2 * kTileThreads, smem, stream>>>(p);
-            return cudaGetLastError();
-        }
+    const ResampleShape s = resample_shape(p.tile_wt != nullptr, p.orig, p.n_groups, p.tg, p.base_min, p.base_max);
+    if (s.kernel != kResampleSimple) {
+        const long long per_cta = (long long)s.geo.rows_per_cta * p.up;
+        long long blocks = (p.total_out + per_cta - 1) / per_cta;
+        const long long resident = 148LL * s.ctas_per_sm;         // CTAs of two independent halves
+        if (blocks > resident) blocks = resident;                  // persistent: the weight table is loaded once per CTA
+        auto kern = s.kernel == kResampleTiledFast ? resample_tiled_kernel<kTileTapsFast> : resample_tiled_kernel<0>;
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)s.smem);
+        if (e != cudaSuccess) return e;
+        kern<<<(unsigned)blocks, 2 * kTileThreads, s.smem, stream>>>(p);
+        return cudaGetLastError();
     }
     const long long blocks = (p.total_out + kResampleThreads - 1) / kResampleThreads;
     resample_kernel<<<(unsigned)blocks, kResampleThreads, 0, stream>>>(p);

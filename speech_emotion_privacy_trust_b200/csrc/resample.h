@@ -8,7 +8,7 @@ namespace sept {
 struct ResampleParams {
     const float* in;            // ragged input, all utterances back to back
     const int64_t* in_off;      // [n_utts + 1]
-    const int64_t* out_off;     // [n_utts + 1], length ceil(new * n_in / orig) per utterance
+    const int64_t* out_off;     // [n_utts + 1], any length per utterance; sept_resample_layout gives torchaudio's
     int n_utts;
     int orig, up;               // orig_freq / gcd, new_freq / gcd
     int width;                  // zero-crossing half width in input samples (torchaudio's `width`)
